@@ -68,7 +68,17 @@ def parse_args():
                          "NVLink + a one-word NCCL all-reduce as the fence; nccl: dist.gather + placement")
     ap.add_argument("--path", default="auto", choices=["auto", "index", "buckets", "blocks", "split"],
                     help="rcp_set_coverage_path: how rcp_coverage finds each region's reads")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the profile matrix of the last timed step (rank 0: the "
+                         "gathered matrix) as DIR/profile.npy, regions x bins float64; above 64 MB a fixed, "
+                         "seeded sample of its rows. The inputs are seeded, so two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm sizes its sample by a timed "
+                 "calibration pass, so its inputs differ from run to run")
+    return args
 
 
 def peaks():
@@ -710,6 +720,21 @@ def run_strong(env, args, world, rank, which="C5"):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def matrix_to_host(mat):
+    """A device matrix [bins, regions] (column-major regions x bins, as the step writes it) as the
+    regions x bins float64 array a caller receives.  Above DUMP_BYTES only whole rows are kept: a
+    sample fixed by its seed and the row count, in row order, so every build keeps the same rows."""
+    import torch
+    ncols, n_rows = mat.shape
+    if n_rows * ncols * 8 > DUMP_BYTES:
+        rows = np.random.default_rng(0).choice(n_rows, size=max(DUMP_BYTES // (8 * ncols), 1), replace=False)
+        mat = mat.index_select(1, torch.from_numpy(np.sort(rows)).to(mat.device))
+    return mat.t().contiguous().cpu().numpy()
+
+
 def bind_cpu_near_gpu(local):
     """One process per GPU: run this process (and place its page-locked buffers, by first touch)
     on the CPUs of the GPU's own NUMA node, so that the N uploads of a step do not cross the socket
@@ -888,6 +913,10 @@ def run_b200(args):
     launches = int(L.rcp_launch_count(0))
     stage = stage_table(L, _lib)
     _lib.check(L.rcp_timing_enable(0))
+    # taken here: the untimed steps below write the same buffers again
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = matrix_to_host(gather_box["full"] if world > 1 else bufs[(args.steps - 1) % len(bufs)])
     # The timed region is a few tens of milliseconds, shorter than one nvidia-smi period: keep
     # the same steps running (untimed) for about a second so that the clock record is taken UNDER
     # THIS LOAD.  The number of extra steps is agreed by all ranks (never a rank-local wall
@@ -1208,6 +1237,9 @@ def run_b200(args):
             out["exchange_verified"] = exchange_ok
         if cpu is not None:
             out["cpu_baseline"] = cpu
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "profile.npy"), dumped)
         print(json.dumps(out))
     if world > 1:
         dist.barrier()
