@@ -230,6 +230,43 @@ int rcp_bam_index(const uint8_t* rec /* host */, int64_t n_bytes, int64_t* n_rec
 int rcp_bam_decode(const uint8_t* rec, int64_t n_bytes, const int64_t* offsets, int64_t n_records,
                    int n_ref, const int64_t* ref_len /* host */, int splice_split, int mem,
                    int* decoded_out, int64_t* n_out);
+/* rcp_bam_decode_param  rcp_bam_decode under a ScanBamParam (readGAlignments(file, param =
+ *   bamParams), Rsamtools / GenomicAlignments documented behaviour).  The filters act on each
+ *   record before its ranges are made; trim(), split and the caller's "remove" act on what passes.
+ *   Every mapped record is checked for errors, whether the filters keep it or not.
+ *   flag       (host) {keep0, keep1} = bamFlag(param, asInteger = TRUE) over the 12 flag bits
+ *              0x1 .. 0x800; NULL = no flag filter.  A record passes iff every bit set in FLAG is
+ *              set in keep1 and every bit clear in FLAG is set in keep0 (scanBamFlag: TRUE clears
+ *              the bit in keep0, FALSE in keep1, NA leaves both).  Unmapped records (0x4) are
+ *              dropped whatever the flag words say, as readGAlignments ANDs isUnmappedQuery = FALSE.
+ *   mapq_min   keep MAPQ >= mapq_min (255 "unavailable" is the number 255); < 0: no filter (NA).
+ *   simple_cigar  != 0: keep only a CIGAR of one M operation (10M5M is not simple).
+ *   which      n_which ranges (host arrays): reference id (into the header's references), start,
+ *              end, 1-based closed, 1 <= start <= end <= 536870912, in the order of
+ *              as(which, "IntegerRangesList").  A record overlaps [s, e] iff POS < e and
+ *              POS + span > s - 1 (POS 0-based; span = the CIGAR's M D N = X, 1 when that is 0,
+ *              htslib bam_endpos), before trim().  The output is range by range, each in file
+ *              order; a record that overlaps k ranges appears k times (each appearance split at
+ *              its N operations under splice_split).  Needs the records sorted by (refID, POS),
+ *              unplaced ones (refID -1) last -- checked on the records, RCP_ERR_DATA if not.
+ *              n_which = 0: no which, file order, unsorted records are fine.
+ *   tagFilter  n_tags (<= 32) tags, tag_names = their 2 characters one after the other; tag k
+ *              accepts the values [tag_ptr[k], tag_ptr[k+1]) of int_values (tag_type[k] = 0,
+ *              matches the integer fields c C s S i I by value) or of str_values (tag_type[k] = 1,
+ *              matches Z and A fields exactly).  A record passes iff every tag is present (first
+ *              occurrence) with an accepted value; a missing tag or one of another type (f, H, B,
+ *              or the other kind) fails.  The aux fields after read_name, CIGAR, seq ((l_seq+1)/2
+ *              bytes) and qual (l_seq bytes) are walked over every SAMv1 4.2.4 type; a field that
+ *              runs past its record is RCP_ERR_DATA.  The values take at most 32 KB.
+ *   With no filter given (flag NULL, mapq_min < 0, simple_cigar 0, n_which 0, n_tags 0) the
+ *   result equals rcp_bam_decode's. */
+int rcp_bam_decode_param(const uint8_t* rec, int64_t n_bytes, const int64_t* offsets, int64_t n_records,
+                         int n_ref, const int64_t* ref_len /* host */, int splice_split, int mem,
+                         const int32_t* flag /* keep0, keep1 */, int mapq_min /* < 0: NA */, int simple_cigar,
+                         int n_which, const int32_t* which_ref, const int32_t* which_start,
+                         const int32_t* which_end, int n_tags, const char* tag_names, const int32_t* tag_ptr,
+                         const int32_t* tag_type /* 0 integer, 1 string */, const int64_t* int_values,
+                         const char* const* str_values, int* decoded_out, int64_t* n_out);
 int rcp_bed_decode(const char* text, int64_t n_bytes, int n_names, const char* const* names /* host */,
                    int mem, int* decoded_out, int64_t* n_out);
 int rcp_decoded_fetch(int decoded, int32_t* chrom, int32_t* start, int32_t* end, int8_t* strand,

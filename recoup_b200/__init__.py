@@ -14,7 +14,8 @@ from .coverage import (CoverageList, DeviceReads, calcCoverage, coverageRef, cov
 from .preprocess import SelectedGRanges, preprocessRanges, readRanges, sampleSorted, widthQuantile
 from .profile import (ProfileMatrix, baseCoverageMatrix, binCoverageMatrix, coverageProfile,
                       haveEqualLengths, profileMatrix)
-from .readers import DecodedGRanges, decodeBam, readBam, readBed, readRangesFile
+from .readers import (DecodedGRanges, ScanBamParam, decodeBam, readBam, readBed, readRangesFile,
+                      scanBamFlag)
 from .ranges import GRanges, GRangesList, Rle, getFlankingRanges, getRegionalRanges
 
 __all__ = [
@@ -24,5 +25,5 @@ __all__ = [
     "haveEqualLengths", "coverageProfile", "ProfileMatrix", "set_verbose", "calcPlotProfiles", "orderProfiles",
     "heatmapScale", "colProfile", "rowStat", "sortIndex", "matrixQuantile", "preprocessRanges",
     "readRanges", "SelectedGRanges", "sampleSorted", "widthQuantile", "readBam", "readBed", "readRangesFile",
-    "decodeBam", "DecodedGRanges",
+    "decodeBam", "DecodedGRanges", "ScanBamParam", "scanBamFlag",
 ]

@@ -69,6 +69,9 @@ SIGNATURES = {
     "rcp_bgzf_inflate": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int]),
     "rcp_bam_index": (C.c_int, [_vp, C.c_int64, _i64p, _vp, C.c_int64]),
     "rcp_bam_decode": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int, _i64p, C.c_int, C.c_int, _ip, _i64p]),
+    "rcp_bam_decode_param": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int, _i64p, C.c_int, C.c_int, _i32p,
+                                       C.c_int, C.c_int, C.c_int, _i32p, _i32p, _i32p, C.c_int, C.c_char_p, _i32p,
+                                       _i32p, _i64p, C.POINTER(C.c_char_p), _ip, _i64p]),
     "rcp_bed_decode": (C.c_int, [_vp, C.c_int64, C.c_int, C.POINTER(C.c_char_p), C.c_int, _ip, _i64p]),
     "rcp_decoded_fetch": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, C.c_int64]),
     "rcp_decoded_free": (C.c_int, [C.c_int]),

@@ -87,10 +87,11 @@ def sampleSorted(lib_sizes, size, seed, sample_kind="Rejection"):
     return [out[i * int(size):(i + 1) * int(size)] for i in range(n.shape[0])]
 
 
-def readRanges(x, reader, spliceAction="keep", spliceRemoveQ=0.75):
+def readRanges(x, reader, spliceAction="keep", spliceRemoveQ=0.75, bamParams=None):
     """readRanges / readBam after the decode (ranges.R:102-134): "keep" and "split" differ only in
     how the file is decoded (the reader's business); "remove" drops the reads wider than the
-    spliceRemoveQ quantile of the widths."""
+    spliceRemoveQ quantile of the widths.  `bamParams` (a ScanBamParam) filters the records of a
+    BAM file; BED files and a `reader` callable do not see it."""
     if spliceAction not in ("keep", "remove", "split"):
         raise ValueError("sa must be one of keep, remove, split")
     if not 0 <= spliceRemoveQ <= 1:
@@ -101,7 +102,7 @@ def readRanges(x, reader, spliceAction="keep", spliceRemoveQ=0.75):
         if x.get("file") is None or x.get("format") is None:
             raise ValueError("One or more input files cannot be read: no file / format and no reader")
         gr = readRangesFile(x["file"], x["format"], "split" if spliceAction == "split" else "keep",
-                            seqlevels=x.get("seqlevels"), seqlengths=x.get("seqlengths"))
+                            seqlevels=x.get("seqlevels"), seqlengths=x.get("seqlengths"), bamParams=bamParams)
     else:
         gr = reader(x)
     if spliceAction != "remove" or len(gr) == 0:
@@ -117,7 +118,9 @@ def preprocessRanges(input, preprocessParams, bamParams=None, rc=None, reader=No
     (ranges.R:2-4); else reads ALL samples through `reader` and applies
     preprocessParams$normalize: "none" / "linear" keep the reads as read (linear acts after the
     coverage), "downsample" draws min(library sizes) reads from every sample, "sampleto" draws
-    preprocessParams$sampleTo, both with ONE set.seed(preprocessParams$seed)."""
+    preprocessParams$sampleTo, both with ONE set.seed(preprocessParams$seed).  `bamParams`: a
+    ScanBamParam for the BAM files read here (ranges.R:18-19); the library sizes that
+    "downsample" / "sampleto" draw from are those of the filtered reads."""
     if not any(x.get("ranges") is None for x in input):
         return input
     pp = preprocessParams
@@ -127,7 +130,8 @@ def preprocessRanges(input, preprocessParams, bamParams=None, rc=None, reader=No
     ranges = []
     for x in input:
         _message("Reading sample ", x.get("name"))
-        ranges.append(readRanges(x, reader, pp.get("spliceAction", "keep"), pp.get("spliceRemoveQ", 0.75)))
+        ranges.append(readRanges(x, reader, pp.get("spliceAction", "keep"), pp.get("spliceRemoveQ", 0.75),
+                                 bamParams))
     if normalize in ("downsample", "sampleto"):
         lib = [len(r) for r in ranges]
         size = min(lib) if normalize == "downsample" else int(pp["sampleTo"])

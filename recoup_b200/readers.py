@@ -7,7 +7,8 @@
 What stays on the host: opening the file, the BGZF inflate (rcp_bgzf_inflate: zlib, one thread per
 core, C++ inside the library), the BAM header (text + reference list) and the walk of the
 length-prefixed record chain (rcp_bam_index, also inside the library).  Everything per read -- flag
-filter, CIGAR walk, N-split, trim, text parsing, compaction in file order -- runs on the device (rcp_bam_decode / rcp_bed_decode); the decoded reads stay in
+filter and the other ScanBamParam filters, CIGAR walk, N-split, trim, text parsing, compaction in file
+order (or in `which` order) -- runs on the device (rcp_bam_decode[_param] / rcp_bed_decode); the decoded reads stay in
 HBM and go to the hot path without a host round trip (rcp_reads_load_decoded).  Their coordinates
 are copied to the host only when somebody reads them.
 """
@@ -101,9 +102,112 @@ def bam_header(raw):
     return names, np.asarray(lens, dtype=np.int64), p
 
 
-def decodeBam(raw, split=False):
-    """Inflated BAM bytes -> DecodedGRanges: readGAlignments + as(., "GRanges") (or
-    unlist(grglist(.)) when `split`) + trim."""
+FLAG_BITS = ("isPaired", "isProperPair", "isUnmappedQuery", "hasUnmappedMate", "isMinusStrand",
+             "isMateMinusStrand", "isFirstMateRead", "isSecondMateRead", "isSecondaryAlignment",
+             "isNotPassingQualityControls", "isDuplicate", "isSupplementaryAlignment")   # 0x1 .. 0x800
+WHICH_MAX_END = 536870912       # 2^29, the largest end Rsamtools accepts
+
+
+def scanBamFlag(isPaired=None, isProperPair=None, isUnmappedQuery=None, hasUnmappedMate=None,
+                isMinusStrand=None, isMateMinusStrand=None, isFirstMateRead=None, isSecondMateRead=None,
+                isSecondaryAlignment=None, isNotPassingQualityControls=None, isDuplicate=None,
+                isSupplementaryAlignment=None):
+    """Rsamtools' scanBamFlag: each argument True, False or None (NA).  Returns the pair
+    bamFlag(asInteger = TRUE) = (keep0, keep1): True clears the bit in keep0 (only records with
+    the bit set pass), False clears it in keep1 (only records with it clear pass)."""
+    args = locals()
+    keep0 = keep1 = 0xfff
+    for bit, name in enumerate(FLAG_BITS):
+        v = args[name]
+        if v is None:
+            continue
+        if not isinstance(v, (bool, np.bool_)):
+            raise ValueError("scanBamFlag: %s must be True, False or None" % name)
+        if v:
+            keep0 &= ~(1 << bit)
+        else:
+            keep1 &= ~(1 << bit)
+    return keep0, keep1
+
+
+class ScanBamParam:
+    """Rsamtools' ScanBamParam, the parts that decide which alignments readGAlignments returns:
+
+    flag         a (keep0, keep1) pair from scanBamFlag; None = every record (unmapped records are
+                 dropped whatever it says: readGAlignments ANDs isUnmappedQuery = FALSE in).
+    mapqFilter   keep MAPQ >= mapqFilter; None = NA, no filter.
+    which        a GRanges, or a list of (seqname, start, end), 1-based closed.  The output is
+                 range by range in the order of as(which, "IntegerRangesList") -- grouped by the
+                 seqlevels of `which` in level order (for a list: the order the seqnames first
+                 appear in), ranges in their given order within a level, file order within a
+                 range -- and a record overlapping k ranges is returned k times.  Needs the
+                 records sorted by position.
+    simpleCigar  keep only alignments whose CIGAR is one M operation.
+    tagFilter    {tag: accepted values}: a record passes iff every tag is present with one of
+                 its values; integers match integer fields, strings Z and A fields.
+    what, tag, reverseComplement  accepted; they only touch columns that as(., "GRanges") drops.
+    """
+
+    def __init__(self, flag=None, mapqFilter=None, which=None, simpleCigar=False, tagFilter=None,
+                 what=None, tag=None, reverseComplement=False):
+        if flag is None:
+            flag = (0xfff, 0xfff)
+        if (len(flag) != 2 or any(isinstance(x, bool) or int(x) != x or not 0 <= int(x) <= 0xfff for x in flag)):
+            raise ValueError("flag must be a (keep0, keep1) pair of 12-bit masks, as scanBamFlag returns")
+        self.flag = (int(flag[0]), int(flag[1]))
+        if mapqFilter is not None:
+            if isinstance(mapqFilter, bool) or int(mapqFilter) != mapqFilter or mapqFilter < 0:
+                raise ValueError("mapqFilter must be a non-negative integer or None")
+            mapqFilter = int(mapqFilter)
+        self.mapqFilter = mapqFilter
+        if not isinstance(simpleCigar, (bool, np.bool_)):
+            raise ValueError("simpleCigar must be True or False")
+        self.simpleCigar = bool(simpleCigar)
+        self.which = None if which is None else _which_ranges(which)
+        if self.which is not None:      # the same as arrays: level names, level index, start, end
+            levels = list(dict.fromkeys(c for c, _, _ in self.which))
+            lut = {c: i for i, c in enumerate(levels)}
+            self._which_arrays = (levels, np.asarray([lut[c] for c, _, _ in self.which], dtype=np.int32),
+                                  np.asarray([x[1] for x in self.which], dtype=np.int32),
+                                  np.asarray([x[2] for x in self.which], dtype=np.int32))
+        self.tagFilter = {}
+        for name, values in (tagFilter or {}).items():
+            if not isinstance(name, str) or len(name) != 2:
+                raise ValueError("tagFilter: tag name %r is not 2 characters" % (name,))
+            vals = list(values) if isinstance(values, (list, tuple, np.ndarray)) else [values]
+            is_str = [isinstance(v, str) for v in vals]
+            if any(is_str) and not all(is_str):
+                raise ValueError("tagFilter: tag %s mixes integer and character values" % name)
+            if not all(is_str) and any(isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, np.integer))
+                                       for v in vals):
+                raise ValueError("tagFilter: tag %s: values must be integers or strings" % name)
+            self.tagFilter[name] = [v if isinstance(v, str) else int(v) for v in vals]
+        self.what, self.tag, self.reverseComplement = what, tag, reverseComplement
+
+    def keep_words(self):
+        """The flag pair readGAlignments applies: the user's AND isUnmappedQuery = FALSE."""
+        return self.flag[0], self.flag[1] & ~0x4
+
+
+def _which_ranges(which):
+    """[(seqname, start, end)] in IntegerRangesList order, validated."""
+    if isinstance(which, GRanges):
+        ids = np.asarray(which.seqnames)
+        rows = [(which.seqlevels[int(c)], int(s), int(e)) for c, s, e in zip(ids, which.start, which.end)]
+        levels = list(which.seqlevels)
+    else:
+        rows = [(str(c), int(s), int(e)) for c, s, e in which]
+        levels = list(dict.fromkeys(c for c, _, _ in rows))
+    for c, s, e in rows:
+        if s < 1 or e < s or e > WHICH_MAX_END:
+            raise ValueError("which: range %s:%d-%d needs 1 <= start <= end <= %d" % (c, s, e, WHICH_MAX_END))
+    rank = {c: i for i, c in enumerate(levels)}
+    return sorted(rows, key=lambda x: rank[x[0]])          # stable: the given order within a level
+
+
+def decodeBam(raw, split=False, params=None):
+    """Inflated BAM bytes -> DecodedGRanges: readGAlignments (with `params`, a ScanBamParam) +
+    as(., "GRanges") (or unlist(grglist(.)) when `split`) + trim."""
     _lib.ensure_init()
     names, lens, first = bam_header(raw)
     rec = np.frombuffer(raw, dtype=np.uint8, offset=first)
@@ -113,21 +217,56 @@ def decodeBam(raw, split=False):
     off = np.zeros(n_rec.value + 1, dtype=np.int64)
     _lib.check(_lib.lib.rcp_bam_index(vp(rec), rec.shape[0], C.byref(n_rec), vp(off), off.shape[0]))
     h, n_out = C.c_int(0), C.c_int64(0)
-    _lib.check(_lib.lib.rcp_bam_decode(vp(rec), rec.shape[0], vp(off), n_rec.value, len(names),
-                                       lens.ctypes.data_as(C.POINTER(C.c_int64)), 1 if split else 0,
-                                       _lib.MEM_HOST, C.byref(h), C.byref(n_out)))
+    lens_p = lens.ctypes.data_as(C.POINTER(C.c_int64))
+    if params is None:
+        _lib.check(_lib.lib.rcp_bam_decode(vp(rec), rec.shape[0], vp(off), n_rec.value, len(names), lens_p,
+                                           1 if split else 0, _lib.MEM_HOST, C.byref(h), C.byref(n_out)))
+    else:
+        _lib.check(bam_decode_param(vp(rec), rec.shape[0], vp(off), n_rec.value, names, lens, split, _lib.MEM_HOST,
+                                    params, h, n_out))
     return DecodedGRanges(h.value, n_out.value, names, lens)
 
 
+def bam_decode_param(rec, n_bytes, off, n_rec, names, lens, split, mem, params, h, n_out):
+    """rcp_bam_decode_param with the arguments of a ScanBamParam; returns the status code."""
+    i32p = C.POINTER(C.c_int32)
+    a32 = lambda x: np.ascontiguousarray(x, dtype=np.int32)
+    flag = a32(params.keep_words())
+    n_which, w_ref, w_start, w_end = 0, a32([]), a32([]), a32([])
+    if params.which is not None:
+        levels, level_idx, w_start, w_end = params._which_arrays
+        lut = {c: i for i, c in enumerate(names)}
+        for c in levels:
+            if c not in lut:
+                raise ValueError("which: seqname %s is not among the BAM header's references" % c)
+        w_ref = a32([lut[c] for c in levels])[level_idx] if levels else a32([])
+        n_which = w_ref.shape[0]
+    tags = list(params.tagFilter.items())
+    tag_names = "".join(t for t, _ in tags).encode("ascii")
+    tag_ptr = a32(np.cumsum([0] + [len(v) for _, v in tags]))
+    tag_type = a32([1 if v and isinstance(v[0], str) else 0 for _, v in tags])
+    flat = [x for _, v in tags for x in v]
+    int_values = np.asarray([x if isinstance(x, int) else 0 for x in flat], dtype=np.int64)
+    str_values = (C.c_char_p * max(len(flat), 1))(*[x.encode("utf-8") if isinstance(x, str) else b"" for x in flat])
+    lens = np.ascontiguousarray(lens, dtype=np.int64)
+    return _lib.lib.rcp_bam_decode_param(
+        rec, n_bytes, off, n_rec, len(names), lens.ctypes.data_as(C.POINTER(C.c_int64)), 1 if split else 0, mem,
+        flag.ctypes.data_as(i32p), -1 if params.mapqFilter is None else params.mapqFilter,
+        1 if params.simpleCigar else 0, n_which, w_ref.ctypes.data_as(i32p), w_start.ctypes.data_as(i32p),
+        w_end.ctypes.data_as(i32p), len(tags), tag_names, tag_ptr.ctypes.data_as(i32p), tag_type.ctypes.data_as(i32p),
+        int_values.ctypes.data_as(C.POINTER(C.c_int64)), str_values, C.byref(h), C.byref(n_out))
+
+
 def readBam(bam, sa="keep", sq=0.75, params=None):
-    """ranges.R:111-134.  `bam`: a path, or the bytes of the file."""
+    """ranges.R:111-134.  `bam`: a path, or the bytes of the file; `params`: a ScanBamParam (the
+    reference's bamParams), None for readGAlignments' default."""
     if sa not in ("keep", "remove", "split"):
         raise ValueError("sa must be one of keep, remove, split")
     if not 0 <= sq <= 1:
         raise ValueError("sq must be in [0, 1]")
     data = bam if isinstance(bam, (bytes, bytearray, memoryview)) else open(bam, "rb").read()
     raw = bgzfInflate(data)                     # BGZF blocks inflated in parallel (host zlib)
-    reads = decodeBam(raw, split=(sa == "split"))
+    reads = decodeBam(raw, split=(sa == "split"), params=params)
     if sa != "remove" or len(reads) == 0:
         return reads
     qu, n_kept = widthQuantile(reads, sq)
@@ -151,10 +290,11 @@ def readBed(bed, seqlevels, seqlengths=None):
     return DecodedGRanges(h.value, n_out.value, seqlevels, seqlengths)
 
 
-def readRangesFile(input, format, sa="keep", sq=0.75, seqlevels=None, seqlengths=None):
-    """readRanges (ranges.R:102-109) for files; "bigwig" has no reads (NULL)."""
+def readRangesFile(input, format, sa="keep", sq=0.75, seqlevels=None, seqlengths=None, bamParams=None):
+    """readRanges (ranges.R:102-109) for files; "bigwig" has no reads (NULL).  `bamParams` (a
+    ScanBamParam) applies to BAM files only, as in the reference."""
     if format == "bam":
-        return readBam(input, sa, sq)
+        return readBam(input, sa, sq, params=bamParams)
     if format == "bed":
         return readBed(input, seqlevels, seqlengths)
     if format == "bigwig":
