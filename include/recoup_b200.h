@@ -320,6 +320,49 @@ int rcp_coverage_rle(int cov, int64_t first, int64_t count, int64_t* run_ptr_out
                      int32_t* values_out, int32_t* lengths_out, int64_t capacity);
 int rcp_coverage_free(int cov);
 
+/* ---------------------------------------------------------------- signal tracks ----------- */
+/* BigWig input (coverageFromBigWig, coverage.R:228-322: import.bw(file, as = "RleList")[[chr]]
+ * subscripted by the window like the reads path).
+ *
+ * rcp_bigwig_load  the whole file (UCSC bbi / bigWig, little-endian) -> a `signal` handle resident
+ *   in HBM.  The header and both trees are parsed on the host and the data blocks inflated there
+ *   (zlib; n_threads host threads, 0 = one per core); the inflated sections are then uploaded once,
+ *   expanded to items (start, end 1-based closed, float value) and validated on the device, with
+ *   one host synchronisation.  RCP_ERR_DATA (the message names the block and item) when: a magic
+ *   is wrong (a bigBed file says so), the file is truncated, a section's size disagrees with its
+ *   item count, the items of a chromosome are not sorted and disjoint, an item leaves
+ *   [1, chromSize], or a value is NaN or infinite.  A big-endian file is RCP_ERR_UNSUPPORTED.
+ *   Zoom levels are skipped.  -0.0 is stored as +0.0.
+ * rcp_signal_info    chromosomes, items, and the bytes rcp_signal_chroms needs for the names.
+ * rcp_signal_chroms  the chromosome names (NUL-terminated, back to back) and sizes, in chromId order.
+ * rcp_signal_fetch   the items (host arrays, any may be NULL) in (chromosome, start) order.
+ * rcp_signal_coverage  calcCoverage(<bigwig>, mask): element g owns ranges ptr[g]..ptr[g+1]-1
+ *   (ptr == NULL: one range per element, a GRanges mask).  chrom = ids into the track's
+ *   chromosomes, -1 = not in the track.  Per element the chromosome and strand are those of its
+ *   FIRST range (coverage.R:182,185); the vector is the track's value per base (0 between items)
+ *   at the element's positions in range order, reversed when that strand is '-'.  NULL when the
+ *   chromosome is not in the track, a range ends past chromSize or starts below 0 (R's subscript
+ *   errors), or the element has no position; a window no item overlaps is a zero vector, not
+ *   NULL.  end < start - 1 is RCP_ERR_DATA.  The result is an ordinary coverage handle of value
+ *   type FLOAT32.
+ * rcp_coverage_value_type  RCP_VALUE_INT32 (reads) or RCP_VALUE_FLOAT32 (signal tracks).  Every
+ *   consumer of a coverage handle accepts both (bins: fp64 sums of the float values; medians
+ *   exact); rcp_coverage_concat3 needs one type in all three.  rcp_coverage_fetch / _rle take
+ *   INT32 handles, the _f32 twins FLOAT32 handles (RCP_ERR_ARG otherwise). */
+#define RCP_VALUE_INT32 0
+#define RCP_VALUE_FLOAT32 1
+int rcp_bigwig_load(const uint8_t* data /* host */, int64_t n_bytes, int n_threads, int* signal_out);
+int rcp_signal_info(int signal, int* n_chrom, int64_t* n_items, int64_t* names_bytes);
+int rcp_signal_chroms(int signal, char* names /* NUL-terminated, back to back */, int64_t* chrom_len);
+int rcp_signal_fetch(int signal, int32_t* chrom, int32_t* start, int32_t* end, float* value, int64_t capacity);
+int rcp_signal_free(int signal);
+int rcp_signal_coverage(int signal, int64_t n_elements, const int64_t* ptr, const int32_t* chrom,
+                        const int32_t* start, const int32_t* end, const int8_t* strand, int mem, int* cov_out);
+int rcp_coverage_value_type(int cov, int* type);
+int rcp_coverage_fetch_f32(int cov, int64_t first, int64_t count, float* out, int64_t capacity);
+int rcp_coverage_rle_f32(int cov, int64_t first, int64_t count, int64_t* run_ptr_out,
+                         float* values_out, int32_t* lengths_out, int64_t capacity);
+
 /* ---------------------------------------------------------------- profile matrix ---------- */
 /* binCoverageMatrix(cvrg, binSize, stat, interpolation, flank, where) (profile.R:153-212) with
  * splitVector (util.R:15-85): writes an [n_regions x n_bins] block, column-major with leading

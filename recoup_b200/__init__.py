@@ -14,8 +14,8 @@ from .coverage import (CoverageList, DeviceReads, calcCoverage, coverageRef, cov
 from .preprocess import SelectedGRanges, preprocessRanges, readRanges, sampleSorted, widthQuantile
 from .profile import (ProfileMatrix, baseCoverageMatrix, binCoverageMatrix, coverageProfile,
                       haveEqualLengths, profileMatrix)
-from .readers import (DecodedGRanges, ScanBamParam, decodeBam, readBam, readBed, readRangesFile,
-                      scanBamFlag)
+from .readers import (BigWigTrack, DecodedGRanges, ScanBamParam, decodeBam, readBam, readBed, readBigWig,
+                      readRangesFile, scanBamFlag)
 from .ranges import GRanges, GRangesList, Rle, getFlankingRanges, getRegionalRanges
 
 __all__ = [
@@ -25,5 +25,5 @@ __all__ = [
     "haveEqualLengths", "coverageProfile", "ProfileMatrix", "set_verbose", "calcPlotProfiles", "orderProfiles",
     "heatmapScale", "colProfile", "rowStat", "sortIndex", "matrixQuantile", "preprocessRanges",
     "readRanges", "SelectedGRanges", "sampleSorted", "widthQuantile", "readBam", "readBed", "readRangesFile",
-    "decodeBam", "DecodedGRanges", "ScanBamParam", "scanBamFlag",
+    "decodeBam", "DecodedGRanges", "ScanBamParam", "scanBamFlag", "readBigWig", "BigWigTrack",
 ]

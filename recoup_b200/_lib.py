@@ -18,6 +18,7 @@ STAT = {"mean": 0, "median": 1}
 INTERP = {"auto": 0, "spline": 1, "linear": 2, "neighborhood": 3}
 SAMPLE_KIND = {"Rejection": 0, "Rounding": 1}
 COVERAGE_PATH = {"auto": 0, "index": 1, "buckets": 2, "blocks": 3, "split": 4}
+VALUE_INT32, VALUE_FLOAT32 = 0, 1
 
 _i32p = C.POINTER(C.c_int32)
 _i64p = C.POINTER(C.c_int64)
@@ -91,6 +92,15 @@ SIGNATURES = {
     "rcp_coverage_fetch": (C.c_int, [C.c_int, C.c_int64, C.c_int64, _i32p, C.c_int64]),
     "rcp_coverage_rle": (C.c_int, [C.c_int, C.c_int64, C.c_int64, _i64p, _i32p, _i32p, C.c_int64]),
     "rcp_coverage_free": (C.c_int, [C.c_int]),
+    "rcp_bigwig_load": (C.c_int, [_vp, C.c_int64, C.c_int, _ip]),
+    "rcp_signal_info": (C.c_int, [C.c_int, _ip, _i64p, _i64p]),
+    "rcp_signal_chroms": (C.c_int, [C.c_int, C.c_char_p, _i64p]),
+    "rcp_signal_fetch": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, C.c_int64]),
+    "rcp_signal_free": (C.c_int, [C.c_int]),
+    "rcp_signal_coverage": (C.c_int, [C.c_int, C.c_int64, _i64p, _vp, _vp, _vp, _vp, C.c_int, _ip]),
+    "rcp_coverage_value_type": (C.c_int, [C.c_int, _ip]),
+    "rcp_coverage_fetch_f32": (C.c_int, [C.c_int, C.c_int64, C.c_int64, _vp, C.c_int64]),
+    "rcp_coverage_rle_f32": (C.c_int, [C.c_int, C.c_int64, C.c_int64, _i64p, _vp, _i32p, C.c_int64]),
     "rcp_bin_matrix": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                  C.c_int, _vp, C.c_int64, C.c_int]),
     "rcp_base_matrix": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _vp, C.c_int64, C.c_int]),

@@ -8,10 +8,14 @@ Same names, argument meaning and error behaviour as the reference's closures:
 
 `rc` (fraction of cores for mclapply, util.R:364-382) is accepted and ignored: the per-region
 map runs as a CUDA grid.  All arithmetic happens in the CUDA library; this file only moves
-arrays across the C ABI.  BAM / BigWig file inputs (coverage.R:228-322) are file I/O and outside
-the scope of this path (SURVEY.md section 2, rows 9-10).
+arrays across the C ABI.  BigWig input (coverageFromBigWig, coverage.R:228-322) runs on the device
+too: the track is loaded with readers.readBigWig and painted into the windows by
+rcp_signal_coverage; its coverage holds float32 values.  BAM file paths stay outside this path:
+pass the decoded ranges (readers.readBam).
 """
 import ctypes as C
+import os
+import re
 import weakref
 
 import numpy as np
@@ -197,6 +201,10 @@ class CoverageList:
         self.n = n.value
         self.total_len = tot.value
         self.n_null = nn.value
+        vt = C.c_int(0)
+        _lib_check(_lib.lib.rcp_coverage_value_type(handle, C.byref(vt)))
+        # int32 read counts, or float32 track values (BigWig input)
+        self.dtype = np.dtype(np.float32) if vt.value == _lib.VALUE_FLOAT32 else np.dtype(np.int32)
         self._lengths = None
         self._fin = weakref.finalize(self, _free_cov, handle)
 
@@ -226,14 +234,18 @@ class CoverageList:
         return self.lengths() == 0
 
     def fetch(self, first=0, count=None):
-        """Unscaled integer coverage of regions [first, first+count) as a list (None = NULL)."""
+        """Unscaled coverage of regions [first, first+count) as a list (None = NULL), of `dtype`."""
         if count is None:
             count = self.n - first
         lens = self.lengths()[first:first + count].astype(np.int64)
         total = int(lens.sum())
-        buf = np.zeros(max(total, 1), dtype=np.int32)
-        _lib_check(_lib.lib.rcp_coverage_fetch(self.handle, first, count,
-                                               buf.ctypes.data_as(C.POINTER(C.c_int32)), total))
+        buf = np.zeros(max(total, 1), dtype=self.dtype)
+        if self.dtype == np.float32:
+            _lib_check(_lib.lib.rcp_coverage_fetch_f32(self.handle, first, count, buf.ctypes.data_as(C.c_void_p),
+                                                       total))
+        else:
+            _lib_check(_lib.lib.rcp_coverage_fetch(self.handle, first, count,
+                                                   buf.ctypes.data_as(C.POINTER(C.c_int32)), total))
         out, pos = [], 0
         for l in lens:
             l = int(l)
@@ -242,20 +254,23 @@ class CoverageList:
         return out
 
     def rle(self, first=0, count=None):
-        """Regions [first, first+count) as integer run-length encodings, the `Rle` objects
-        calcCoverage returns in the reference (coverage.R:171-173): a list of (values, lengths)
-        int32 array pairs, None for NULL.  Encoded on the device; only the runs are copied."""
+        """Regions [first, first+count) as run-length encodings, the `Rle` objects calcCoverage
+        returns in the reference (coverage.R:171-173): a list of (values, lengths) array pairs
+        (values of `dtype`, lengths int32), None for NULL.  Encoded on the device; only the runs
+        are copied."""
         if count is None:
             count = self.n - first
+        f32 = self.dtype == np.float32
+        rle = _lib.lib.rcp_coverage_rle_f32 if f32 else _lib.lib.rcp_coverage_rle
         ptr = np.zeros(count + 1, dtype=np.int64)
         pp = ptr.ctypes.data_as(C.POINTER(C.c_int64))
-        _lib_check(_lib.lib.rcp_coverage_rle(self.handle, first, count, pp, None, None, 0))
+        _lib_check(rle(self.handle, first, count, pp, None, None, 0))
         total = int(ptr[count])
-        vals = np.zeros(max(total, 1), dtype=np.int32)
+        vals = np.zeros(max(total, 1), dtype=self.dtype)
         lens = np.zeros(max(total, 1), dtype=np.int32)
         i32 = C.POINTER(C.c_int32)
-        _lib_check(_lib.lib.rcp_coverage_rle(self.handle, first, count, pp, vals.ctypes.data_as(i32),
-                                             lens.ctypes.data_as(i32), total))
+        _lib_check(rle(self.handle, first, count, pp, vals.ctypes.data if f32 else vals.ctypes.data_as(i32),
+                       lens.ctypes.data_as(i32), total))
         null = self.is_null()[first:first + count]
         return [None if null[i] else (vals[ptr[i]:ptr[i + 1]].copy(), lens[ptr[i]:ptr[i + 1]].copy())
                 for i in range(count)]
@@ -303,17 +318,54 @@ def _map_chrom(mask_gr, reads_gr):
     return table[mask_gr.seqnames]
 
 
+_BIGWIG_PATH = re.compile(r"\.(bigwig|bw)$", re.IGNORECASE)     # the reference's dispatch
+_BAD_INPUT = ("The input argument must be a GenomicRanges object or a valid "
+              "BAM/BigWig file or a list of GenomicRanges")                        # coverage.R:129
+
+
+def _signal_coverage(track, mask):
+    """rcp_signal_coverage of a BigWigTrack over a GRanges / GRangesList mask."""
+    h = C.c_int(0)
+    gr = mask.unlisted if isinstance(mask, GRangesList) else mask
+    chrom = np.ascontiguousarray(_map_chrom(gr, track), dtype=np.int32)     # -1: not in the track
+    start = np.ascontiguousarray(gr.start, dtype=np.int32)
+    end = np.ascontiguousarray(gr.end, dtype=np.int32)
+    strand = np.ascontiguousarray(gr.strand, dtype=np.int8)
+    ptr = None
+    if isinstance(mask, GRangesList):
+        ptr = np.ascontiguousarray(mask.ptr, dtype=np.int64).ctypes.data_as(C.POINTER(C.c_int64))
+    _lib_check(_lib.lib.rcp_signal_coverage(track.handle, len(mask), ptr, _ptr(chrom), _ptr(start), _ptr(end),
+                                            _ptr(strand), _lib.MEM_HOST, C.byref(h)))
+    return CoverageList(h.value, names=mask.names)
+
+
 def calcCoverage(input, mask, strand=None, ignore_strand=True, rc=None, frag_len=0):
-    """coverage.R:126-174.  Returns a CoverageList named by names(mask)."""
-    reads = _as_reads(input)
-    if reads is None:
+    """coverage.R:126-174.  Returns a CoverageList named by names(mask).  `input` may also be a
+    BigWigTrack or a path ending in .bigwig / .bw (coverageFromBigWig, coverage.R:228-322): the
+    coverage then holds the track's float32 values, and `strand` / `ignore_strand` have nothing to
+    act on (a bigWig has no strand)."""
+    from .readers import BigWigTrack, readBigWig
+    track, owned = None, False
+    if isinstance(input, BigWigTrack):
+        track = input
+    elif isinstance(input, str) and _BIGWIG_PATH.search(input):
+        if not os.path.isfile(input):
+            raise ValueError(_BAD_INPUT)
+        track, owned = readBigWig(input), True
+    reads = None if track is not None else _as_reads(input)
+    if reads is None and track is None:
         if isinstance(input, str):
-            raise NotImplementedError("BAM/BigWig file input (coverage.R:228-322) is file I/O, "
+            raise NotImplementedError("BAM file input (coverage.R:228-322) is file I/O, "
                                       "outside the accelerated path; pass decoded ranges")
-        raise ValueError("The input argument must be a GenomicRanges object or a valid "
-                         "BAM/BigWig file or a list of GenomicRanges")               # coverage.R:129
+        raise ValueError(_BAD_INPUT)
     if not isinstance(mask, (GRanges, GRangesList)):
         raise ValueError("The mask argument must be a GRanges or GRangesList object")  # coverage.R:132
+    if track is not None:
+        try:
+            return _signal_coverage(track, mask)
+        finally:
+            if owned:
+                track.free()
     if strand is not None:
         _message("Retrieving ", strand, " reads...")                                    # coverage.R:142
         strand_filter = int(strand_to_code(strand)[0])
@@ -378,12 +430,27 @@ def coverageRef(input, genomeRanges, region="tss", flank=(2000, 2000), strandedP
     mainRanges = getRegionalRanges(genomeRanges, region, flank)            # coverage.R:28,46
     for x in input:
         _message("Calculating ", region, " coverage for ", x.get("name"))
-        if x.get("ranges") is None:
-            raise NotImplementedError("sample %r has no decoded ranges; BAM/BigWig input is "
-                                      "outside the accelerated path" % (x.get("id"),))
+        track = _sample_track(x)
+        if track is not None:
+            x["coverage"] = calcCoverage(track, mainRanges)
+            track.free()
+            continue
         x["coverage"] = calcCoverage(x["ranges"], mainRanges, strand=strand, ignore_strand=ignore,
                                      rc=rc)
     return input
+
+
+def _sample_track(x):
+    """The BigWigTrack of a sample without reads whose format is "bigwig" (readRanges gives it
+    no ranges; the coverage comes from the file).  None for a sample with ranges; any other
+    sample without ranges is outside the accelerated path."""
+    if x.get("ranges") is not None:
+        return None
+    if x.get("format") == "bigwig" and x.get("file") is not None:
+        from .readers import readBigWig
+        return readBigWig(x["file"])
+    raise NotImplementedError("sample %r has no decoded ranges; BAM input is outside the accelerated "
+                              "path" % (x.get("id"),))
 
 
 def coverageRnaRef(input, genomeRanges, helperRanges, flank, strandedParams=None, bamParams=None,
@@ -397,14 +464,16 @@ def coverageRnaRef(input, genomeRanges, helperRanges, flank, strandedParams=None
     leftRanges = getFlankingRanges(helperRanges, 1 if f1 == 0 else f1, "upstream")
     rightRanges = getFlankingRanges(helperRanges, 1 if f1 == 0 else f2, "downstream")
     for x in input:
-        if x.get("ranges") is None:
-            raise NotImplementedError("sample %r has no decoded ranges" % (x.get("id"),))
+        track = _sample_track(x)            # one load serves the three passes
+        src = x["ranges"] if track is None else track
         _message("Calculating genebody coverage for ", x.get("name"))
-        center = calcCoverage(x["ranges"], genomeRanges, strand=strand, ignore_strand=ignore, rc=rc)
-        left = calcCoverage(x["ranges"], leftRanges, strand=strand, ignore_strand=ignore, rc=rc)
-        right = calcCoverage(x["ranges"], rightRanges, strand=strand, ignore_strand=ignore, rc=rc)
+        center = calcCoverage(src, genomeRanges, strand=strand, ignore_strand=ignore, rc=rc)
+        left = calcCoverage(src, leftRanges, strand=strand, ignore_strand=ignore, rc=rc)
+        right = calcCoverage(src, rightRanges, strand=strand, ignore_strand=ignore, rc=rc)
         x["coverage"] = _concat3(left, center, right, genomeRanges.names)   # coverage.R:115-121
         left.free()
         center.free()
         right.free()
+        if track is not None:
+            track.free()
     return input

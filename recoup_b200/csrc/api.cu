@@ -242,6 +242,7 @@ static void drop_coverage(int h) {
 
 // implemented in the other translation units
 void decoded_release_all();     // import.cu
+void signal_release_all();      // bigwig.cu
 int reads_load_impl(ReadsIdx& r, int64_t n, const int32_t* chrom, int64_t n_runs,
                     const int32_t* run_chrom, const int32_t* run_len, const int32_t* start,
                     const int32_t* end, const int8_t* strand, int n_chrom,
@@ -533,6 +534,7 @@ int rcp_shutdown(void) {
     for (auto& kv : g_covs) coverage_release(*kv.second);
     g_covs.clear();
     decoded_release_all();
+    signal_release_all();
     cache_release_all();
     g_big_live.clear();
     host_cache_release_all();
@@ -974,9 +976,12 @@ int rcp_coverage_concat3(int left, int center, int right, int* cov_out) {
     Coverage *a = get_coverage(left), *b = get_coverage(center), *c = get_coverage(right);
     if (!a || !b || !c) return fail(RCP_ERR_HANDLE, "unknown coverage handle");
     if (cov_out == nullptr) return fail(RCP_ERR_ARG, "cov_out is NULL");
+    if (a->value_type != b->value_type || b->value_type != c->value_type)
+        return fail(RCP_ERR_ARG, "concat3: the three coverages have different value types");
     Coverage* cv;
     int h;
     RCP_TRY(new_coverage(&cv, &h));
+    cv->value_type = b->value_type;
     int rc = coverage_concat3(*a, *b, *c, cv);
     if (rc != RCP_OK) {
         drop_coverage(h);
@@ -1031,7 +1036,24 @@ int rcp_coverage_fetch(int cov, int64_t first, int64_t count, int32_t* out, int6
     RCP_TRY(require_ready());
     Coverage* cv = get_coverage(cov);
     if (!cv) return fail(RCP_ERR_HANDLE, "unknown coverage handle %d", cov);
+    if (cv->value_type != RCP_VALUE_INT32) return fail(RCP_ERR_ARG, "rcp_coverage_fetch: a FLOAT32 coverage (use _f32)");
     return coverage_fetch(*cv, first, count, out, capacity);
+}
+
+int rcp_coverage_fetch_f32(int cov, int64_t first, int64_t count, float* out, int64_t capacity) {
+    RCP_TRY(require_ready());
+    Coverage* cv = get_coverage(cov);
+    if (!cv) return fail(RCP_ERR_HANDLE, "unknown coverage handle %d", cov);
+    if (cv->value_type != RCP_VALUE_FLOAT32) return fail(RCP_ERR_ARG, "rcp_coverage_fetch_f32: an INT32 coverage");
+    return coverage_fetch(*cv, first, count, reinterpret_cast<int32_t*>(out), capacity);
+}
+
+int rcp_coverage_value_type(int cov, int* type) {
+    Coverage* cv = get_coverage(cov);
+    if (!cv) return fail(RCP_ERR_HANDLE, "unknown coverage handle %d", cov);
+    if (type == nullptr) return fail(RCP_ERR_ARG, "type is NULL");
+    *type = cv->value_type;
+    return RCP_OK;
 }
 
 int rcp_coverage_rle(int cov, int64_t first, int64_t count, int64_t* run_ptr_out,
@@ -1039,7 +1061,20 @@ int rcp_coverage_rle(int cov, int64_t first, int64_t count, int64_t* run_ptr_out
     RCP_TRY(require_ready());
     Coverage* cv = get_coverage(cov);
     if (!cv) return fail(RCP_ERR_HANDLE, "unknown coverage handle %d", cov);
+    if (cv->value_type != RCP_VALUE_INT32) return fail(RCP_ERR_ARG, "rcp_coverage_rle: a FLOAT32 coverage (use _f32)");
     return coverage_rle(*cv, first, count, run_ptr_out, values_out, lengths_out, capacity);
+}
+
+// float runs: -0.0 is stored as +0.0, so equal bits are equal values and the integer run
+// encoding serves unchanged
+int rcp_coverage_rle_f32(int cov, int64_t first, int64_t count, int64_t* run_ptr_out, float* values_out,
+                         int32_t* lengths_out, int64_t capacity) {
+    RCP_TRY(require_ready());
+    Coverage* cv = get_coverage(cov);
+    if (!cv) return fail(RCP_ERR_HANDLE, "unknown coverage handle %d", cov);
+    if (cv->value_type != RCP_VALUE_FLOAT32) return fail(RCP_ERR_ARG, "rcp_coverage_rle_f32: an INT32 coverage");
+    return coverage_rle(*cv, first, count, run_ptr_out, reinterpret_cast<int32_t*>(values_out), lengths_out,
+                        capacity);
 }
 
 int rcp_coverage_free(int cov) {

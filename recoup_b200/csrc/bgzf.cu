@@ -60,6 +60,65 @@ int walk(const uint8_t* d, int64_t n, std::vector<Block>* blocks, int64_t* total
 }
 
 }  // namespace
+
+// The thread pool of every host inflate (BGZF members here, bigWig data blocks in bigwig.cu):
+// workers take 16 jobs at a time from a shared counter, one z_stream each.
+int64_t inflate_jobs(const uint8_t* data, InflateJob* jobs, int64_t n_jobs, uint8_t* out, int n_threads,
+                     int kind) {
+    unsigned nt = n_threads > 0 ? (unsigned)n_threads : std::thread::hardware_concurrency();
+    nt = std::max(1u, std::min<unsigned>(nt, (unsigned)std::max<int64_t>(n_jobs / 16, 1)));
+    std::atomic<int64_t> next{0};
+    std::atomic<int64_t> bad{-1};
+    auto work = [&]() {
+        z_stream z;
+        memset(&z, 0, sizeof z);
+        if (kind != INFLATE_COPY && inflateInit2(&z, kind == INFLATE_RAW_CRC ? -15 : 15) != Z_OK) {
+            bad.store(-2);
+            return;
+        }
+        for (;;) {
+            const int64_t i0 = next.fetch_add(16);      // 16 blocks (<= 1 MB of output) at a time
+            if (i0 >= n_jobs || bad.load() != -1) break;
+            for (int64_t i = i0; i < std::min<int64_t>(i0 + 16, n_jobs); i++) {
+                InflateJob& b = jobs[i];
+                bool ok;
+                if (kind == INFLATE_COPY) {
+                    ok = b.in_len <= (int64_t)b.out_cap;
+                    if (ok) {
+                        memcpy(out + b.out_off, data + b.in_off, (size_t)b.in_len);
+                        b.out_len = (uint32_t)b.in_len;
+                    }
+                } else {
+                    inflateReset(&z);
+                    z.next_in = const_cast<Bytef*>(data + b.in_off);
+                    z.avail_in = (uInt)b.in_len;
+                    z.next_out = out + b.out_off;
+                    z.avail_out = b.out_cap;
+                    if (kind == INFLATE_RAW_CRC) {
+                        const int rc = b.out_cap == 0 && b.in_len <= 2 ? Z_STREAM_END : inflate(&z, Z_FINISH);
+                        ok = (rc == Z_STREAM_END || (b.out_cap == 0 && rc == Z_BUF_ERROR)) && z.avail_out == 0 &&
+                             (uint32_t)crc32(crc32(0L, Z_NULL, 0), out + b.out_off, b.out_cap) == b.crc;
+                    } else {
+                        // a zlib stream that must end within out_cap bytes
+                        ok = inflate(&z, Z_FINISH) == Z_STREAM_END;
+                    }
+                    b.out_len = b.out_cap - z.avail_out;
+                }
+                if (!ok) {
+                    bad.store(i);
+                    break;
+                }
+            }
+        }
+        if (kind != INFLATE_COPY) inflateEnd(&z);
+    };
+    std::vector<std::thread> pool;
+    for (unsigned t = 1; t < nt; t++) pool.emplace_back(work);
+    work();
+    for (auto& th : pool) th.join();
+    return bad.load();
+}
+
 }  // namespace rcp
 
 using namespace rcp;
@@ -83,45 +142,18 @@ int rcp_bgzf_inflate(const uint8_t* data, int64_t n_bytes, uint8_t* out, int64_t
     RCP_TRY(walk(data, n_bytes, &blocks, &total));
     if (total > capacity)
         return fail(RCP_ERR_ARG, "rcp_bgzf_inflate: %lld inflated bytes, room for %lld", (long long)total, (long long)capacity);
-    unsigned nt = n_threads > 0 ? (unsigned)n_threads : std::thread::hardware_concurrency();
-    nt = std::max(1u, std::min<unsigned>(nt, (unsigned)std::max<size_t>(blocks.size() / 16, 1)));
-    std::atomic<size_t> next{0};
-    std::atomic<int64_t> bad{-1};
-    auto work = [&]() {
-        z_stream z;
-        memset(&z, 0, sizeof z);
-        if (inflateInit2(&z, -15) != Z_OK) {
-            bad.store(-2);
-            return;
-        }
-        for (;;) {
-            const size_t i0 = next.fetch_add(16);       // 16 blocks (<= 1 MB of output) at a time
-            if (i0 >= blocks.size() || bad.load() != -1) break;
-            for (size_t i = i0; i < std::min(i0 + 16, blocks.size()); i++) {
-                const Block& b = blocks[i];
-                inflateReset(&z);
-                z.next_in = const_cast<Bytef*>(data + b.in_off);
-                z.avail_in = (uInt)b.in_len;
-                z.next_out = out + b.out_off;
-                z.avail_out = b.out_len;
-                const int rc = b.out_len == 0 && b.in_len <= 2 ? Z_STREAM_END : inflate(&z, Z_FINISH);
-                const bool ok = (rc == Z_STREAM_END || (b.out_len == 0 && rc == Z_BUF_ERROR)) && z.avail_out == 0 &&
-                                (uint32_t)crc32(crc32(0L, Z_NULL, 0), out + b.out_off, b.out_len) == b.crc;
-                if (!ok) {
-                    bad.store((int64_t)i);
-                    break;
-                }
-            }
-        }
-        inflateEnd(&z);
-    };
-    std::vector<std::thread> pool;
-    for (unsigned t = 1; t < nt; t++) pool.emplace_back(work);
-    work();
-    for (auto& th : pool) th.join();
-    if (bad.load() == -2) return fail(RCP_ERR_CUDA, "rcp_bgzf_inflate: zlib could not be initialised");
-    if (bad.load() >= 0)
-        return fail(RCP_ERR_DATA, "BGZF: block %lld does not inflate to its ISIZE / CRC32", (long long)bad.load());
+    std::vector<InflateJob> jobs(blocks.size());
+    for (size_t i = 0; i < blocks.size(); i++) {
+        jobs[i].in_off = blocks[i].in_off;
+        jobs[i].in_len = blocks[i].in_len;
+        jobs[i].out_off = blocks[i].out_off;
+        jobs[i].out_cap = blocks[i].out_len;
+        jobs[i].crc = blocks[i].crc;
+    }
+    const int64_t bad = inflate_jobs(data, jobs.data(), (int64_t)jobs.size(), out, n_threads, INFLATE_RAW_CRC);
+    if (bad == -2) return fail(RCP_ERR_CUDA, "rcp_bgzf_inflate: zlib could not be initialised");
+    if (bad >= 0)
+        return fail(RCP_ERR_DATA, "BGZF: block %lld does not inflate to its ISIZE / CRC32", (long long)bad);
     return RCP_OK;
 }
 

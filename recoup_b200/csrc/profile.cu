@@ -8,9 +8,15 @@
 //   interp_kernel        regions shorter than the bin count (util.R:17-73): fmm spline or
 //                        neighbourhood fill, one warp per flagged region
 //   base_matrix_kernel   per-base matrix: int32 -> fp64 tiled transpose (profile.R:100-151)
+//
+// Every kernel that reads coverage values is a template on the value type V of the handle:
+// int32_t (reads: 64-bit integer sums) or float (signal tracks: fp64 sums; the words hold float
+// bits).  The helpers below are the only places the two differ; for int32_t they are the casts
+// the kernels always used.
 
 #include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 
 #include "r_rng.cuh"
 #include "rcp_internal.cuh"
@@ -21,6 +27,55 @@ namespace {
 
 constexpr int CTA = 256;
 constexpr int WARPS = CTA / 32;
+
+template <class V>
+struct Val;
+template <>
+struct Val<int32_t> {
+    using Sum = long long;
+    using Key = int;                                    // median bisection over the values
+    static constexpr int KEY_MIN = -0x7fffffff - 1, KEY_MAX = 0x7fffffff;
+};
+template <>
+struct Val<float> {
+    using Sum = double;
+    using Key = unsigned;                               // order-preserving key of the float
+    static constexpr unsigned KEY_MIN = 0u, KEY_MAX = 0xffffffffu;
+};
+// a staged word -> its term in a sum
+template <class V>
+__device__ __forceinline__ typename Val<V>::Sum word_sum(uint32_t w) {
+    if constexpr (std::is_same<V, float>::value) return (double)__uint_as_float(w);
+    else return (long long)w;
+}
+// a loaded word -> its value (int stays int)
+template <class V>
+__device__ __forceinline__ auto word_val(int w) {
+    if constexpr (std::is_same<V, float>::value) return (double)__int_as_float(w);
+    else return w;
+}
+template <class V>
+__device__ __forceinline__ double word_double(int w) {
+    if constexpr (std::is_same<V, float>::value) return (double)__int_as_float(w);
+    else return (double)w;
+}
+// median keys: the value itself for int32; for float the bits with the sign flipped (positive)
+// or all bits flipped (negative), so that unsigned order is float order (-0.0 never occurs)
+template <class V>
+__device__ __forceinline__ typename Val<V>::Key word_key(int w) {
+    if constexpr (std::is_same<V, float>::value) {
+        const unsigned u = (unsigned)w;
+        return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+    } else {
+        return w;
+    }
+}
+template <class V>
+__device__ __forceinline__ double key_double(typename Val<V>::Key k) {
+    if constexpr (std::is_same<V, float>::value)
+        return (double)__uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+    else return (double)k;
+}
 
 struct Seg {
     int a, b;   // [a, b) inside the region's coverage vector
@@ -82,7 +137,9 @@ __device__ __forceinline__ long long warp_range_sum(const int32_t* __restrict__ 
 }
 
 // Median bins (sumStat = "median"): one CTA per region.  dynamic smem: edges[n + 1].
+template <class V>
 __global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
+    using K = typename Val<V>::Key;
     extern __shared__ __align__(16) int sh[];
     int* edges = sh;                    // n + 1
     __shared__ int wcount[WARPS];
@@ -145,9 +202,9 @@ __global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
         const int lo = ok ? edges[i] : 0, hi = ok ? edges[i + 1] : 0;
         const int cnt = hi - lo;
         // k-th smallest = least v with #{x <= v} >= k+1
-        int vmin = 0x7fffffff, vmax = -0x7fffffff - 1;
+        K vmin = Val<V>::KEY_MAX, vmax = Val<V>::KEY_MIN;
         for (int q = lo + li; q < hi; q += g) {
-            const int v = __ldg(src + q);
+            const K v = word_key<V>(__ldg(src + q));
             vmin = min(vmin, v);
             vmax = max(vmax, v);
         }
@@ -156,19 +213,19 @@ __global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
             vmax = max(vmax, __shfl_xor_sync(0xffffffffu, vmax, d));
         }
         const int k1 = (cnt - 1) / 2, k2 = cnt / 2;
-        int res[2];
+        K res[2];
 #pragma unroll
         for (int t = 0; t < 2; t++) {
             const int k = t == 0 ? k1 : k2;
-            int a = vmin, b = vmax;          // answer in [a, b]
+            K a = vmin, b = vmax;            // answer in [a, b]
             // every lane of the WARP iterates the same number of times (the shuffles are
             // warp-wide): bound by the warp-wide maximum range
-            int span = ok ? (b - a) : 0;
+            K span = ok ? (b - a) : 0;
             for (int d = 16; d > 0; d >>= 1) span = max(span, __shfl_xor_sync(0xffffffffu, span, d));
             while (span > 0) {
-                const int mid = a + ((b - a) >> 1);
+                const K mid = a + ((b - a) >> 1);
                 int c = 0;
-                for (int q = lo + li; q < hi; q += g) c += (__ldg(src + q) <= mid);
+                for (int q = lo + li; q < hi; q += g) c += (word_key<V>(__ldg(src + q)) <= mid);
                 for (int d = g >> 1; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
                 if (a < b) {
                     if (c >= k + 1) b = mid;
@@ -179,7 +236,7 @@ __global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
             res[t] = a;
         }
         if (ok && li == 0)
-            out[(int64_t)i * p.ld] = p.scale * (((double)res[0] + (double)res[1]) * 0.5);
+            out[(int64_t)i * p.ld] = p.scale * ((key_double<V>(res[0]) + key_double<V>(res[1])) * 0.5);
     }
 }
 
@@ -293,8 +350,10 @@ __device__ __forceinline__ BinDesc load_bin_desc(const BinDesc* __restrict__ p) 
 // to the interpolation list (util.R:17).
 constexpr int NBUF_MAX = 8;
 
+template <class V>
 __global__ void __launch_bounds__(BT)
 bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_ints, int nbuf) {
+    using S = typename Val<V>::Sum;
     extern __shared__ __align__(16) int sh[];
     int* edges = sh;                                         // n + 1 (unequal bins only)
     uint32_t* bufs = reinterpret_cast<uint32_t*>(sh + ((p.n + 1 + 3) & ~3));
@@ -409,7 +468,7 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
                     const int part = tid & (g - 1);
                     for (int b0 = bin0; b0 < bin1; b0 += BT / g) {      // whole warps stay together
                         const int b = b0 + tid / g;
-                        long long s64 = 0;
+                        S s64 = 0;
                         int eb0 = 0, eb1 = 1;
                         if (b < bin1) {
                             eb0 = edge(b);
@@ -418,12 +477,12 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
                             const int share = (blen + g - 1) / g;
                             int q = eb0 - lo_al + part * share;
                             const int qe = min(q + share, eb1 - lo_al);
-                            while (q < qe && (q & 3)) s64 += (long long)stage[q++];
+                            while (q < qe && (q & 3)) s64 += word_sum<V>(stage[q++]);
                             for (; q + 4 <= qe; q += 4) {
                                 const uint4 x = *reinterpret_cast<const uint4*>(stage + q);
-                                s64 += ((long long)x.x + x.y) + ((long long)x.z + x.w);
+                                s64 += (word_sum<V>(x.x) + word_sum<V>(x.y)) + (word_sum<V>(x.z) + word_sum<V>(x.w));
                             }
-                            while (q < qe) s64 += (long long)stage[q++];
+                            while (q < qe) s64 += word_sum<V>(stage[q++]);
                         }
                         for (int dd = g >> 1; dd > 0; dd >>= 1) s64 += __shfl_xor_sync(0xffffffffu, s64, dd);
                         if (b < bin1 && part == 0)
@@ -441,7 +500,7 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
                 if (i0 < i1) {
                     const int lo = edge(i0), hi = edge(i1);
                     int k = i0, nxt = edge(i0 + 1);
-                    long long acc = 0;
+                    S acc = 0;
                     constexpr int UW = 4;
                     for (int q0 = lo & ~3; q0 < hi; q0 += 128 * UW) {
                         int4 x[UW];
@@ -456,19 +515,20 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
                             const int row = q0 + u * 128;
                             if (row >= hi) break;
                             const int q = row + lane * 4;
-                            int a0 = x[u].x, a1 = x[u].y, a2 = x[u].z, a3 = x[u].w;
+                            auto a0 = word_val<V>(x[u].x), a1 = word_val<V>(x[u].y), a2 = word_val<V>(x[u].z),
+                                 a3 = word_val<V>(x[u].w);
                             if (row < lo || row + 128 > hi) {           // first / last row of the run
                                 a0 = (q >= lo && q < hi) ? a0 : 0;
                                 a1 = (q + 1 >= lo && q + 1 < hi) ? a1 : 0;
                                 a2 = (q + 2 >= lo && q + 2 < hi) ? a2 : 0;
                                 a3 = (q + 3 >= lo && q + 3 < hi) ? a3 : 0;
                             }
-                            const long long tot = ((long long)a0 + a1) + ((long long)a2 + a3);
+                            const S tot = ((S)a0 + a1) + ((S)a2 + a3);
                             if (row + 128 >= nxt) {                     // this row ends the current bin
                                 const int c = nxt - q;                  // this lane's elements before the edge
-                                const long long before = (long long)(c > 0 ? a0 : 0) + (c > 1 ? a1 : 0) +
-                                                         (c > 2 ? a2 : 0) + (c > 3 ? a3 : 0);
-                                long long t = acc + before;
+                                const S before = (S)(c > 0 ? a0 : 0) + (c > 1 ? a1 : 0) +
+                                                 (c > 2 ? a2 : 0) + (c > 3 ? a3 : 0);
+                                S t = acc + before;
 #pragma unroll
                                 for (int dd = 16; dd > 0; dd >>= 1) t += __shfl_xor_sync(0xffffffffu, t, dd);
                                 const int b0 = edge(k);
@@ -498,9 +558,11 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
 // once per bin.  Bin i has bsz + [rank[i] <= dif] elements (util.R:74-80).
 constexpr int WIDE_RUN = 16;
 
+template <class V>
 __global__ void __launch_bounds__(BT, 3)
 bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __restrict__ long_list,
                 unsigned int* __restrict__ long_count) {
+    using S = typename Val<V>::Sum;
     const int lane = threadIdx.x & 31;
     const int n = p.n;
     const int runs = (n + WIDE_RUN - 1) / WIDE_RUN;
@@ -531,7 +593,7 @@ bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __re
         const int32_t* src = p.cov + (int64_t)(((uint64_t)(uint32_t)d.off_hi << 32) | (uint32_t)d.off_lo);
         double* out = p.out + r;
         int k = i0, b0 = lo, nxt = lo + bsz + (int)(extra & 1u);
-        long long acc = 0;
+        S acc = 0;
         constexpr int UW = 4;
         // the rows of the NEXT trip are requested before this trip's rows are summed
         auto fetch = [&](int q0, int4* x) {
@@ -551,19 +613,20 @@ bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __re
                 const int row = q0 + v * 128;
                 if (row >= hi) break;
                 const int q = row + lane * 4;
-                int a0 = x[v].x, a1 = x[v].y, a2 = x[v].z, a3 = x[v].w;
+                auto a0 = word_val<V>(x[v].x), a1 = word_val<V>(x[v].y), a2 = word_val<V>(x[v].z),
+                     a3 = word_val<V>(x[v].w);
                 if (row < lo || row + 128 > hi) {           // first / last row of the run
                     a0 = (q >= lo && q < hi) ? a0 : 0;
                     a1 = (q + 1 >= lo && q + 1 < hi) ? a1 : 0;
                     a2 = (q + 2 >= lo && q + 2 < hi) ? a2 : 0;
                     a3 = (q + 3 >= lo && q + 3 < hi) ? a3 : 0;
                 }
-                const long long tot = ((long long)a0 + a1) + ((long long)a2 + a3);
+                const S tot = ((S)a0 + a1) + ((S)a2 + a3);
                 if (row + 128 >= nxt) {                     // this row ends the current bin
                     const int c = nxt - q;                  // this lane's elements before the edge
-                    const long long before = (long long)(c > 0 ? a0 : 0) + (c > 1 ? a1 : 0) +
-                                             (c > 2 ? a2 : 0) + (c > 3 ? a3 : 0);
-                    long long t = acc + before;
+                    const S before = (S)(c > 0 ? a0 : 0) + (c > 1 ? a1 : 0) +
+                                     (c > 2 ? a2 : 0) + (c > 3 ? a3 : 0);
+                    S t = acc + before;
 #pragma unroll
                     for (int dd = 16; dd > 0; dd >>= 1) t += __shfl_xor_sync(0xffffffffu, t, dd);
                     if (lane == 0) out[(int64_t)k * p.ld] = p.scale * ((double)t / (double)(nxt - b0));
@@ -596,6 +659,7 @@ struct InterpArgs {
 };
 
 // dynamic smem per warp-CTA: 4n doubles + 2n ints + RRng
+template <class V>
 __global__ void __launch_bounds__(32) interp_kernel(InterpArgs p) {
     extern __shared__ double shd[];
     const int n = p.n;
@@ -613,7 +677,7 @@ __global__ void __launch_bounds__(32) interp_kernel(InterpArgs p) {
         const int L_all = p.len[r];
         const Seg sg = segment_of(L_all, p.where, p.f1, p.f2);
         const int L = sg.b - sg.a;
-        const int32_t* src = p.cov + p.off[r] + sg.a;
+        const V* src = reinterpret_cast<const V*>(p.cov) + p.off[r] + sg.a;
         double* out = p.out + r;
         __syncwarp();
         bool neighborhood = p.interp == RCP_INTERP_NEIGHBORHOOD;
@@ -744,6 +808,7 @@ struct BaseArgs {
     int64_t ld;
 };
 
+template <class V>
 __global__ void __launch_bounds__(256) base_matrix_kernel(BaseArgs p) {
     __shared__ int tile[32][33];
     __shared__ int64_t r_off[32];
@@ -775,7 +840,7 @@ __global__ void __launch_bounds__(256) base_matrix_kernel(BaseArgs p) {
     __syncthreads();
     for (int jj = ty; jj < 32; jj += 8) {
         const int64_t k = k0 + jj, r = r0 + tx;
-        if (r < p.R && k < p.n_cols) p.out[k * p.ld + r] = p.scale * (double)tile[tx][jj];
+        if (r < p.R && k < p.n_cols) p.out[k * p.ld + r] = p.scale * word_double<V>(tile[tx][jj]);
     }
 }
 
@@ -785,6 +850,7 @@ __global__ void __launch_bounds__(256) base_matrix_kernel(BaseArgs p) {
 // stores.  The tile index runs along x (linear, no 65535 limit).
 constexpr int BW_ROWS = 32, BW_COLS = 256;
 
+template <class V>
 __global__ void __launch_bounds__(256) base_matrix_wide_kernel(BaseArgs p, int64_t col_tiles,
                                                                int vec_store) {
     __shared__ int tile[BW_ROWS][BW_COLS + 1];
@@ -836,21 +902,19 @@ __global__ void __launch_bounds__(256) base_matrix_wide_kernel(BaseArgs p, int64
         // lanes 0..15 write column c, lanes 16..31 column c + 1; each lane two regions (16 bytes)
         const int rr = (lane & 15) * 2, dc = lane >> 4;
         for (int c = warp * 2 + dc; c < ncol; c += 16) {
-            const double2 v = make_double2(p.scale * (double)tile[rr][c], p.scale * (double)tile[rr + 1][c]);
+            const double2 v = make_double2(p.scale * word_double<V>(tile[rr][c]), p.scale * word_double<V>(tile[rr + 1][c]));
             *reinterpret_cast<double2*>(p.out + (k0 + c) * p.ld + r0 + rr) = v;
         }
     } else {
         const int64_t r = r0 + lane;
         if (r < p.R)
-            for (int c = warp; c < ncol; c += 8) p.out[(k0 + c) * p.ld + r] = p.scale * (double)tile[lane][c];
+            for (int c = warp; c < ncol; c += 8) p.out[(k0 + c) * p.ld + r] = p.scale * word_double<V>(tile[lane][c]);
     }
 }
 
-}  // namespace
-
-// out points to DEVICE memory here; the api layer stages host outputs.
-int bin_matrix_device(const Coverage& cv, int where, int f1, int f2, int n_bins, int stat,
-                      int interp, int seed, int sample_kind, double* d_out, int64_t ld) {
+template <class V>
+int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, int stat,
+                    int interp, int seed, int sample_kind, double* d_out, int64_t ld) {
     const int64_t R = cv.n_regions;
     if (R == 0) return RCP_OK;
     // rank table of `set.seed(seed); sample(1:n, n)` (host, n is small)
@@ -897,9 +961,9 @@ int bin_matrix_device(const Coverage& cv, int where, int f1, int f2, int n_bins,
         StageTimer t(ST_PROF_BIN);
         const size_t smem = edge_bytes;
         if (smem > 48 * 1024)
-            RCP_CUDA(cudaFuncSetAttribute(bin_median_kernel,
+            RCP_CUDA(cudaFuncSetAttribute(bin_median_kernel<V>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        bin_median_kernel<<<(unsigned)R, CTA, smem, g_ctx.stream>>>(a);
+        bin_median_kernel<V><<<(unsigned)R, CTA, smem, g_ctx.stream>>>(a);
         RCP_LAUNCHED();
     } else {
         // two staging buffers per CTA; the kernel is persistent (one resident wave of CTAs)
@@ -940,16 +1004,16 @@ int bin_matrix_device(const Coverage& cv, int where, int f1, int f2, int n_bins,
         nbuf = (int)((budget - edge_bytes) / ((size_t)buf_ints * sizeof(int)));
         nbuf = std::max(1, std::min(nbuf, NBUF_MAX));
         const size_t smem = edge_bytes + (size_t)nbuf * buf_ints * sizeof(int);
-        RCP_CUDA(cudaFuncSetAttribute(bin_mean_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        RCP_CUDA(cudaFuncSetAttribute(bin_mean_kernel<V>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)smem));
         int fit = 0;
-        RCP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, bin_mean_kernel, BT, smem));
+        RCP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, bin_mean_kernel<V>, BT, smem));
         if (fit < 1) return fail(RCP_ERR_UNSUPPORTED, "bin kernel does not fit (%zu bytes of shared memory)", smem);
         const int64_t grid = std::min<int64_t>(R, (int64_t)g_ctx.sm_count * std::min(fit, per_sm));
-        bin_mean_kernel<<<(unsigned)grid, BT, smem, g_ctx.stream>>>(a, d_desc, R, buf_ints, nbuf);
+        bin_mean_kernel<V><<<(unsigned)grid, BT, smem, g_ctx.stream>>>(a, d_desc, R, buf_ints, nbuf);
         RCP_LAUNCHED();
         // (nothing to do when no region is long: the warps find zero units)
-        bin_wide_kernel<<<(unsigned)(g_ctx.sm_count * 8), BT, 0, g_ctx.stream>>>(a, d_desc, long_list, long_count);
+        bin_wide_kernel<V><<<(unsigned)(g_ctx.sm_count * 8), BT, 0, g_ctx.stream>>>(a, d_desc, long_list, long_count);
         RCP_LAUNCHED();
     }
     InterpArgs ia;
@@ -972,13 +1036,13 @@ int bin_matrix_device(const Coverage& cv, int where, int f1, int f2, int n_bins,
     if (ismem > 220 * 1024)
         return fail(RCP_ERR_UNSUPPORTED, "interpolation supports at most ~5500 bins per segment");
     if (ismem > 48 * 1024)
-        RCP_CUDA(cudaFuncSetAttribute(interp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        RCP_CUDA(cudaFuncSetAttribute(interp_kernel<V>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)ismem));
     int iblocks = g_ctx.sm_count * 8;
     if ((int64_t)iblocks > R) iblocks = (int)R;
     {
         StageTimer t(ST_PROF_INTERP);
-        interp_kernel<<<(unsigned)iblocks, 32, ismem, g_ctx.stream>>>(ia);
+        interp_kernel<V><<<(unsigned)iblocks, 32, ismem, g_ctx.stream>>>(ia);
         RCP_LAUNCHED();
     }
     dfree(d_desc);
@@ -990,8 +1054,9 @@ int bin_matrix_device(const Coverage& cv, int where, int f1, int f2, int n_bins,
     return RCP_OK;
 }
 
-int base_matrix_device(const Coverage& cv, int where, int f1, int f2, int64_t n_cols,
-                       double* d_out, int64_t ld) {
+template <class V>
+int base_matrix_impl(const Coverage& cv, int where, int f1, int f2, int64_t n_cols,
+                     double* d_out, int64_t ld) {
     const int64_t R = cv.n_regions;
     if (R == 0 || n_cols == 0) return RCP_OK;
     BaseArgs a;
@@ -1013,7 +1078,7 @@ int base_matrix_device(const Coverage& cv, int where, int f1, int f2, int64_t n_
         const int64_t col_tiles = (n_cols + BW_COLS - 1) / BW_COLS, row_tiles = (R + BW_ROWS - 1) / BW_ROWS;
         if (col_tiles * row_tiles <= 0x7fffffff) {
             const int vec = ((ld & 1) == 0) && ((reinterpret_cast<uintptr_t>(d_out) & 15u) == 0);
-            base_matrix_wide_kernel<<<(unsigned)(col_tiles * row_tiles), 256, 0, g_ctx.stream>>>(
+            base_matrix_wide_kernel<V><<<(unsigned)(col_tiles * row_tiles), 256, 0, g_ctx.stream>>>(
                 a, col_tiles, vec);
             RCP_LAUNCHED();
             return RCP_OK;
@@ -1031,14 +1096,30 @@ int base_matrix_device(const Coverage& cv, int where, int f1, int f2, int64_t n_
             s.R = (R - rows0) < 65535 * 32 ? (R - rows0) : 65535 * 32;
             s.out = a.out + rows0;
             const int64_t gys = (s.R + 31) / 32;
-            base_matrix_kernel<<<dim3((unsigned)gx, (unsigned)gys), dim3(32, 8), 0, g_ctx.stream>>>(s);
+            base_matrix_kernel<V><<<dim3((unsigned)gx, (unsigned)gys), dim3(32, 8), 0, g_ctx.stream>>>(s);
             RCP_LAUNCHED();
         }
     } else {
-        base_matrix_kernel<<<dim3((unsigned)gx, (unsigned)gy), dim3(32, 8), 0, g_ctx.stream>>>(a);
+        base_matrix_kernel<V><<<dim3((unsigned)gx, (unsigned)gy), dim3(32, 8), 0, g_ctx.stream>>>(a);
         RCP_LAUNCHED();
     }
     return RCP_OK;
+}
+
+}  // namespace
+
+// out points to DEVICE memory here; the api layer stages host outputs.
+int bin_matrix_device(const Coverage& cv, int where, int f1, int f2, int n_bins, int stat,
+                      int interp, int seed, int sample_kind, double* d_out, int64_t ld) {
+    if (cv.value_type == RCP_VALUE_FLOAT32)
+        return bin_matrix_impl<float>(cv, where, f1, f2, n_bins, stat, interp, seed, sample_kind, d_out, ld);
+    return bin_matrix_impl<int32_t>(cv, where, f1, f2, n_bins, stat, interp, seed, sample_kind, d_out, ld);
+}
+
+int base_matrix_device(const Coverage& cv, int where, int f1, int f2, int64_t n_cols,
+                       double* d_out, int64_t ld) {
+    if (cv.value_type == RCP_VALUE_FLOAT32) return base_matrix_impl<float>(cv, where, f1, f2, n_cols, d_out, ld);
+    return base_matrix_impl<int32_t>(cv, where, f1, f2, n_cols, d_out, ld);
 }
 
 }  // namespace rcp

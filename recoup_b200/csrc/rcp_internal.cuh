@@ -160,6 +160,24 @@ struct DevIn {
     ~DevIn() { dfree(owned); }
 };
 
+// ------------------------------------------------------------------ host inflate -----------
+// One compressed block of a file: in_len bytes at data + in_off inflate to at most out_cap bytes
+// at out + out_off; out_len receives the inflated size.
+struct InflateJob {
+    int64_t in_off = 0, in_len = 0, out_off = 0;
+    uint32_t out_cap = 0, out_len = 0;
+    uint32_t crc = 0;       // INFLATE_RAW_CRC: the CRC32 of the out_cap inflated bytes
+};
+enum {
+    INFLATE_RAW_CRC = 0,    // raw deflate that fills out_cap exactly, CRC32 checked (BGZF)
+    INFLATE_ZLIB = 1,       // zlib stream of at most out_cap bytes (bigWig data blocks)
+    INFLATE_COPY = 2        // stored bytes, copied (bigWig files written uncompressed)
+};
+// Runs the jobs on n_threads host threads (0: one per core).  Returns -1 when every job
+// succeeded, -2 when zlib could not be initialised, else the index of a failed job.
+int64_t inflate_jobs(const uint8_t* data, InflateJob* jobs, int64_t n_jobs, uint8_t* out, int n_threads,
+                     int kind);
+
 // ------------------------------------------------------------------ reads index ------------
 // Strand classes of the sorted arrays.  ALL is used when no strand restriction applies.
 enum { CLS_ALL = 0, CLS_PLUS = 1, CLS_MINUS = 2, CLS_STAR = 3, CLS_N = 4 };
@@ -279,7 +297,8 @@ struct Coverage {
     unsigned long long* d_stats = nullptr;   // [0] n_null [1] total_len [2] max_len [3] candidates
     bool stats_pending = false;
     double scale = 1.0;
-    int32_t* cov = nullptr;      // dense int32, region r at [off[r], off[r] + len[r])
+    int value_type = RCP_VALUE_INT32;   // RCP_VALUE_FLOAT32: `cov` holds float bits (signal tracks)
+    int32_t* cov = nullptr;      // dense 4-byte words, region r at [off[r], off[r] + len[r])
     int64_t* off = nullptr;      // n_regions + 1, multiples of 32 ints
     int32_t* len = nullptr;      // n_regions, 0 for NULL
     uint8_t* is_null = nullptr;  // n_regions

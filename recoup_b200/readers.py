@@ -3,6 +3,7 @@
 
     readBam(bam, sa = c("keep", "remove", "split"), sq = 0.75)        ranges.R:111-134
     readBed(bed, bg)                                                  ranges.R:136-146
+    readBigWig(bw)                  import.bw(bw) of coverageFromBigWig, coverage.R:228-322
 
 What stays on the host: opening the file, the BGZF inflate (rcp_bgzf_inflate: zlib, one thread per
 core, C++ inside the library), the BAM header (text + reference list) and the walk of the
@@ -10,7 +11,9 @@ length-prefixed record chain (rcp_bam_index, also inside the library).  Everythi
 filter and the other ScanBamParam filters, CIGAR walk, N-split, trim, text parsing, compaction in file
 order (or in `which` order) -- runs on the device (rcp_bam_decode[_param] / rcp_bed_decode); the decoded reads stay in
 HBM and go to the hot path without a host round trip (rcp_reads_load_decoded).  Their coordinates
-are copied to the host only when somebody reads them.
+are copied to the host only when somebody reads them.  A bigWig track is parsed and inflated on the
+host (rcp_bigwig_load, threads inside the library) and expanded into items on the device; its items
+stay in HBM behind a `signal` handle.
 """
 import ctypes as C
 import gzip
@@ -290,8 +293,61 @@ def readBed(bed, seqlevels, seqlengths=None):
     return DecodedGRanges(h.value, n_out.value, seqlevels, seqlengths)
 
 
+def _free_signal(h):
+    try:
+        _lib.lib.rcp_signal_free(h)
+    except Exception:
+        pass
+
+
+class BigWigTrack:
+    """A bigWig track resident on the device (a `signal` handle): its items are the runs of
+    import.bw(file, as = "RleList") that are not zero -- start, end (1-based, closed) and a float32
+    value.  `seqlevels` / `seqlengths` are the file's chromosomes in chromId order."""
+
+    def __init__(self, handle):
+        self.handle = int(handle)
+        self._fin = weakref.finalize(self, _free_signal, self.handle)
+        n_chrom, n_items, nb = C.c_int(0), C.c_int64(0), C.c_int64(0)
+        _lib.check(_lib.lib.rcp_signal_info(self.handle, C.byref(n_chrom), C.byref(n_items), C.byref(nb)))
+        names = C.create_string_buffer(max(nb.value, 1))
+        lens = np.zeros(max(n_chrom.value, 1), dtype=np.int64)
+        _lib.check(_lib.lib.rcp_signal_chroms(self.handle, names, lens.ctypes.data_as(C.POINTER(C.c_int64))))
+        raw = names.raw[:nb.value]
+        self.seqlevels = [x.decode("utf-8", "replace") for x in raw.split(b"\0")[:n_chrom.value]]
+        self.seqlengths = lens[:n_chrom.value].copy()
+        self._n = n_items.value
+
+    def __len__(self):
+        return self._n
+
+    def fetch(self):
+        """(chrom ids, start, end, value) of every item, in (chromosome, start) order."""
+        n = self._n
+        chrom, start, end = (np.zeros(max(n, 1), dtype=np.int32) for _ in range(3))
+        value = np.zeros(max(n, 1), dtype=np.float32)
+        p = lambda a: a.ctypes.data_as(C.c_void_p)
+        _lib.check(_lib.lib.rcp_signal_fetch(self.handle, p(chrom), p(start), p(end), p(value), n))
+        return chrom[:n], start[:n], end[:n], value[:n]
+
+    def free(self):
+        self._fin()
+
+
+def readBigWig(bw, threads=0):
+    """import.bw(bw) of the whole file (coverage.R:228-322) -> BigWigTrack.  `bw`: a path, or
+    the bytes of the file; `threads`: host threads of the inflate (0 = one per core)."""
+    _lib.ensure_init()
+    data = bw if isinstance(bw, (bytes, bytearray, memoryview)) else open(bw, "rb").read()
+    buf = np.frombuffer(bytes(data) if isinstance(data, memoryview) else data, dtype=np.uint8)
+    h = C.c_int(0)
+    _lib.check(_lib.lib.rcp_bigwig_load(buf.ctypes.data_as(C.c_void_p), buf.shape[0], int(threads), C.byref(h)))
+    return BigWigTrack(h.value)
+
+
 def readRangesFile(input, format, sa="keep", sq=0.75, seqlevels=None, seqlengths=None, bamParams=None):
-    """readRanges (ranges.R:102-109) for files; "bigwig" has no reads (NULL).  `bamParams` (a
+    """readRanges (ranges.R:102-109) for files; "bigwig" has no reads (NULL: coverageRef reads the
+    track itself from the sample's `file`, see readBigWig).  `bamParams` (a
     ScanBamParam) applies to BAM files only, as in the reference."""
     if format == "bam":
         return readBam(input, sa, sq, params=bamParams)
