@@ -359,6 +359,11 @@ int rcp_signal_free(int signal);
 int rcp_signal_coverage(int signal, int64_t n_elements, const int64_t* ptr, const int32_t* chrom,
                         const int32_t* start, const int32_t* end, const int8_t* strand, int mem, int* cov_out);
 int rcp_coverage_value_type(int cov, int* type);
+/* rcp_coverage_storage_bytes  2 or 4: the bytes per stored element of an INT32 handle.  The split
+ *   path stores uint16 counts when no tile of the call can exceed 65 535 (environment variable
+ *   RCP_COVERAGE_WIDE set: always 4); fetch, RLE and every consumer see the same int32 values
+ *   either way.  May synchronise the library stream. */
+int rcp_coverage_storage_bytes(int cov, int* bytes);
 int rcp_coverage_fetch_f32(int cov, int64_t first, int64_t count, float* out, int64_t capacity);
 int rcp_coverage_rle_f32(int cov, int64_t first, int64_t count, int64_t* run_ptr_out,
                          float* values_out, int32_t* lengths_out, int64_t capacity);

@@ -99,6 +99,7 @@ SIGNATURES = {
     "rcp_signal_free": (C.c_int, [C.c_int]),
     "rcp_signal_coverage": (C.c_int, [C.c_int, C.c_int64, _i64p, _vp, _vp, _vp, _vp, C.c_int, _ip]),
     "rcp_coverage_value_type": (C.c_int, [C.c_int, _ip]),
+    "rcp_coverage_storage_bytes": (C.c_int, [C.c_int, _ip]),
     "rcp_coverage_fetch_f32": (C.c_int, [C.c_int, C.c_int64, C.c_int64, _vp, C.c_int64]),
     "rcp_coverage_rle_f32": (C.c_int, [C.c_int, C.c_int64, C.c_int64, _i64p, _vp, _i32p, C.c_int64]),
     "rcp_bin_matrix": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,

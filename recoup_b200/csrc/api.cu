@@ -1056,6 +1056,21 @@ int rcp_coverage_value_type(int cov, int* type) {
     return RCP_OK;
 }
 
+int rcp_coverage_storage_bytes(int cov, int* bytes) {
+    RCP_TRY(require_ready());
+    Coverage* cv = get_coverage(cov);
+    if (!cv) return fail(RCP_ERR_HANDLE, "unknown coverage handle %d", cov);
+    if (bytes == nullptr) return fail(RCP_ERR_ARG, "bytes is NULL");
+    *bytes = 4;
+    if (cv->d_bound) {
+        unsigned long long bound = 0;
+        const FetchItem items[1] = {{cv->d_bound, &bound, 8}};
+        RCP_TRY(fetch_and_sync(items, 1));
+        if (bound <= NARROW_MAX) *bytes = 2;
+    }
+    return RCP_OK;
+}
+
 int rcp_coverage_rle(int cov, int64_t first, int64_t count, int64_t* run_ptr_out,
                      int32_t* values_out, int32_t* lengths_out, int64_t capacity) {
     RCP_TRY(require_ready());

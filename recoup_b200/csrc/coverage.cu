@@ -540,25 +540,29 @@ concat_copy_kernel(const int32_t* __restrict__ c0, const int64_t* __restrict__ o
                    const int64_t* __restrict__ o1, const int32_t* __restrict__ l1,
                    const int32_t* __restrict__ c2, const int64_t* __restrict__ o2,
                    const int32_t* __restrict__ l2, const int32_t* __restrict__ len,
-                   const int64_t* __restrict__ off, int32_t* __restrict__ cov) {
+                   const int64_t* __restrict__ off, int32_t* __restrict__ cov,
+                   const unsigned long long* __restrict__ w0, const unsigned long long* __restrict__ w1,
+                   const unsigned long long* __restrict__ w2) {
     const int64_t r = blockIdx.x;
     if (len[r] == 0) return;
     int32_t* dst = cov + off[r];
     const int a = l0[r], b = l1[r], c = l2[r];
-    for (int i = threadIdx.x; i < a; i += CTA) dst[i] = c0[o0[r] + i];
-    for (int i = threadIdx.x; i < b; i += CTA) dst[a + i] = c1[o1[r] + i];
-    for (int i = threadIdx.x; i < c; i += CTA) dst[a + b + i] = c2[o2[r] + i];
+    const bool n0 = cov_narrow(w0), n1 = cov_narrow(w1), n2 = cov_narrow(w2);
+    for (int i = threadIdx.x; i < a; i += CTA) dst[i] = cov_at(c0, o0[r] + i, n0);
+    for (int i = threadIdx.x; i < b; i += CTA) dst[a + i] = cov_at(c1, o1[r] + i, n1);
+    for (int i = threadIdx.x; i < c; i += CTA) dst[a + b + i] = cov_at(c2, o2[r] + i, n2);
 }
 
 __global__ void __launch_bounds__(CTA)
 pack_kernel(const int32_t* __restrict__ cov, const int64_t* __restrict__ off,
             const int32_t* __restrict__ len, const int64_t* __restrict__ packed_off,
-            int64_t first, int32_t* __restrict__ out) {
+            int64_t first, int32_t* __restrict__ out, const unsigned long long* __restrict__ bound) {
     const int64_t r = first + blockIdx.x;
     const int L = len[r];
-    const int32_t* src = cov + off[r];
+    const bool narrow = cov_narrow(bound);
+    const int64_t o = off[r];
     int32_t* dst = out + packed_off[blockIdx.x];
-    for (int i = threadIdx.x; i < L; i += CTA) dst[i] = src[i];
+    for (int i = threadIdx.x; i < L; i += CTA) dst[i] = cov_at(cov, o + i, narrow);
 }
 
 __global__ void __launch_bounds__(CTA)
@@ -572,13 +576,16 @@ len_to_i64_kernel(int64_t n, const int32_t* __restrict__ len, int64_t* __restric
 // runs of region r = #{i : i == 0 or cov[i] != cov[i-1]}
 __global__ void __launch_bounds__(CTA)
 rle_count_kernel(const int32_t* __restrict__ cov, const int64_t* __restrict__ off,
-                 const int32_t* __restrict__ len, int64_t first, int64_t* __restrict__ n_runs) {
+                 const int32_t* __restrict__ len, int64_t first, int64_t* __restrict__ n_runs,
+                 const unsigned long long* __restrict__ bound) {
     __shared__ int wsum[WARPS];
     const int64_t r = first + blockIdx.x;
     const int L = len[r];
-    const int32_t* x = cov + off[r];
+    const bool narrow = cov_narrow(bound);
+    const int64_t o = off[r];
     int c = 0;
-    for (int i = threadIdx.x; i < L; i += CTA) c += (i == 0) || (x[i] != x[i - 1]);
+    for (int i = threadIdx.x; i < L; i += CTA)
+        c += (i == 0) || (cov_at(cov, o + i, narrow) != cov_at(cov, o + i - 1, narrow));
     for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
     if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = c;
     __syncthreads();
@@ -595,12 +602,13 @@ __global__ void __launch_bounds__(CTA)
 rle_write_kernel(const int32_t* __restrict__ cov, const int64_t* __restrict__ off,
                  const int32_t* __restrict__ len, int64_t first,
                  const int64_t* __restrict__ run_ptr, int32_t* __restrict__ values,
-                 int32_t* __restrict__ starts) {
+                 int32_t* __restrict__ starts, const unsigned long long* __restrict__ bound) {
     __shared__ int wsum[WARPS];
     __shared__ int carry_s;
     const int64_t r = first + blockIdx.x;
     const int L = len[r];
-    const int32_t* x = cov + off[r];
+    const bool narrow = cov_narrow(bound);
+    const int64_t o = off[r];
     const int64_t base = run_ptr[blockIdx.x];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (threadIdx.x == 0) carry_s = 0;
@@ -610,8 +618,8 @@ rle_write_kernel(const int32_t* __restrict__ cov, const int64_t* __restrict__ of
         int v = 0;
         bool head = false;
         if (i < L) {
-            v = x[i];
-            head = (i == 0) || (v != x[i - 1]);
+            v = cov_at(cov, o + i, narrow);
+            head = (i == 0) || (v != cov_at(cov, o + i - 1, narrow));
         }
         const unsigned bal = __ballot_sync(0xffffffffu, head);
         if (lane == 0) wsum[warp] = __popc(bal);
@@ -753,6 +761,7 @@ void coverage_release(Coverage& c) {
     dfree(c.len);
     dfree(c.is_null);
     dfree(c.d_stats);
+    c.d_bound = nullptr;
     c.stats_pending = false;
 }
 
@@ -767,14 +776,14 @@ __global__ void __launch_bounds__(CTA)
 na_rule_kernel(int64_t R, const int32_t* __restrict__ chrom, const int8_t* __restrict__ strand,
                const uint8_t* __restrict__ len_na, int n_chrom, const int64_t* __restrict__ off,
                int32_t* __restrict__ len, uint8_t* __restrict__ is_null, const int32_t* __restrict__ cov,
-               const int64_t* __restrict__ end_pos) {
+               const int64_t* __restrict__ end_pos, const unsigned long long* __restrict__ bound) {
     const int64_t r = (int64_t)blockIdx.x * CTA + threadIdx.x;
     if (r >= R) return;
     const int32_t L = len[r];
     const int c = chrom[r];
     if (L <= 0 || c < 0 || c >= n_chrom || !len_na[c]) return;
     const int64_t idx = end_pos ? end_pos[r] : ((strand && strand[r] < 0) ? 0 : (int64_t)L - 1);
-    if (idx < 0 || idx >= L || cov[off[r] + idx] == 0) {
+    if (idx < 0 || idx >= L || cov_at(cov, off[r] + idx, cov_narrow(bound)) == 0) {
         len[r] = 0;
         is_null[r] = 1;
     }
@@ -810,7 +819,7 @@ int coverage_na_rule(const ReadsIdx& rd, Coverage& cv, int64_t R, const int32_t*
     const unsigned long long h[4] = {0ull, 0ull, 0ull, (unsigned long long)cv.candidates};
     RCP_CUDA(cudaMemcpyAsync(cv.d_stats, h, 32, cudaMemcpyHostToDevice, g_ctx.stream));
     na_rule_kernel<<<blocks_for(R, CTA), CTA, 0, g_ctx.stream>>>(R, d_chrom, d_strand, rd.d_len_na, rd.n_chrom, cv.off,
-                                                               cv.len, cv.is_null, cv.cov, d_end_pos);
+                                                               cv.len, cv.is_null, cv.cov, d_end_pos, cv.d_bound);
     RCP_LAUNCHED();
     len_stats_kernel<<<blocks_for(R, CTA), CTA, 0, g_ctx.stream>>>(R, cv.len, cv.d_stats);
     RCP_LAUNCHED();
@@ -1019,7 +1028,8 @@ int coverage_concat3(const Coverage& a, const Coverage& b, const Coverage& c, Co
     if (R > 0) {
         concat_copy_kernel<<<(unsigned)R, CTA, 0, g_ctx.stream>>>(a.cov, a.off, a.len, b.cov, b.off,
                                                                  b.len, c.cov, c.off, c.len,
-                                                                 cv->len, cv->off, cv->cov);
+                                                                 cv->len, cv->off, cv->cov, a.d_bound,
+                                                                 b.d_bound, c.d_bound);
         RCP_LAUNCHED();
     }
     dfree(padded);
@@ -1051,7 +1061,7 @@ int coverage_fetch(const Coverage& cv, int64_t first, int64_t count, int32_t* ou
         rc = dalloc(&packed, (size_t)total);
         if (rc == RCP_OK) {
             pack_kernel<<<(unsigned)count, CTA, 0, g_ctx.stream>>>(cv.cov, cv.off, cv.len, poff,
-                                                                  first, packed);
+                                                                  first, packed, cv.d_bound);
             g_ctx.launches++;
             cudaError_t e = cudaMemcpyAsync(out, packed, (size_t)total * 4, cudaMemcpyDeviceToHost,
                                             g_ctx.stream);
@@ -1079,7 +1089,7 @@ int coverage_rle(const Coverage& cv, int64_t first, int64_t count, int64_t* run_
     int64_t *n_runs = nullptr, *d_ptr = nullptr;
     RCP_TRY(dalloc(&n_runs, (size_t)count));
     RCP_TRY(dalloc(&d_ptr, (size_t)count + 1));
-    rle_count_kernel<<<(unsigned)count, CTA, 0, g_ctx.stream>>>(cv.cov, cv.off, cv.len, first, n_runs);
+    rle_count_kernel<<<(unsigned)count, CTA, 0, g_ctx.stream>>>(cv.cov, cv.off, cv.len, first, n_runs, cv.d_bound);
     RCP_LAUNCHED();
     RCP_TRY(exclusive_scan_i64(n_runs, d_ptr, count, d_ptr + count));
     RCP_CUDA(cudaMemcpyAsync(run_ptr, d_ptr, ((size_t)count + 1) * 8, cudaMemcpyDeviceToHost,
@@ -1099,7 +1109,7 @@ int coverage_rle(const Coverage& cv, int64_t first, int64_t count, int64_t* run_
             if (rc == RCP_OK) rc = dalloc(&d_len, (size_t)total);
             if (rc == RCP_OK) {
                 rle_write_kernel<<<(unsigned)count, CTA, 0, g_ctx.stream>>>(cv.cov, cv.off, cv.len, first,
-                                                                           d_ptr, d_val, d_start);
+                                                                           d_ptr, d_val, d_start, cv.d_bound);
                 g_ctx.launches++;
                 rle_lengths_kernel<<<(unsigned)count, CTA, 0, g_ctx.stream>>>(cv.len, first, d_ptr,
                                                                              d_start, d_len);

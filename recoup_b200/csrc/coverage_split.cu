@@ -85,9 +85,9 @@ sp_plan_kernel(int64_t R, const int32_t* __restrict__ chrom, const int32_t* __re
                int32_t* __restrict__ plen, uint8_t* __restrict__ flags, int64_t* __restrict__ ntile,
                int64_t* __restrict__ padded, uint32_t* __restrict__ tab, unsigned int* __restrict__ err,
                unsigned long long* __restrict__ pstats /* [0] total len [1] max len [2] 2^32 - min len */,
-               unsigned long long* __restrict__ zero4 /* the coverage's stats words: cleared here */) {
+               unsigned long long* __restrict__ zero5 /* the coverage's stats words: cleared here */) {
     const int64_t r = (int64_t)blockIdx.x * CTA + threadIdx.x;
-    if (r < 4) zero4[r] = 0ull;
+    if (r < 5) zero5[r] = 0ull;
     unsigned long long my_len = 0;
     if (r < R) {
         const int st = strand ? (int)strand[r] : 0;
@@ -145,6 +145,9 @@ struct __align__(16) SpDesc {
 // '-' region tile j covers the mirrored positions) and which candidates can reach it: those that
 // start from (tile start - widest read + 1) on: the run of the sub-bins [first, last] in boff (the
 // group sort is queued before this kernel: the host learns the tile count while it runs).
+// bound (nullptr: fused or int32 storage): the most reads any tile applies -- n words plus the long
+// reads -- goes to this word, one atomicMax per warp.  Each read adds at most 1 to a position, so
+// no count of the call exceeds it.
 __global__ void __launch_bounds__(CTA)
 sp_tiles_kernel(int64_t R, int64_t T, const int64_t* __restrict__ off_tile, const uint32_t* __restrict__ gs,
                 const int32_t* __restrict__ plen, const uint8_t* __restrict__ flags,
@@ -154,8 +157,9 @@ sp_tiles_kernel(int64_t R, int64_t T, const int64_t* __restrict__ off_tile, cons
                 uint32_t max_w, uint32_t pmask, const uint32_t* __restrict__ boff, SpDesc* __restrict__ desc,
                 uint32_t* __restrict__ tabs,
                 const uint32_t* __restrict__ lxs, const uint32_t* __restrict__ lmax, uint32_t ln,
-                uint2* __restrict__ lrange) {
+                uint2* __restrict__ lrange, unsigned long long* __restrict__ bound) {
     const int64_t t = (int64_t)blockIdx.x * CTA + threadIdx.x;
+    const unsigned live = __ballot_sync(0xffffffffu, t < T);      // the low lanes of the warp
     if (t >= T) return;
     const int64_t r = sp_owner_of(off_tile, R, t);
     const int L = plen[r];
@@ -185,6 +189,7 @@ sp_tiles_kernel(int64_t R, int64_t T, const int64_t* __restrict__ off_tile, cons
     d.flags = flags[r];
     d.region = (uint32_t)r;
     desc[t] = d;
+    uint32_t most = d.n;
     if (ln) {           // the handle keeps long reads aside: those that can meet this tile
         tabs[t] = tstart;
         const uint32_t hi = tstart + tlen - 1u;
@@ -203,6 +208,11 @@ sp_tiles_kernel(int64_t R, int64_t T, const int64_t* __restrict__ off_tile, cons
             else b = mid;
         }
         lrange[t] = make_uint2(a, c1);
+        most = most + (c1 - a) < most ? 0xffffffffu : most + (c1 - a);
+    }
+    if (bound) {
+        most = __reduce_max_sync(live, most);
+        if ((threadIdx.x & 31) == 0) atomicMax(bound, (unsigned long long)most);
     }
 }
 
@@ -805,9 +815,11 @@ __device__ __forceinline__ bool sp_apply_fast(uint32_t e, uint32_t cts, int tlen
 // RPW * 16 bytes: conflict-free for odd RPW); the lane sums its run, one warp scan orders the
 // lanes, the run is rescanned from the right start and written back in place; the TMA unit then
 // stores the tile as ONE bulk copy (cp.async.bulk.global.shared::cta), so no thread spends LSU
-// wavefronts on the 4 B / base output.
-template <int RPW, bool STORE = true>
-__device__ __forceinline__ void warp_scan_store_fwd(int* diff, int tlen, int32_t* __restrict__ dst) {
+// wavefronts on the 4 B / base output.  O = uint16_t (narrow storage): the counts are packed into
+// the first half of the tile buffer (lane l's 4 * RPW of them at byte l * 8 * RPW) and stored the
+// same way; the store runs to the next multiple of 8 counts, inside the region's padding.
+template <int RPW, class O = int32_t>
+__device__ __forceinline__ void warp_scan_store_fwd(int* diff, int tlen, O* __restrict__ dst) {
     const int lane = threadIdx.x & 31;
     int* mine = diff + lane * 4 * RPW;
     int4 v[RPW];
@@ -819,6 +831,7 @@ __device__ __forceinline__ void warp_scan_store_fwd(int* diff, int tlen, int32_t
     }
     const int inc = warp_inclusive_scan(sum);
     int run = inc - sum;
+    if (sizeof(O) == 2) __syncwarp();       // every lane has read its run before the packed half is written
 #pragma unroll
     for (int k = 0; k < RPW; k++) {
         int4 o;
@@ -826,13 +839,37 @@ __device__ __forceinline__ void warp_scan_store_fwd(int* diff, int tlen, int32_t
         o.y = (run += v[k].y);
         o.z = (run += v[k].z);
         o.w = (run += v[k].w);
-        *(reinterpret_cast<int4*>(mine) + k) = o;
+        if (sizeof(O) == 2)
+            *(reinterpret_cast<uint2*>(diff) + lane * RPW + k) =
+                make_uint2(((uint32_t)o.x & 0xffffu) | ((uint32_t)o.y << 16), ((uint32_t)o.z & 0xffffu) | ((uint32_t)o.w << 16));
+        else
+            *(reinterpret_cast<int4*>(mine) + k) = o;
     }
     __syncwarp();
-    if (STORE && lane == 0) {
+    if (lane == 0) {
         fence_proxy_async_smem();
-        tma_store_1d(dst, diff, (uint32_t)((tlen + 3) & ~3) * 4u);
+        constexpr int E = 16 / (int)sizeof(O);      // elements per 16-byte granule
+        tma_store_1d(dst, diff, (uint32_t)((tlen + E - 1) & ~(E - 1)) * (uint32_t)sizeof(O));
         tma_store_commit();
+    }
+}
+
+// 8 rows (a whole region of 897..1024 bp) in narrow storage: row by row (conflict-free, like the
+// int32 case), each lane storing its 4 counts as one 8-byte word; the region's padding takes the
+// ragged tail.
+__device__ __forceinline__ void warp_rows_store_u16(const int* diff, int tlen, uint16_t* __restrict__ dst) {
+    const int lane = threadIdx.x & 31;
+    int pre = 0;
+    for (int row = 0; row * ROW < tlen; row++) {
+        const int4 v = *(reinterpret_cast<const int4*>(diff + row * ROW) + lane);
+        const int i0 = v.x, i1 = i0 + v.y, i2 = i1 + v.z, i3 = i2 + v.w;
+        const int inc = warp_inclusive_scan(i3);
+        const int ex = pre + inc - i3;
+        if (row * ROW + lane * 4 < tlen)
+            *reinterpret_cast<uint2*>(dst + row * ROW + lane * 4) =
+                make_uint2(((uint32_t)(ex + i0) & 0xffffu) | ((uint32_t)(ex + i1) << 16),
+                           ((uint32_t)(ex + i2) & 0xffffu) | ((uint32_t)(ex + i3) << 16));
+        pre += __shfl_sync(0xffffffffu, inc, 31);
     }
 }
 
@@ -962,8 +999,10 @@ template <bool STRANDED, bool FUSED>
 __global__ void __launch_bounds__(CTA, RCP_WTILE_OCC)
 sp_wtile_kernel(int64_t T, const SpDesc* __restrict__ desc, const uint32_t* __restrict__ cand, int P,
                 int32_t* __restrict__ cov, uint8_t* __restrict__ region_hit, FusedBins fb, LongIdx lg,
-                const uint32_t* __restrict__ tabs, const uint2* __restrict__ lrange) {
+                const uint32_t* __restrict__ tabs, const uint2* __restrict__ lrange,
+                const unsigned long long* __restrict__ bound) {
     extern __shared__ __align__(16) unsigned char wt_smem[];
+    const bool narrow = !FUSED && cov_narrow(bound);       // the same for every warp of the grid
     const int warp = threadIdx.x >> 5;
     const uint32_t lane = threadIdx.x & 31;
     int* diff = reinterpret_cast<int*>(wt_smem) + warp * WT_ONE;
@@ -1084,6 +1123,18 @@ sp_wtile_kernel(int64_t T, const SpDesc* __restrict__ desc, const uint32_t* __re
                     default: prefixed = warp_scan_prefix2<8>(diff); break;
                 }
                 tile_to_bins(diff, d, fb, prefixed);
+            }
+        } else if (narrow) {
+            uint16_t* dst = reinterpret_cast<uint16_t*>(cov) + d.out;
+            switch (rows) {
+                case 1: warp_scan_store_fwd<1>(diff, d.tlen, dst); break;
+                case 2: warp_scan_store_fwd<2>(diff, d.tlen, dst); break;
+                case 3: warp_scan_store_fwd<3>(diff, d.tlen, dst); break;
+                case 4: warp_scan_store_fwd<4>(diff, d.tlen, dst); break;
+                case 5: warp_scan_store_fwd<5>(diff, d.tlen, dst); break;
+                case 6: warp_scan_store_fwd<6>(diff, d.tlen, dst); break;
+                case 7: warp_scan_store_fwd<7>(diff, d.tlen, dst); break;
+                default: warp_rows_store_u16(diff, d.tlen, dst); break;
             }
         } else {
             int32_t* dst = cov + d.out;
@@ -1656,7 +1707,7 @@ static int split_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32
     RCP_TRY(dalloc(&cv->off, r + 1));
     RCP_TRY(dalloc(&cv->len, r));
     RCP_TRY(dalloc(&cv->is_null, r));
-    RCP_TRY(dalloc(&cv->d_stats, 4));
+    RCP_TRY(dalloc(&cv->d_stats, 5));
     auto give_up = [&]() {
         dfree(cv->off);
         dfree(cv->len);
@@ -1667,7 +1718,7 @@ static int split_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32
     {
         StageTimer t(ST_SP_PLAN);
         RCP_CUDA(cudaMemsetAsync(A.base, 0, zero_bytes, g_ctx.stream));
-        if (R == 0) RCP_CUDA(cudaMemsetAsync(cv->d_stats, 0, 32, g_ctx.stream));     // else: sp_plan_kernel
+        if (R == 0) RCP_CUDA(cudaMemsetAsync(cv->d_stats, 0, 40, g_ctx.stream));     // else: sp_plan_kernel
         if (R > 0) {
             sp_plan_kernel<<<blocks_for(R, CTA), CTA, 0, g_ctx.stream>>>(
                 R, d_chrom.ptr, d_start.ptr, d_end.ptr, d_strand.ptr, rd.d_chrom_off, rd.d_chrom_len,
@@ -1747,8 +1798,11 @@ static int split_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32
         cv->max_len = (int32_t)h.pstats[1];
         cv->n_null = 0;
         cv->stats_pending = true;
+        // 4 bytes per element: the storage width is decided on the device, after this allocation
         RCP_TRY(dalloc(&cv->cov, (size_t)h.total_padded));
+        if (getenv("RCP_COVERAGE_WIDE") == nullptr) cv->d_bound = cv->d_stats + 4;
     }
+    unsigned long long* bound = cv->d_bound ? cv->d_stats + 4 : nullptr;     // nullptr: int32 storage
 
     // ---- the sorted candidates: the handle's binned index when it has one, else this mask's ----
     bool words_stranded = stranded;
@@ -1774,7 +1828,7 @@ static int split_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32
         sp_tiles_kernel<<<blocks_for(T, CTA), CTA, 0, g_ctx.stream>>>(R, T, off_tile, gs, plen, flags,
                                                                      fz ? nullptr : cv->off, fb.edge, fb.n, max_w, pmask, boff,
                                                                      desc, tabs,
-                                                                     lg.xs, lg.maxe1, lg.n, lrange);
+                                                                     lg.xs, lg.maxe1, lg.n, lrange, bound);
         RCP_LAUNCHED();
     }
     if (T > 0) {
@@ -1788,7 +1842,7 @@ static int split_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32
                 per_sm = std::max(per_sm, 1);
                 kern<<<(unsigned)std::min<int64_t>(want, (int64_t)g_ctx.sm_count * per_sm), CTA, WTILE_SMEM,
                        g_ctx.stream>>>(
-                    T, desc, cand, P, cv->cov, region_hit, fb, lg, tabs, lrange);
+                    T, desc, cand, P, cv->cov, region_hit, fb, lg, tabs, lrange, bound);
                 RCP_LAUNCHED();
                 return RCP_OK;
             };

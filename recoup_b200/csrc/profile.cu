@@ -7,12 +7,17 @@
 //   bin_median_kernel    1 CTA / region: exact median by value bisection
 //   interp_kernel        regions shorter than the bin count (util.R:17-73): fmm spline or
 //                        neighbourhood fill, one warp per flagged region
-//   base_matrix_kernel   per-base matrix: int32 -> fp64 tiled transpose (profile.R:100-151)
+//   base_matrix_kernel   per-base matrix: counts -> fp64 tiled transpose (profile.R:100-151)
 //
 // Every kernel that reads coverage values is a template on the value type V of the handle:
 // int32_t (reads: 64-bit integer sums) or float (signal tracks: fp64 sums; the words hold float
 // bits).  The helpers below are the only places the two differ; for int32_t they are the casts
 // the kernels always used.
+//
+// Each such kernel also has a storage type S: int32_t (4-byte words) or, for int32 counts of the
+// split path that no tile could push past 65 535, uint16_t (cov_narrow).  The kernel reads the
+// coverage's decision word once at entry and runs the matching instance of its body: the branch is
+// uniform over the grid, and the host never waits for the word.
 
 #include <algorithm>
 #include <cstdlib>
@@ -77,6 +82,41 @@ __device__ __forceinline__ double key_double(typename Val<V>::Key k) {
     else return (double)k;
 }
 
+// storage: log2 of the elements in 16 bytes, and the unsigned word a staged element is read as
+template <class S>
+constexpr int LOG_PER16 = sizeof(S) == 2 ? 3 : 2;
+template <class S>
+using Word = typename std::conditional<sizeof(S) == 2, uint16_t, uint32_t>::type;
+// a staged 16-byte unit -> its term in a sum (8 counts of at most 65 535 fit 32 bits)
+template <class V, class S>
+__device__ __forceinline__ typename Val<V>::Sum unit_sum(uint4 x) {
+    if constexpr (sizeof(S) == 2) {
+        return (long long)(((x.x & 0xffffu) + (x.x >> 16)) + ((x.y & 0xffffu) + (x.y >> 16)) +
+                           ((x.z & 0xffffu) + (x.z >> 16)) + ((x.w & 0xffffu) + (x.w >> 16)));
+    } else {
+        return (word_sum<V>(x.x) + word_sum<V>(x.y)) + (word_sum<V>(x.z) + word_sum<V>(x.w));
+    }
+}
+// elements [q, q + 4) (q a multiple of 4) as loaded: 16 bytes, or 8 when narrow; widen4 unpacks them.
+// The streaming loops keep rows packed in registers and, when narrow, put twice the rows in flight,
+// so that a warp has as many bytes outstanding in either layout.
+template <class S>
+using Raw4 = typename std::conditional<sizeof(S) == 2, uint2, int4>::type;
+__device__ __forceinline__ int4 widen4(int4 v) { return v; }
+__device__ __forceinline__ int4 widen4(uint2 u) {
+    return make_int4((int)(u.x & 0xffffu), (int)(u.x >> 16), (int)(u.y & 0xffffu), (int)(u.y >> 16));
+}
+template <class S>
+__device__ __forceinline__ Raw4<S> load4_cs(const S* p) {
+    return __ldcs(reinterpret_cast<const Raw4<S>*>(p));
+}
+template <class S>
+__device__ __forceinline__ int4 load4_g(const S* p) {
+    return widen4(__ldg(reinterpret_cast<const Raw4<S>*>(p)));
+}
+template <class S>
+constexpr int ROWS_IN_FLIGHT = sizeof(S) == 2 ? 8 : 4;
+
 struct Seg {
     int a, b;   // [a, b) inside the region's coverage vector
 };
@@ -97,6 +137,7 @@ __device__ __forceinline__ Seg segment_of(int L, int where, int f1, int f2) {
 
 struct BinArgs {
     const int32_t* cov;
+    const unsigned long long* bound;   // Coverage::d_bound
     const int64_t* off;
     const int32_t* len;
     const uint8_t* is_null;
@@ -137,13 +178,18 @@ __device__ __forceinline__ long long warp_range_sum(const int32_t* __restrict__ 
 }
 
 // Median bins (sumStat = "median"): one CTA per region.  dynamic smem: edges[n + 1].
-template <class V>
-__global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
+// (static shared memory lives in the kernel, so that the two instances of a body share it)
+struct MedianSmem {
+    int wcount[WARPS];
+    int chunk_carry;
+};
+template <class V, class S>
+__device__ __forceinline__ void bin_median_run(const BinArgs& p, MedianSmem& sm) {
     using K = typename Val<V>::Key;
     extern __shared__ __align__(16) int sh[];
     int* edges = sh;                    // n + 1
-    __shared__ int wcount[WARPS];
-    __shared__ int chunk_carry;
+    auto& wcount = sm.wcount;
+    auto& chunk_carry = sm.chunk_carry;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int64_t r = blockIdx.x;
     const int n = p.n;
@@ -190,7 +236,7 @@ __global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
         if (tid == 0) edges[n] = sg.b;
         __syncthreads();
     }
-    const int32_t* src = p.cov + p.off[r];
+    const S* src = reinterpret_cast<const S*>(p.cov) + p.off[r];
     // ---- median: groups of g lanes per bin, exact order statistics by value bisection ----
     int g = 1;
     while (g < 32 && g < bsz) g <<= 1;
@@ -240,6 +286,15 @@ __global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
     }
 }
 
+template <class V>
+__global__ void __launch_bounds__(CTA) bin_median_kernel(BinArgs p) {
+    __shared__ MedianSmem sm;
+    if constexpr (std::is_same<V, int32_t>::value) {
+        if (cov_narrow(p.bound)) return bin_median_run<V, uint16_t>(p, sm);
+    }
+    bin_median_run<V, int32_t>(p, sm);
+}
+
 // ---- TMA (1-D bulk copy) + mbarrier helpers for the staging of bin_mean_kernel ----------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return (uint32_t)__cvta_generic_to_shared(p);
@@ -285,7 +340,7 @@ __device__ __forceinline__ void fence_proxy_async() {
 //   z, w   the segment [a, b) to bin (b <= a: NULL or empty -> zero row)
 //   bsz, dif   bin width and the number of bins one base wider (util.R:74-80); bsz = 0: the
 //              segment is shorter than the bin count (interpolation list)
-//   lo_al, nvec   staging run (4-aligned first base, int4 count) when the whole segment is ONE
+//   lo_al, nvec   staging run (16-byte aligned first base, 16-byte units) when the whole segment is ONE
 //              staged run of narrow bins -- only those are prefetched; nvec = 0 otherwise
 struct __align__(16) BinDesc {
     int off_lo, off_hi, a, b;
@@ -299,9 +354,12 @@ __global__ void __launch_bounds__(CTA)
 bin_desc_kernel(int64_t R, const int64_t* __restrict__ off, const int32_t* __restrict__ len,
                 const uint8_t* __restrict__ is_null, int where, int f1, int f2, int n,
                 int buf_ints, BinDesc* __restrict__ desc, int32_t* __restrict__ long_list,
-                unsigned int* __restrict__ long_count) {
+                unsigned int* __restrict__ long_count, const unsigned long long* __restrict__ bound) {
     const int64_t r = (int64_t)blockIdx.x * CTA + threadIdx.x;
     if (r >= R) return;
+    const bool narrow = cov_narrow(bound);
+    const int sh = narrow ? 3 : 2;                      // log2 of the elements in a 16-byte unit
+    const int cap = narrow ? (buf_ints >> 1) & ~3 : buf_ints;     // ints of one buffer of bin_mean_kernel
     Seg sg;
     sg.a = sg.b = 0;
     if (!is_null[r]) sg = segment_of(len[r], where, f1, f2);
@@ -314,11 +372,11 @@ bin_desc_kernel(int64_t R, const int64_t* __restrict__ off, const int32_t* __res
     const int Ls = sg.b - sg.a;
     d.bsz = Ls >= n ? Ls / n : 0;
     d.dif = Ls >= n ? Ls - d.bsz * n : 0;
-    d.lo_al = sg.a & ~3;
+    d.lo_al = sg.a & ~((1 << sh) - 1);
     d.nvec = 0;
     if (d.bsz > 0 && d.bsz < STAGE_MAX_BIN) {
-        const int nvec = (sg.b - d.lo_al + 3) >> 2;
-        if (nvec * 4 <= buf_ints) d.nvec = nvec;
+        const int nvec = (sg.b - d.lo_al + (1 << sh) - 1) >> sh;
+        if (nvec * 4 <= cap) d.nvec = nvec;             // 16 bytes per unit, 4 per int of the buffer
     }
     // a long region with wide bins (gene bodies run to megabases) would keep ONE CTA busy long
     // after the others have finished: its bins go to bin_wide_kernel, one warp per bin, spread
@@ -350,17 +408,28 @@ __device__ __forceinline__ BinDesc load_bin_desc(const BinDesc* __restrict__ p) 
 // to the interpolation list (util.R:17).
 constexpr int NBUF_MAX = 8;
 
-template <class V>
-__global__ void __launch_bounds__(BT)
-bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_ints, int nbuf) {
+struct MeanSmem {
+    int wcount[BWARPS];
+    int chunk_carry;
+    __align__(8) uint64_t full_bar[NBUF_MAX];     // one per staging buffer
+    BinDesc ring[NBUF_MAX];                       // descriptor of the region in each buffer
+};
+template <class V, class ST>
+__device__ __forceinline__ void bin_mean_run(const BinArgs& p, const BinDesc* __restrict__ desc, int64_t R,
+                                             int buf_ints, int nbuf, MeanSmem& sm) {
     using S = typename Val<V>::Sum;
+    constexpr int ESH = LOG_PER16<ST>, E = 1 << ESH;     // elements per 16-byte unit
+    if (sizeof(ST) == 2) {      // a region takes half the bytes: twice the buffers in the same shared memory
+        buf_ints = (buf_ints >> 1) & ~3;
+        nbuf = min(2 * nbuf, NBUF_MAX);
+    }
     extern __shared__ __align__(16) int sh[];
     int* edges = sh;                                         // n + 1 (unequal bins only)
     uint32_t* bufs = reinterpret_cast<uint32_t*>(sh + ((p.n + 1 + 3) & ~3));
-    __shared__ int wcount[BWARPS];
-    __shared__ int chunk_carry;
-    __shared__ __align__(8) uint64_t full_bar[NBUF_MAX];     // one per staging buffer
-    __shared__ BinDesc ring[NBUF_MAX];                       // descriptor of the region in each buffer
+    auto& wcount = sm.wcount;
+    auto& chunk_carry = sm.chunk_carry;
+    auto& full_bar = sm.full_bar;
+    auto& ring = sm.ring;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int n = p.n;
     const int64_t step = gridDim.x;
@@ -375,7 +444,7 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
     none.off_lo = none.off_hi = none.a = none.b = none.bsz = none.dif = none.lo_al = none.nvec = 0;
 
     auto src_of = [&](const BinDesc& d) {
-        return p.cov + (int64_t)(((uint64_t)(uint32_t)d.off_hi << 32) | (uint32_t)d.off_lo);
+        return reinterpret_cast<const ST*>(p.cov) + (int64_t)(((uint64_t)(uint32_t)d.off_hi << 32) | (uint32_t)d.off_lo);
     };
     // thread 0 starts the copy of one region into buffer `which` (regions that are not one staged
     // run just complete the barrier phase) and publishes its descriptor beside it
@@ -443,14 +512,15 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
                 __syncthreads();
             }
             auto edge = [&](int i) { return equal ? d.a + i * bsz : edges[i]; };
-            const int32_t* src = src_of(d);
+            const ST* src = src_of(d);
+            const Word<ST>* staged = reinterpret_cast<const Word<ST>*>(stage);
             if (bsz < STAGE_MAX_BIN) {
                 const bool preloaded = d.nvec > 0;
-                const int bins_per_chunk = preloaded ? n : max(1, (buf_ints - 4) / (bsz + 1));
+                const int bins_per_chunk = preloaded ? n : max(1, ((buf_ints << (ESH - 2)) - E) / (bsz + 1));
                 for (int bin0 = 0; bin0 < n; bin0 += bins_per_chunk) {
                     const int bin1 = min(n, bin0 + bins_per_chunk);
-                    const int lo_al = preloaded ? d.lo_al : (edge(bin0) & ~3);
-                    const int nvec = preloaded ? d.nvec : ((edge(bin1) - lo_al + 3) >> 2);
+                    const int lo_al = preloaded ? d.lo_al : (edge(bin0) & ~(E - 1));
+                    const int nvec = preloaded ? d.nvec : ((edge(bin1) - lo_al + E - 1) >> ESH);
                     if (!preloaded) {       // several runs per region: staged here, no overlap
                         __syncthreads();
                         const int4* gsrc = reinterpret_cast<const int4*>(src + lo_al);
@@ -477,12 +547,9 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
                             const int share = (blen + g - 1) / g;
                             int q = eb0 - lo_al + part * share;
                             const int qe = min(q + share, eb1 - lo_al);
-                            while (q < qe && (q & 3)) s64 += word_sum<V>(stage[q++]);
-                            for (; q + 4 <= qe; q += 4) {
-                                const uint4 x = *reinterpret_cast<const uint4*>(stage + q);
-                                s64 += (word_sum<V>(x.x) + word_sum<V>(x.y)) + (word_sum<V>(x.z) + word_sum<V>(x.w));
-                            }
-                            while (q < qe) s64 += word_sum<V>(stage[q++]);
+                            while (q < qe && (q & (E - 1))) s64 += word_sum<V>(staged[q++]);
+                            for (; q + E <= qe; q += E) s64 += unit_sum<V, ST>(*reinterpret_cast<const uint4*>(staged + q));
+                            while (q < qe) s64 += word_sum<V>(staged[q++]);
                         }
                         for (int dd = g >> 1; dd > 0; dd >>= 1) s64 += __shfl_xor_sync(0xffffffffu, s64, dd);
                         if (b < bin1 && part == 0)
@@ -501,22 +568,23 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
                     const int lo = edge(i0), hi = edge(i1);
                     int k = i0, nxt = edge(i0 + 1);
                     S acc = 0;
-                    constexpr int UW = 4;
+                    constexpr int UW = ROWS_IN_FLIGHT<ST>;
                     for (int q0 = lo & ~3; q0 < hi; q0 += 128 * UW) {
-                        int4 x[UW];
+                        Raw4<ST> x[UW];
 #pragma unroll
                         for (int u = 0; u < UW; u++) {
                             const int q = q0 + u * 128 + lane * 4;
-                            x[u] = make_int4(0, 0, 0, 0);
-                            if (q < hi) x[u] = __ldcs(reinterpret_cast<const int4*>(src + q));
+                            x[u] = Raw4<ST>{};
+                            if (q < hi) x[u] = load4_cs(src + q);
                         }
 #pragma unroll
                         for (int u = 0; u < UW; u++) {
                             const int row = q0 + u * 128;
                             if (row >= hi) break;
                             const int q = row + lane * 4;
-                            auto a0 = word_val<V>(x[u].x), a1 = word_val<V>(x[u].y), a2 = word_val<V>(x[u].z),
-                                 a3 = word_val<V>(x[u].w);
+                            const int4 xu = widen4(x[u]);
+                            auto a0 = word_val<V>(xu.x), a1 = word_val<V>(xu.y), a2 = word_val<V>(xu.z),
+                                 a3 = word_val<V>(xu.w);
                             if (row < lo || row + 128 > hi) {           // first / last row of the run
                                 a0 = (q >= lo && q < hi) ? a0 : 0;
                                 a1 = (q + 1 >= lo && q + 1 < hi) ? a1 : 0;
@@ -551,6 +619,16 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
     // the copy issued for the (non-existent) region after the last one carries no bytes
 }
 
+template <class V>
+__global__ void __launch_bounds__(BT)
+bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_ints, int nbuf) {
+    __shared__ MeanSmem sm;
+    if constexpr (std::is_same<V, int32_t>::value) {
+        if (cov_narrow(p.bound)) return bin_mean_run<V, uint16_t>(p, desc, R, buf_ints, nbuf, sm);
+    }
+    bin_mean_run<V, int32_t>(p, desc, R, buf_ints, nbuf, sm);
+}
+
 // ---- long regions with wide bins: runs of WIDE_RUN bins of all such regions in one pool --------
 // One warp STREAMS a run of consecutive bins -- one contiguous stretch of coverage -- with
 // 16-byte loads, four 512-byte rows in flight.  A row (128 bases) meets at most one bin edge
@@ -558,10 +636,10 @@ bin_mean_kernel(BinArgs p, const BinDesc* __restrict__ desc, int64_t R, int buf_
 // once per bin.  Bin i has bsz + [rank[i] <= dif] elements (util.R:74-80).
 constexpr int WIDE_RUN = 16;
 
-template <class V>
-__global__ void __launch_bounds__(BT, 3)
-bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __restrict__ long_list,
-                unsigned int* __restrict__ long_count) {
+template <class V, class ST>
+__device__ __forceinline__ void bin_wide_run(const BinArgs& p, const BinDesc* __restrict__ desc,
+                                             const int32_t* __restrict__ long_list,
+                                             unsigned int* __restrict__ long_count) {
     using S = typename Val<V>::Sum;
     const int lane = threadIdx.x & 31;
     const int n = p.n;
@@ -590,21 +668,21 @@ bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __re
         }
         const int lo = d.a + i0 * bsz + pre;
         const int hi = lo + (i1 - i0) * bsz + __popc(extra);
-        const int32_t* src = p.cov + (int64_t)(((uint64_t)(uint32_t)d.off_hi << 32) | (uint32_t)d.off_lo);
+        const ST* src = reinterpret_cast<const ST*>(p.cov) + (int64_t)(((uint64_t)(uint32_t)d.off_hi << 32) | (uint32_t)d.off_lo);
         double* out = p.out + r;
         int k = i0, b0 = lo, nxt = lo + bsz + (int)(extra & 1u);
         S acc = 0;
-        constexpr int UW = 4;
+        constexpr int UW = ROWS_IN_FLIGHT<ST>;
         // the rows of the NEXT trip are requested before this trip's rows are summed
-        auto fetch = [&](int q0, int4* x) {
+        auto fetch = [&](int q0, Raw4<ST>* x) {
 #pragma unroll
             for (int v = 0; v < UW; v++) {
                 const int q = q0 + v * 128 + lane * 4;
-                x[v] = make_int4(0, 0, 0, 0);
-                if (q < hi) x[v] = __ldcs(reinterpret_cast<const int4*>(src + q));
+                x[v] = Raw4<ST>{};
+                if (q < hi) x[v] = load4_cs(src + q);
             }
         };
-        int4 x[UW], y[UW];
+        Raw4<ST> x[UW], y[UW];
         fetch(lo & ~3, x);
         for (int q0 = lo & ~3; q0 < hi; q0 += 128 * UW) {
             if (q0 + 128 * UW < hi) fetch(q0 + 128 * UW, y);
@@ -613,8 +691,9 @@ bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __re
                 const int row = q0 + v * 128;
                 if (row >= hi) break;
                 const int q = row + lane * 4;
-                auto a0 = word_val<V>(x[v].x), a1 = word_val<V>(x[v].y), a2 = word_val<V>(x[v].z),
-                     a3 = word_val<V>(x[v].w);
+                const int4 xv = widen4(x[v]);
+                auto a0 = word_val<V>(xv.x), a1 = word_val<V>(xv.y), a2 = word_val<V>(xv.z),
+                     a3 = word_val<V>(xv.w);
                 if (row < lo || row + 128 > hi) {           // first / last row of the run
                     a0 = (q >= lo && q < hi) ? a0 : 0;
                     a1 = (q + 1 >= lo && q + 1 < hi) ? a1 : 0;
@@ -644,9 +723,20 @@ bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __re
     }
 }
 
+template <class V>
+__global__ void __launch_bounds__(BT, 3)
+bin_wide_kernel(BinArgs p, const BinDesc* __restrict__ desc, const int32_t* __restrict__ long_list,
+                unsigned int* __restrict__ long_count) {
+    if constexpr (std::is_same<V, int32_t>::value) {
+        if (cov_narrow(p.bound)) return bin_wide_run<V, uint16_t>(p, desc, long_list, long_count);
+    }
+    bin_wide_run<V, int32_t>(p, desc, long_list, long_count);
+}
+
 // ---- interpolation of short segments (util.R:17-73) ------------------------------------------
 struct InterpArgs {
     const int32_t* cov;
+    const unsigned long long* bound;
     const int64_t* off;
     const int32_t* len;
     int where, f1, f2, n;
@@ -659,8 +749,9 @@ struct InterpArgs {
 };
 
 // dynamic smem per warp-CTA: 4n doubles + 2n ints + RRng
-template <class V>
-__global__ void __launch_bounds__(32) interp_kernel(InterpArgs p) {
+template <class V, class ST>
+__device__ __forceinline__ void interp_run(const InterpArgs& p) {
+    using E = typename std::conditional<sizeof(ST) == 2, uint16_t, V>::type;     // an element as stored
     extern __shared__ double shd[];
     const int n = p.n;
     double* y = shd;               // input values (L) / neighbourhood vector (n)
@@ -677,7 +768,7 @@ __global__ void __launch_bounds__(32) interp_kernel(InterpArgs p) {
         const int L_all = p.len[r];
         const Seg sg = segment_of(L_all, p.where, p.f1, p.f2);
         const int L = sg.b - sg.a;
-        const V* src = reinterpret_cast<const V*>(p.cov) + p.off[r] + sg.a;
+        const E* src = reinterpret_cast<const E*>(p.cov) + p.off[r] + sg.a;
         double* out = p.out + r;
         __syncwarp();
         bool neighborhood = p.interp == RCP_INTERP_NEIGHBORHOOD;
@@ -795,9 +886,18 @@ __global__ void __launch_bounds__(32) interp_kernel(InterpArgs p) {
     }
 }
 
+template <class V>
+__global__ void __launch_bounds__(32) interp_kernel(InterpArgs p) {
+    if constexpr (std::is_same<V, int32_t>::value) {
+        if (cov_narrow(p.bound)) return interp_run<V, uint16_t>(p);
+    }
+    interp_run<V, int32_t>(p);
+}
+
 // ---- per-base matrix --------------------------------------------------------------------------
 struct BaseArgs {
     const int32_t* cov;
+    const unsigned long long* bound;
     const int64_t* off;
     const int32_t* len;
     const uint8_t* is_null;
@@ -808,11 +908,17 @@ struct BaseArgs {
     int64_t ld;
 };
 
-template <class V>
-__global__ void __launch_bounds__(256) base_matrix_kernel(BaseArgs p) {
-    __shared__ int tile[32][33];
-    __shared__ int64_t r_off[32];
-    __shared__ int r_a[32], r_b[32];
+struct BaseSmem {
+    int tile[32][33];
+    int64_t r_off[32];
+    int r_a[32], r_b[32];
+};
+template <class V, class S>
+__device__ __forceinline__ void base_matrix_run(const BaseArgs& p, BaseSmem& sm) {
+    auto& tile = sm.tile;
+    auto& r_off = sm.r_off;
+    auto& r_a = sm.r_a;
+    auto& r_b = sm.r_b;
     const int tx = threadIdx.x, ty = threadIdx.y;
     const int64_t r0 = (int64_t)blockIdx.y * 32, k0 = (int64_t)blockIdx.x * 32;
     if (ty == 0) {
@@ -834,7 +940,7 @@ __global__ void __launch_bounds__(256) base_matrix_kernel(BaseArgs p) {
         const int64_t k = k0 + tx;
         const int q = r_a[jj] + (int)k;
         int v = 0;
-        if (k < p.n_cols && q < r_b[jj]) v = __ldg(p.cov + r_off[jj] + q);
+        if (k < p.n_cols && q < r_b[jj]) v = __ldg(reinterpret_cast<const S*>(p.cov) + r_off[jj] + q);
         tile[jj][tx] = v;
     }
     __syncthreads();
@@ -844,18 +950,33 @@ __global__ void __launch_bounds__(256) base_matrix_kernel(BaseArgs p) {
     }
 }
 
+template <class V>
+__global__ void __launch_bounds__(256) base_matrix_kernel(BaseArgs p) {
+    __shared__ BaseSmem sm;
+    if constexpr (std::is_same<V, int32_t>::value) {
+        if (cov_narrow(p.bound)) return base_matrix_run<V, uint16_t>(p, sm);
+    }
+    base_matrix_run<V, int32_t>(p, sm);
+}
+
 // Wide-tile version of the same transpose: 32 regions x 256 columns per CTA.  Rows are read with
 // 16-byte loads when the segment start is 4-aligned (always for whole windows), columns leave as
 // 256-byte runs of 32 consecutive regions, two doubles per lane when the output allows 16-byte
 // stores.  The tile index runs along x (linear, no 65535 limit).
 constexpr int BW_ROWS = 32, BW_COLS = 256;
 
-template <class V>
-__global__ void __launch_bounds__(256) base_matrix_wide_kernel(BaseArgs p, int64_t col_tiles,
-                                                               int vec_store) {
-    __shared__ int tile[BW_ROWS][BW_COLS + 1];
-    __shared__ int64_t r_off[BW_ROWS];
-    __shared__ int r_a[BW_ROWS], r_b[BW_ROWS];
+struct BaseWideSmem {
+    int tile[BW_ROWS][BW_COLS + 1];
+    int64_t r_off[BW_ROWS];
+    int r_a[BW_ROWS], r_b[BW_ROWS];
+};
+template <class V, class S>
+__device__ __forceinline__ void base_matrix_wide_run(const BaseArgs& p, int64_t col_tiles, int vec_store,
+                                                     BaseWideSmem& sm) {
+    auto& tile = sm.tile;
+    auto& r_off = sm.r_off;
+    auto& r_a = sm.r_a;
+    auto& r_b = sm.r_b;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int64_t r0 = ((int64_t)blockIdx.x / col_tiles) * BW_ROWS;
     const int64_t k0 = ((int64_t)blockIdx.x % col_tiles) * BW_COLS;
@@ -876,14 +997,14 @@ __global__ void __launch_bounds__(256) base_matrix_wide_kernel(BaseArgs p, int64
     __syncthreads();
     for (int jj = warp; jj < BW_ROWS; jj += 8) {
         const int a = r_a[jj], b = r_b[jj];
-        const int32_t* src = p.cov + r_off[jj] + a + k0;       // column k0 of this region
+        const S* src = reinterpret_cast<const S*>(p.cov) + r_off[jj] + a + k0;       // column k0 of this region
         const int avail = (int)min((int64_t)(b - a) - k0, (int64_t)BW_COLS);   // columns with data
 #pragma unroll
         for (int h = 0; h < BW_COLS / 128; h++) {
             const int c = h * 128 + lane * 4;
             int4 v = make_int4(0, 0, 0, 0);
             if ((a & 3) == 0 && c + 3 < avail) {
-                v = __ldg(reinterpret_cast<const int4*>(src + c));
+                v = load4_g(src + c);
             } else {
                 if (c < avail) v.x = __ldg(src + c);
                 if (c + 1 < avail) v.y = __ldg(src + c + 1);
@@ -913,6 +1034,15 @@ __global__ void __launch_bounds__(256) base_matrix_wide_kernel(BaseArgs p, int64
 }
 
 template <class V>
+__global__ void __launch_bounds__(256) base_matrix_wide_kernel(BaseArgs p, int64_t col_tiles, int vec_store) {
+    __shared__ BaseWideSmem sm;
+    if constexpr (std::is_same<V, int32_t>::value) {
+        if (cov_narrow(p.bound)) return base_matrix_wide_run<V, uint16_t>(p, col_tiles, vec_store, sm);
+    }
+    base_matrix_wide_run<V, int32_t>(p, col_tiles, vec_store, sm);
+}
+
+template <class V>
 int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, int stat,
                     int interp, int seed, int sample_kind, double* d_out, int64_t ld) {
     const int64_t R = cv.n_regions;
@@ -939,6 +1069,7 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
     // memory returns after the source has been staged, so `rank` may go out of scope later.
     BinArgs a;
     a.cov = cv.cov;
+    a.bound = cv.d_bound;
     a.off = cv.off;
     a.len = cv.len;
     a.is_null = cv.is_null;
@@ -974,7 +1105,8 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
         if (where == RCP_WHERE_UPSTREAM) seg_max = std::min<int64_t>(seg_max, f1);
         else if (where == RCP_WHERE_DOWNSTREAM) seg_max = std::min<int64_t>(seg_max, f2);
         else if (where == RCP_WHERE_CENTER) seg_max = std::max<int64_t>(seg_max - f1 - f2, 0);
-        int buf_ints = (int)std::min<int64_t>(STAGE_INTS, ((seg_max + 10) & ~(int64_t)3));
+        // (+ 8 more: a narrow coverage stages from an 8-aligned base into half a buffer)
+        int buf_ints = (int)std::min<int64_t>(STAGE_INTS, ((seg_max + 18) & ~(int64_t)3));
         // CTAs per SM: four, unless the typical bin is wide (mean segment / bins >= 128 bases:
         // gene bodies).  Wide bins are summed straight from global memory by one warp each and
         // are bound by the loads in flight, so they want all 64 warps of the SM; the staging
@@ -995,7 +1127,8 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
         RCP_TRY(dalloc(&long_count, 4));        // [0] regions in the list, [2..3] unit counter of bin_wide_kernel
         RCP_CUDA(cudaMemsetAsync(long_count, 0, 4 * sizeof(unsigned int), g_ctx.stream));
         bin_desc_kernel<<<(unsigned)((R + CTA - 1) / CTA), CTA, 0, g_ctx.stream>>>(
-            R, cv.off, cv.len, cv.is_null, where, f1, f2, n_bins, buf_ints, d_desc, long_list, long_count);
+            R, cv.off, cv.len, cv.is_null, where, f1, f2, n_bins, buf_ints, d_desc, long_list, long_count,
+            cv.d_bound);
         RCP_LAUNCHED();
         // CTAs per SM and buffers per CTA: as much shared memory as possible in flight
         int nbuf = 2;
@@ -1018,6 +1151,7 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
     }
     InterpArgs ia;
     ia.cov = cv.cov;
+    ia.bound = cv.d_bound;
     ia.off = cv.off;
     ia.len = cv.len;
     ia.where = where;
@@ -1061,6 +1195,7 @@ int base_matrix_impl(const Coverage& cv, int where, int f1, int f2, int64_t n_co
     if (R == 0 || n_cols == 0) return RCP_OK;
     BaseArgs a;
     a.cov = cv.cov;
+    a.bound = cv.d_bound;
     a.off = cv.off;
     a.len = cv.len;
     a.is_null = cv.is_null;

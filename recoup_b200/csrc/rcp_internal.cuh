@@ -294,17 +294,33 @@ struct Coverage {
     int64_t candidates = 0;      // block / split path: reads that passed the bitmap filter
     // split path: n_null / total_len / candidates are produced on the device after the call has
     // returned; they are fetched on first use (coverage_resolve_stats)
-    unsigned long long* d_stats = nullptr;   // [0] n_null [1] total_len [2] max_len [3] candidates
+    unsigned long long* d_stats = nullptr;   // [0] n_null [1] total_len [2] max_len [3] candidates [4] bound
     bool stats_pending = false;
     double scale = 1.0;
     int value_type = RCP_VALUE_INT32;   // RCP_VALUE_FLOAT32: `cov` holds float bits (signal tracks)
-    int32_t* cov = nullptr;      // dense 4-byte words, region r at [off[r], off[r] + len[r])
+    // Split path: d_stats + 4, the most reads any tile of the call can apply (see cov_narrow).
+    // nullptr (every other path, and RCP_COVERAGE_WIDE=1): `cov` holds 4-byte words.
+    const unsigned long long* d_bound = nullptr;
+    int32_t* cov = nullptr;      // dense 4-byte words (2-byte when narrow), region r at [off[r], off[r] + len[r])
     int64_t* off = nullptr;      // n_regions + 1, multiples of 32 ints
     int32_t* len = nullptr;      // n_regions, 0 for NULL
     uint8_t* is_null = nullptr;  // n_regions
 };
 void coverage_release(Coverage& c);
 int coverage_resolve_stats(Coverage& c);
+
+// Narrow storage.  Every read adds at most 1 to any position, so no count of a tile exceeds the
+// number of reads the tile applies; when that bound is <= 65 535 for every tile of a call, the
+// split path stores the coverage as uint16 (same element offsets, half the bytes).  The decision
+// is a device word, read by every kernel that reads the coverage: the host never waits for it.
+constexpr unsigned long long NARROW_MAX = 0xffffull;
+__device__ __forceinline__ bool cov_narrow(const unsigned long long* bound) {
+    return bound != nullptr && *bound <= NARROW_MAX;
+}
+// element i of a coverage in either layout
+__device__ __forceinline__ int32_t cov_at(const int32_t* cov, int64_t i, bool narrow) {
+    return narrow ? (int32_t)reinterpret_cast<const uint16_t*>(cov)[i] : cov[i];
+}
 // NA seqlengths: regions on such chromosomes whose genomic END position nobody covers become NULL.
 // end_pos == nullptr: GRanges mask (the end is the last stored position, the first on '-'
 // regions); else the index of that position inside each stitched element (GRangesList masks).
