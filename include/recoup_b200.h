@@ -437,6 +437,41 @@ int rcp_order(const double* v, int64_t n, int decreasing, int mem, int32_t* ix /
 int rcp_matrix_quantile(const double* m, int64_t n_rows, int64_t n_cols, int64_t ld, const double* probs,
                         int k, int mem, double* out /* k, host */);
 
+/* ---------------------------------------------------------------- k-means ----------------- */
+/* rcp_kmeans: set.seed(seed); kmeans(x, centers = k, iter.max, nstart, algorithm) -- stats::kmeans
+ *   as kmeansDesign calls it (util.R:140-197, recoup.R:602).  x: column-major m x p, leading
+ *   dimension ld; `mem` says where x, cluster, centers, withinss and size live; totss, iter,
+ *   ifault and warnings are host scalars.
+ *   Draws (host, one stream): nstart == 1: x[sample.int(m, k), ]; when those rows hold a duplicate,
+ *   or nstart >= 2: cn <- unique(x) (distinct rows in first-occurrence order, -0.0 == 0.0, exact
+ *   comparison), then cn[sample.int(nrow(cn), k), ] per start.  All starts run on the device; the
+ *   result is the first start with the strictly smallest sum(withinss), as in R.  Distances and
+ *   centres use R's floating-point operations in R's order (kmeans.c, kmns.f / AS 136), so
+ *   cluster, centers, size and iter equal R's; withinss and totss are summed in another order.
+ *   k == 1 runs MacQueen, as kmeans does.  k <= 256 (RCP_ERR_UNSUPPORTED above).
+ *   Errors: k < 1, nstart < 1, iter_max < 1, m < k, an unknown algorithm: RCP_ERR_ARG.
+ *   RCP_ERR_DATA: a non-finite x ("NA/NaN/Inf in foreign function call"), fewer distinct rows than
+ *   k, Hartigan-Wong with k >= m (IFAULT 3) or an empty cluster after its first assignment
+ *   (IFAULT 1), in any start.
+ *   ifault (the chosen start): 0, 2 (no convergence in iter_max; iter = iter_max + 1) or 4 (the
+ *   Hartigan-Wong quick-transfer stage reached 50 m steps).  warnings: RCP_KMEANS_WARN_* bits of
+ *   the warnings R raises across ALL starts. */
+#define RCP_KMEANS_HARTIGAN_WONG 1
+#define RCP_KMEANS_LLOYD 2           /* "Lloyd" and "Forgy" */
+#define RCP_KMEANS_MACQUEEN 3
+#define RCP_KMEANS_WARN_NOT_CONVERGED 1    /* "did not converge in %d iterations"             */
+#define RCP_KMEANS_WARN_EMPTY_CLUSTER 2    /* Lloyd / MacQueen: "empty cluster: try a better
+                                              set of initial centers"                        */
+#define RCP_KMEANS_WARN_QUICK_TRANSFER 4   /* "Quick-TRANSfer stage steps exceeded maximum"   */
+int rcp_kmeans(const double* x, int64_t m, int64_t p, int64_t ld, int k, int nstart, int iter_max,
+               int algorithm, int seed, int sample_kind, int mem, int32_t* cluster /* m, 1-based */,
+               double* centers /* k x p, column-major */, double* withinss /* k */, int32_t* size /* k */,
+               double* totss, int* iter, int* ifault, int* warnings);
+/* rcp_r_sample_int: rcp_r_sample_sorted without the sort -- set.seed(seed) once, then
+ *   sample.int(n[c], k[c]) for c = 0..n_calls-1 from the one stream, in draw order (1-based). */
+int rcp_r_sample_int(int seed, int sample_kind, int n_calls, const int64_t* n, const int64_t* k,
+                     int32_t* out /* host, sum(k) */);
+
 /* ---------------------------------------------------------------- multi-GPU helper -------- */
 /* Scatter a row block into the gathered matrix: dst[row_index[i] + c*ld_dst] =
  * src[i + c*ld_src] for i < n_rows, c < n_cols (all pointers on the device).  Used after the

@@ -116,6 +116,9 @@ SIGNATURES = {
     "rcp_shared_close": (C.c_int, [C.c_void_p]),
     "rcp_shared_free": (C.c_int, [C.c_void_p]),
     "rcp_rows_scatter": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, _vp, _vp, C.c_int64]),
+    "rcp_kmeans": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                             C.c_int, C.c_int, _vp, _vp, _vp, _vp, _f64p, _ip, _ip, _ip]),
+    "rcp_r_sample_int": (C.c_int, [C.c_int, C.c_int, C.c_int, _i64p, _i64p, _vp]),
 }
 
 

@@ -4,6 +4,8 @@ over librecoup_b200.so (SURVEY 8f, N4):
     calcPlotProfiles(input, opts, ...)   average curve + band per sample        plot.R:949-990
     orderProfiles(input, opts)           heat-map row order (sum / max / avg)   plot.R:1035-1150
     heatmapScale(input, ...)             upper colour limit from quantiles      plot.R:513-545
+    kmeans(x, centers, ...)              stats::kmeans as kmeansDesign calls it
+    kmeansDesign(input, design, kmParams) heat-map clusters as a design column  util.R:140-197
 
 `opts` is the nested dict of the reference (`opts["plotParams"]["sumStat"]`, ...).  Matrices are
 the `ProfileMatrix` objects profileMatrix() returns (host, column-major); they are staged to the
@@ -12,6 +14,7 @@ GPU by the library, so a device pointer can be passed through the C ABI directly
 """
 import ctypes as C
 import re
+import warnings
 
 import numpy as np
 
@@ -137,3 +140,110 @@ def heatmapScale(input, heatmapScale="common", heatmapFactor=1.0):
         return out
     sup = max(float(matrixQuantile(x["profile"], [0.95])[0]) for x in input)
     return [heatmapFactor * sup] * len(input)
+
+
+_KM_ALGORITHMS = ("Hartigan-Wong", "Lloyd", "Forgy", "MacQueen")
+_KM_CODE = {"Hartigan-Wong": 1, "Lloyd": 2, "Forgy": 2, "MacQueen": 3}
+
+
+class NamedVector(np.ndarray):
+    """A vector carrying R's names attribute (`names`, None when unnamed)."""
+
+    def __new__(cls, array, names=None):
+        obj = np.asarray(array).view(cls)
+        obj.names = names
+        return obj
+
+    def __array_finalize__(self, obj):
+        if obj is not None:
+            self.names = getattr(obj, "names", None)
+
+
+def _match_algorithm(algorithm):
+    """match.arg(algorithm): exact name or unique prefix; "Forgy" is "Lloyd"."""
+    if isinstance(algorithm, (list, tuple)):
+        algorithm = algorithm[0]
+    if algorithm in _KM_ALGORITHMS:
+        return algorithm
+    hits = [a for a in _KM_ALGORITHMS if algorithm and a.startswith(algorithm)]
+    if len(hits) != 1:
+        raise ValueError("'arg' should be one of %s" % ", ".join('"%s"' % a for a in _KM_ALGORITHMS))
+    return hits[0]
+
+
+def kmeans(x, centers, iter_max=10, nstart=1, algorithm="Hartigan-Wong", seed=42, sample_kind="Rejection"):
+    """`set.seed(seed); kmeans(x, centers, iter.max, nstart, algorithm)` on the device
+    (rcp_kmeans).  `centers` is the number of clusters.  Returns dict(cluster (1-based, named by
+    x.rownames for a ProfileMatrix), centers (k x p), totss, withinss, tot_withinss, betweenss,
+    size, iter, ifault) and raises R's warnings."""
+    if isinstance(centers, (bool, np.bool_)) or not isinstance(centers, (int, np.integer)):
+        raise TypeError("centers must be the number of clusters")
+    algorithm = _match_algorithm(algorithm)
+    m = _f(x)
+    n, p = m.shape
+    k = int(centers)
+    _lib.ensure_init()
+    cluster = np.empty(n, dtype=np.int32)
+    cen = np.empty((max(k, 0), p), dtype=np.float64, order="F")
+    wss = np.empty(max(k, 0), dtype=np.float64)
+    size = np.empty(max(k, 0), dtype=np.int32)
+    totss = C.c_double(0.0)
+    it, ifault, warn = C.c_int(0), C.c_int(0), C.c_int(0)
+    _lib.check(_lib.lib.rcp_kmeans(_vp(m), n, p, max(n, 1), k, int(nstart), int(iter_max), _KM_CODE[algorithm],
+                                   int(seed), _lib.SAMPLE_KIND[sample_kind], _lib.MEM_HOST, _vp(cluster), _vp(cen),
+                                   _vp(wss), _vp(size), C.byref(totss), C.byref(it), C.byref(ifault),
+                                   C.byref(warn)))
+    w = warn.value
+    if w & 1:
+        warnings.warn("did not converge in %d iteration%s" % (iter_max, "" if iter_max == 1 else "s"),
+                      stacklevel=2)
+    if w & 4:
+        warnings.warn("Quick-TRANSfer stage steps exceeded maximum (= %d)" % min(2147483647, 50 * n),
+                      stacklevel=2)
+    if w & 2:
+        warnings.warn("empty cluster: try a better set of initial centers", stacklevel=2)
+    tot_w = float(np.sum(wss.astype(np.longdouble)))
+    return {"cluster": NamedVector(cluster, getattr(x, "rownames", None)), "centers": cen,
+            "totss": totss.value, "withinss": wss, "tot_withinss": tot_w, "betweenss": totss.value - tot_w,
+            "size": size, "iter": it.value, "ifault": ifault.value}
+
+
+_KM_DEFAULTS = {"k": 0, "nstart": 20, "algorithm": "Hartigan-Wong", "iterMax": 20, "reference": None, "seed": 42}
+
+
+def kmeansDesign(input, design=None, kmParams=None):
+    """util.R:140-197 (parity unpinned): split the heat map into k-means clusters.  kmParams =
+    dict(k, nstart, algorithm, iterMax, reference, seed) over the defaults above; k == 0 returns
+    `design` unchanged.  The matrix is the profile of the sample whose `id` is `reference`, else
+    the cbind of every sample's profile in sample order (an unknown reference warns and uses all
+    samples).  Returns the design -- a dict of equal-length columns, created when None -- with a
+    `Cluster` column of "Cluster <n>" labels, one per row in row order."""
+    kp = dict(_KM_DEFAULTS)
+    kp.update(kmParams or {})
+    if int(kp["k"]) == 0:
+        return design
+    ref = kp.get("reference")
+    mats = None
+    if ref is not None:
+        ids = [s.get("id") for s in input]
+        if ref in ids:
+            mats = [input[ids.index(ref)]["profile"]]
+        else:
+            warnings.warn("reference %s not found in the input sample ids; using all samples for k-means "
+                          "clustering" % ref, stacklevel=2)
+    if mats is None:
+        mats = [s["profile"] for s in input]
+    x = np.asfortranarray(np.hstack([np.asarray(mm, dtype=np.float64) for mm in mats]))
+    names = getattr(mats[0], "rownames", None)
+    if names is not None:
+        from .profile import ProfileMatrix
+        x = ProfileMatrix(x, rownames=names)
+    km = kmeans(x, int(kp["k"]), iter_max=int(kp["iterMax"]), nstart=int(kp["nstart"]),
+                algorithm=kp["algorithm"], seed=int(kp["seed"]))
+    labels = np.array(["Cluster %d" % c for c in np.asarray(km["cluster"])], dtype=object)
+    out = {} if design is None else dict(design)
+    for col, v in out.items():
+        if len(v) != labels.shape[0]:
+            raise ValueError("design column %s has %d rows, the profiles %d" % (col, len(v), labels.shape[0]))
+    out["Cluster"] = labels
+    return out

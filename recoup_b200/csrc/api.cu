@@ -487,6 +487,26 @@ int common_length(const Coverage& cv, int64_t* out) {
 }
 
 }  // namespace
+
+// sample.int(n, k) as base R dispatches it: the hash variant (do_sample2: draw, redraw on a
+// duplicate, at most 100 tries) when n > 1e7 and k <= n/2, else the partial Fisher-Yates loop.
+void r_sample_int(RRng& rng, int64_t n, int64_t k, int32_t* out) {
+    if (n > 10000000 && k <= n / 2) {
+        std::vector<uint64_t> seen((size_t)((n + 63) / 64), 0);
+        for (int64_t i = 0; i < k; i++) {
+            uint32_t v = 0;
+            for (int j = 0; j < 100; j++) {
+                v = rng.index((uint32_t)n);
+                if (!((seen[v >> 6] >> (v & 63)) & 1ull)) break;
+            }
+            seen[v >> 6] |= 1ull << (v & 63);
+            out[i] = (int32_t)(v + 1);
+        }
+        return;
+    }
+    std::vector<int> x((size_t)n);
+    rng.sample((int)n, (int)k, x.data(), out);
+}
 }  // namespace rcp
 
 using namespace rcp;
@@ -668,32 +688,13 @@ int rcp_r_sample(int n, int k, int seed, int sample_kind, int* out) {
     return RCP_OK;
 }
 
-// sample.int(n, k) as base R dispatches it: the hash variant (do_sample2: draw, redraw on a
-// duplicate, at most 100 tries) when n > 1e7 and k <= n/2, else the partial Fisher-Yates loop.
-static void r_sample_int(RRng& rng, int64_t n, int64_t k, int32_t* out) {
-    if (n > 10000000 && k <= n / 2) {
-        std::vector<uint64_t> seen((size_t)((n + 63) / 64), 0);
-        for (int64_t i = 0; i < k; i++) {
-            uint32_t v = 0;
-            for (int j = 0; j < 100; j++) {
-                v = rng.index((uint32_t)n);
-                if (!((seen[v >> 6] >> (v & 63)) & 1ull)) break;
-            }
-            seen[v >> 6] |= 1ull << (v & 63);
-            out[i] = (int32_t)(v + 1);
-        }
-        return;
-    }
-    std::vector<int> x((size_t)n);
-    rng.sample((int)n, (int)k, x.data(), out);
-}
-
-int rcp_r_sample_sorted(int seed, int sample_kind, int n_calls, const int64_t* n, const int64_t* k,
-                        int32_t* out) {
+// set.seed(seed) once, then sample.int(n[c], k[c]) for every call from the one stream; sorted or not
+static int r_sample_calls(const char* who, int seed, int sample_kind, int n_calls, const int64_t* n,
+                          const int64_t* k, int32_t* out, bool sorted) {
     if (sample_kind != RCP_SAMPLE_REJECTION && sample_kind != RCP_SAMPLE_ROUNDING)
         return fail(RCP_ERR_ARG, "unknown sample kind %d", sample_kind);
     if (n_calls < 0 || (n_calls > 0 && (n == nullptr || k == nullptr)))
-        return fail(RCP_ERR_ARG, "rcp_r_sample_sorted: bad argument");
+        return fail(RCP_ERR_ARG, "%s: bad argument", who);
     std::unique_ptr<RRng> rng(new RRng);
     rng->seed((uint32_t)seed, sample_kind);
     int64_t at = 0;
@@ -703,10 +704,20 @@ int rcp_r_sample_sorted(int seed, int sample_kind, int n_calls, const int64_t* n
                         (long long)k[c], (long long)n[c]);
         if (k[c] > 0 && out == nullptr) return fail(RCP_ERR_ARG, "out is NULL");
         r_sample_int(*rng, n[c], k[c], out + at);
-        std::sort(out + at, out + at + k[c]);
+        if (sorted) std::sort(out + at, out + at + k[c]);
         at += k[c];
     }
     return RCP_OK;
+}
+
+int rcp_r_sample_sorted(int seed, int sample_kind, int n_calls, const int64_t* n, const int64_t* k,
+                        int32_t* out) {
+    return r_sample_calls("rcp_r_sample_sorted", seed, sample_kind, n_calls, n, k, out, true);
+}
+
+int rcp_r_sample_int(int seed, int sample_kind, int n_calls, const int64_t* n, const int64_t* k,
+                     int32_t* out) {
+    return r_sample_calls("rcp_r_sample_int", seed, sample_kind, n_calls, n, k, out, false);
 }
 
 int rcp_r_rank_table(int n, int seed, int sample_kind, int* rank_out) {

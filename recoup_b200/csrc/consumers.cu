@@ -333,6 +333,11 @@ int column_medians(const double* m, int64_t n_rows, int64_t n_cols, int64_t ld, 
 }
 
 }  // namespace
+
+int sort_pairs_u64_i32(unsigned long long*& keys, int32_t*& vals, int64_t n) {
+    return sort_pairs(keys, vals, n, 0, 64);
+}
+
 }  // namespace rcp
 
 using namespace rcp;

@@ -344,6 +344,11 @@ int exclusive_scan_u32(const uint32_t* in, uint32_t* out, int64_t n, uint32_t* d
 // launch is sized for n_upper and the blocks beyond the real length return at once
 int exclusive_scan_u32_bounded(const uint32_t* in, uint32_t* out, int64_t n_upper, const uint32_t* n_dev,
                                uint32_t* d_total);
+// stable radix sort of (64-bit key, int32 value) pairs over all 64 key bits (consumers.cu)
+int sort_pairs_u64_i32(unsigned long long*& keys, int32_t*& vals, int64_t n);
+// sample.int(n, k) from a running base-R stream, dispatched as base R does (api.cu); out 1-based
+struct RRng;
+void r_sample_int(RRng& rng, int64_t n, int64_t k, int32_t* out);
 int exclusive_scan2_i64(const int64_t* in0, int64_t* out0, int64_t* d_total0, const int64_t* in1,
                         int64_t* out1, int64_t* d_total1, int64_t n);
 

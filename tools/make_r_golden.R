@@ -68,6 +68,23 @@ for (s in names(inp)) {
     write_cov(inp[[s]]$coverage,file.path(out,paste0("rna_",s,"_coverage.csv")))
     write_mat(inp[[s]]$profile,file.path(out,paste0("rna_",s,"_profile.csv")))
 }
+# ---- kmeans of the C1 profiles, both samples cbind-ed (kmeansDesign, util.R:140-197) ----
+inp <- coverageRef(test.input,genomeRanges=genes,region="tss",flank=c(2000,2000))
+inp <- profileMatrix(inp,flank=c(2000,2000),binParams=list(flankBinSize=0,
+    regionBinSize=100,sumStat="mean",interpolation="auto"),rc=NULL)
+km_x <- do.call("cbind",lapply(inp,function(s) s$profile))
+for (alg in c("Hartigan-Wong","Lloyd","MacQueen")) {
+    for (ns in c(1,20)) {
+        set.seed(42)
+        km <- kmeans(km_x,centers=5,iter.max=20,nstart=ns,algorithm=alg)
+        f <- file.path(out,paste0("kmeans_",gsub("-","",alg),"_nstart",ns,"_"))
+        writeLines(as.character(km$cluster),paste0(f,"cluster.txt"))
+        write.table(format(km$centers,digits=17),paste0(f,"centers.csv"),sep=",",quote=FALSE,
+            col.names=FALSE,row.names=FALSE)
+        writeLines(format(km$withinss,digits=17),paste0(f,"withinss.txt"))
+        writeLines(as.character(km$iter),paste0(f,"iter.txt"))
+    }
+}
 # ---- base-R known answers ----
 kat <- list()
 set.seed(42); kat$sample_42_10 <- sample(1:10)
