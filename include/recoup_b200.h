@@ -371,7 +371,10 @@ int rcp_coverage_rle_f32(int cov, int64_t first, int64_t count, int64_t* run_ptr
 /* ---------------------------------------------------------------- profile matrix ---------- */
 /* binCoverageMatrix(cvrg, binSize, stat, interpolation, flank, where) (profile.R:153-212) with
  * splitVector (util.R:15-85): writes an [n_regions x n_bins] block, column-major with leading
- * dimension ld >= n_regions, at `out`.  NULL coverage -> zero row (profile.R:191-197). */
+ * dimension ld >= n_regions, at `out`.  NULL coverage -> zero row (profile.R:191-197).
+ * n_bins <= 38399 (RCP_ERR_UNSUPPORTED above).  A segment shorter than n_bins is interpolated
+ * (util.R:17-73), which holds at most 5569 bins: with more bins such a segment is
+ * RCP_ERR_UNSUPPORTED (the matrix is then incomplete); without one, any n_bins up to 38399 works. */
 int rcp_bin_matrix(int cov, int where, int f1, int f2, int n_bins, int stat, int interp,
                    int seed, int sample_kind, double* out, int64_t ld, int mem);
 /* baseCoverageMatrix(cvrg, flank, where) (profile.R:100-151): [n_regions x n_cols] per-base

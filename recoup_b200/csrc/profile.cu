@@ -117,6 +117,16 @@ __device__ __forceinline__ int4 load4_g(const S* p) {
 template <class S>
 constexpr int ROWS_IN_FLIGHT = sizeof(S) == 2 ? 8 : 4;
 
+// the part of a lane's four elements at or after a bin edge (c of them lie before it): for
+// integers the row total minus the part before; for floats the sum of those elements, since
+// tot - before loses the small ones beside a large one (1e20 + 7 - 1e20 == 0)
+template <class V, class S, class A>
+__device__ __forceinline__ S after_edge(S tot, S before, int c, A a0, A a1, A a2, A a3) {
+    if constexpr (std::is_same<V, float>::value)
+        return (S)(c <= 0 ? a0 : 0) + (c <= 1 ? a1 : 0) + (c <= 2 ? a2 : 0) + (c <= 3 ? a3 : 0);
+    else return tot - before;
+}
+
 struct Seg {
     int a, b;   // [a, b) inside the region's coverage vector
 };
@@ -601,7 +611,7 @@ __device__ __forceinline__ void bin_mean_run(const BinArgs& p, const BinDesc* __
                                 for (int dd = 16; dd > 0; dd >>= 1) t += __shfl_xor_sync(0xffffffffu, t, dd);
                                 const int b0 = edge(k);
                                 if (lane == 0) out[(int64_t)k * p.ld] = p.scale * ((double)t / (double)(nxt - b0));
-                                acc = tot - before;
+                                acc = after_edge<V>(tot, before, c, a0, a1, a2, a3);
                                 k++;
                                 nxt = k < i1 ? edge(k + 1) : 0x7fffffff;
                             } else {
@@ -709,7 +719,7 @@ __device__ __forceinline__ void bin_wide_run(const BinArgs& p, const BinDesc* __
 #pragma unroll
                     for (int dd = 16; dd > 0; dd >>= 1) t += __shfl_xor_sync(0xffffffffu, t, dd);
                     if (lane == 0) out[(int64_t)k * p.ld] = p.scale * ((double)t / (double)(nxt - b0));
-                    acc = tot - before;
+                    acc = after_edge<V>(tot, before, c, a0, a1, a2, a3);
                     k++;
                     b0 = nxt;
                     nxt = k < i1 ? nxt + bsz + (int)((extra >> (k - i0)) & 1u) : 0x7fffffff;
@@ -1059,6 +1069,25 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
     int* d_rank = nullptr;
     int32_t* short_list = nullptr;
     unsigned int* short_count = nullptr;
+    BinDesc* d_desc = nullptr;
+    int32_t* long_list = nullptr;
+    unsigned int* long_count = nullptr;
+    struct Release {            // every exit, error returns included, frees the scratch buffers
+        int** rank;
+        int32_t** shorts;
+        unsigned int** short_n;
+        BinDesc** desc;
+        int32_t** longs;
+        unsigned int** long_n;
+        ~Release() {
+            dfree(*desc);
+            dfree(*longs);
+            dfree(*long_n);
+            dfree(*rank);
+            dfree(*shorts);
+            dfree(*short_n);
+        }
+    } release{&d_rank, &short_list, &short_count, &d_desc, &long_list, &long_count};
     RCP_TRY(dalloc(&d_rank, (size_t)n_bins));
     RCP_TRY(dalloc(&short_list, (size_t)R));
     RCP_TRY(dalloc(&short_count, 1));
@@ -1084,10 +1113,7 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
     a.short_list = short_list;
     a.short_count = short_count;
     const size_t edge_bytes = (((size_t)n_bins + 1 + 3) & ~(size_t)3) * sizeof(int);
-    if (edge_bytes > 150 * 1024) return fail(RCP_ERR_UNSUPPORTED, "more than ~38000 bins per segment");
-    BinDesc* d_desc = nullptr;
-    int32_t* long_list = nullptr;
-    unsigned int* long_count = nullptr;
+    if (edge_bytes > 150 * 1024) return fail(RCP_ERR_UNSUPPORTED, "more than 38399 bins per segment");
     if (stat == RCP_STAT_MEDIAN) {
         StageTimer t(ST_PROF_BIN);
         const size_t smem = edge_bytes;
@@ -1131,11 +1157,16 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
             cv.d_bound);
         RCP_LAUNCHED();
         // CTAs per SM and buffers per CTA: as much shared memory as possible in flight
-        int nbuf = 2;
         if (const char* e = getenv("RCP_BIN_CTAS")) per_sm = std::max(1, atoi(e));     // tuning
-        const size_t budget = 220u * 1024u / (size_t)per_sm - 1024u;
-        nbuf = (int)((budget - edge_bytes) / ((size_t)buf_ints * sizeof(int)));
-        nbuf = std::max(1, std::min(nbuf, NBUF_MAX));
+        // the edges of many bins leave no room for a staging buffer at this many CTAs per SM:
+        // fewer CTAs (150 KB of edges and one 48 KB buffer fit one CTA)
+        const int64_t buf_bytes = (int64_t)buf_ints * (int64_t)sizeof(int);
+        auto budget_at = [](int k) { return (int64_t)(220 * 1024 / k) - 1024; };
+        while (per_sm > 1 && budget_at(per_sm) - (int64_t)edge_bytes < buf_bytes) per_sm--;
+        const int64_t room = budget_at(per_sm) - (int64_t)edge_bytes;
+        if (room < buf_bytes)
+            return fail(RCP_ERR_UNSUPPORTED, "bin kernel does not fit (%zu bytes of bin edges)", edge_bytes);
+        const int nbuf = (int)std::min<int64_t>(room / buf_bytes, NBUF_MAX);
         const size_t smem = edge_bytes + (size_t)nbuf * buf_ints * sizeof(int);
         RCP_CUDA(cudaFuncSetAttribute(bin_mean_kernel<V>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)smem));
@@ -1167,8 +1198,18 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
     ia.short_list = short_list;
     ia.short_count = short_count;
     const size_t ismem = (size_t)n_bins * (4 * sizeof(double) + 2 * sizeof(int)) + 8 + sizeof(RRng);
-    if (ismem > 220 * 1024)
-        return fail(RCP_ERR_UNSUPPORTED, "interpolation supports at most ~5500 bins per segment");
+    if (ismem > 220 * 1024) {
+        // more bins than the interpolation kernel can hold: fine as long as no segment is shorter
+        // than the bin count.  The bin kernels have listed those; one read-back tells.
+        unsigned int n_short = 0;
+        RCP_CUDA(cudaMemcpyAsync(&n_short, short_count, sizeof(unsigned int), cudaMemcpyDeviceToHost,
+                                 g_ctx.stream));
+        RCP_CUDA(cudaStreamSynchronize(g_ctx.stream));
+        if (n_short == 0) return RCP_OK;
+        return fail(RCP_ERR_UNSUPPORTED,
+                    "%u segments are shorter than the %d bins; interpolation supports at most %d bins",
+                    n_short, n_bins, (int)((220 * 1024 - 8 - sizeof(RRng)) / (4 * sizeof(double) + 2 * sizeof(int))));
+    }
     if (ismem > 48 * 1024)
         RCP_CUDA(cudaFuncSetAttribute(interp_kernel<V>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)ismem));
@@ -1179,12 +1220,6 @@ int bin_matrix_impl(const Coverage& cv, int where, int f1, int f2, int n_bins, i
         interp_kernel<V><<<(unsigned)iblocks, 32, ismem, g_ctx.stream>>>(ia);
         RCP_LAUNCHED();
     }
-    dfree(d_desc);
-    dfree(long_list);
-    dfree(long_count);
-    dfree(d_rank);
-    dfree(short_list);
-    dfree(short_count);
     return RCP_OK;
 }
 
