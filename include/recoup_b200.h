@@ -475,6 +475,26 @@ int rcp_kmeans(const double* x, int64_t m, int64_t p, int64_t ld, int k, int nst
 int rcp_r_sample_int(int seed, int sample_kind, int n_calls, const int64_t* n, const int64_t* k,
                      int32_t* out /* host, sum(k) */);
 
+/* ---------------------------------------------------------------- hierarchical clustering - */
+/* rcp_hclust: hclust(dist(x), method = "complete") -- stats::hclust of the Euclidean distances of
+ *   the rows, as ComplexHeatmap clusters heat-map rows (cluster_rows = TRUE) for orderBy$what =
+ *   "hc<n>" / "hca".  x: column-major n x p, leading dimension ld; `mem` says where x, merge,
+ *   height and order live.  Distances use R_euclidean's floating-point operations in its order
+ *   (no FMA, correctly rounded sqrt); the merges are hclust.f's (F. Murtagh, as R ships it) and
+ *   merge / order are HCASS2's, so all three equal R's bit for bit:
+ *     merge:  column-major (n-1) x 2; singletons -i (1-based row), clusters +s (their step);
+ *             a singleton first in a mixed row, two clusters ascending;
+ *     height: the n-1 merge heights;  order: the leaves left to right, 1-based.
+ *   The n x n distance matrix (8 n^2 bytes) lives on the device only and is released before return.
+ *   Errors: n < 2 ("must have n >= 2 objects to cluster"), n > 65536 ("size cannot be NA nor exceed
+ *   65536"), p < 1 or ld < n: RCP_ERR_ARG.  A method other than RCP_HCLUST_COMPLETE:
+ *   RCP_ERR_UNSUPPORTED.  A non-finite x or a distance >= 1e300 (hclust.f's INF): RCP_ERR_DATA.
+ *   Too little device memory for the matrix: RCP_ERR_CUDA, naming the bytes it needs. */
+#define RCP_HCLUST_COMPLETE 3      /* index in R's METHODS vector of hclust() */
+int rcp_hclust(const double* x, int64_t n, int64_t p, int64_t ld, int method, int mem,
+               int32_t* merge /* (n-1) x 2, column-major, R's signs */,
+               double* height /* n-1 */, int32_t* order /* n, 1-based */);
+
 /* ---------------------------------------------------------------- multi-GPU helper -------- */
 /* Scatter a row block into the gathered matrix: dst[row_index[i] + c*ld_dst] =
  * src[i + c*ld_src] for i < n_rows, c < n_cols (all pointers on the device).  Used after the

@@ -7,8 +7,8 @@ compute call requires a B200 -- there is no CPU fallback.
 """
 from . import _lib
 from ._lib import RecoupError, init, set_coverage_path, shutdown
-from .consumers import (NamedVector, calcPlotProfiles, colProfile, heatmapScale, kmeans, kmeansDesign,
-                        matrixQuantile, orderProfiles, rowStat, sortIndex)
+from .consumers import (NamedVector, calcPlotProfiles, colProfile, hclust, heatmapClusters, heatmapScale, kmeans,
+                        kmeansDesign, matrixQuantile, orderProfiles, rowStat, sortIndex)
 from .coverage import (CoverageList, DeviceReads, calcCoverage, coverageRef, coverageRnaRef,
                        device_reads, set_verbose)
 from .preprocess import SelectedGRanges, preprocessRanges, readRanges, sampleSorted, widthQuantile
@@ -26,5 +26,5 @@ __all__ = [
     "heatmapScale", "colProfile", "rowStat", "sortIndex", "matrixQuantile", "preprocessRanges",
     "readRanges", "SelectedGRanges", "sampleSorted", "widthQuantile", "readBam", "readBed", "readRangesFile",
     "decodeBam", "DecodedGRanges", "ScanBamParam", "scanBamFlag", "readBigWig", "BigWigTrack",
-    "kmeans", "kmeansDesign", "NamedVector",
+    "kmeans", "kmeansDesign", "NamedVector", "hclust", "heatmapClusters",
 ]

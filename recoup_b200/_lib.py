@@ -119,6 +119,7 @@ SIGNATURES = {
     "rcp_kmeans": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                              C.c_int, C.c_int, _vp, _vp, _vp, _vp, _f64p, _ip, _ip, _ip]),
     "rcp_r_sample_int": (C.c_int, [C.c_int, C.c_int, C.c_int, _i64p, _i64p, _vp]),
+    "rcp_hclust": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, _vp, _vp, _vp]),
 }
 
 

@@ -6,6 +6,8 @@ over librecoup_b200.so (SURVEY 8f, N4):
     heatmapScale(input, ...)             upper colour limit from quantiles      plot.R:513-545
     kmeans(x, centers, ...)              stats::kmeans as kmeansDesign calls it
     kmeansDesign(input, design, kmParams) heat-map clusters as a design column  util.R:140-197
+    hclust(x, method)                    stats::hclust(dist(x)) of heat-map rows
+    heatmapClusters(input, opts, split)  the cluster_rows dendrograms of orderBy = "hc<n>" / "hca"
 
 `opts` is the nested dict of the reference (`opts["plotParams"]["sumStat"]`, ...).  Matrices are
 the `ProfileMatrix` objects profileMatrix() returns (host, column-major); they are staged to the
@@ -246,4 +248,76 @@ def kmeansDesign(input, design=None, kmParams=None):
         if len(v) != labels.shape[0]:
             raise ValueError("design column %s has %d rows, the profiles %d" % (col, len(v), labels.shape[0]))
     out["Cluster"] = labels
+    return out
+
+
+_HC_METHODS = ("ward.D", "single", "complete", "average", "mcquitty", "median", "centroid", "ward.D2")
+
+
+def hclust(x, method="complete"):
+    """`hclust(dist(x), method)` on the device (rcp_hclust): Euclidean distances of the rows, then
+    the merges of hclust.f, bit for bit as R computes them.  Only method = "complete" (hclust's
+    default, and ComplexHeatmap's) is implemented.  Returns dict(merge ((n-1) x 2, R's signs),
+    height, order (1-based), labels (x.rownames for a ProfileMatrix, else None), method,
+    dist_method)."""
+    if method == "ward":
+        method = "ward.D"
+    hits = [mm for mm in _HC_METHODS if mm == method] or [mm for mm in _HC_METHODS if method and
+                                                          mm.startswith(method)]
+    if not hits:
+        raise ValueError("invalid clustering method %s" % method)
+    if len(hits) > 1:
+        raise ValueError("ambiguous clustering method %s" % method)
+    m = _f(x)
+    n, p = m.shape
+    _lib.ensure_init()
+    merge = np.empty(2 * max(n - 1, 1), dtype=np.int32)
+    height = np.empty(max(n - 1, 1), dtype=np.float64)
+    order = np.empty(max(n, 1), dtype=np.int32)
+    _lib.check(_lib.lib.rcp_hclust(_vp(m), n, p, max(n, 1), _HC_METHODS.index(hits[0]) + 1, _lib.MEM_HOST,
+                                   _vp(merge), _vp(height), _vp(order)))
+    return {"merge": merge.reshape((n - 1, 2), order="F"), "height": height, "order": order,
+            "labels": getattr(x, "rownames", None), "method": hits[0], "dist_method": "euclidean"}
+
+
+def heatmapClusters(input, opts, split=None):
+    """The row dendrograms of recoup's heat maps (cluster_rows) for opts["orderBy"]["what"] =
+    "hc<n>" (the profile of sample n, 1-based) or "hca" (the cbind of every sample's profile in
+    sample order, as kmeansDesign builds it); any other `what` returns None, and orderBy$order
+    does not apply to a dendrogram.  Without `split` the result is hclust() of that matrix.  With
+    `split` (one label per row, e.g. a design column or kmeansDesign's Cluster) every level's rows
+    are clustered on their own, as ComplexHeatmap does with row_split: a list of (level, rows
+    (1-based), hclust) per level in factor() order (sorted labels); a one-row level gets None."""
+    what = opts["orderBy"].get("what", "none")
+    m = re.match(r"^hc(\d+|a)$", what or "")
+    if not m:
+        return None
+    if m.group(1) == "a":
+        mats = [s["profile"] for s in input]
+    else:
+        ref = int(m.group(1))
+        if not 1 <= ref <= len(input):
+            raise ValueError("orderBy$what = %s: there are %d samples" % (what, len(input)))
+        mats = [input[ref - 1]["profile"]]
+    names = getattr(mats[0], "rownames", None)
+    x = np.asfortranarray(np.hstack([np.asarray(mm, dtype=np.float64) for mm in mats]))
+    if split is None:
+        if names is not None:
+            from .profile import ProfileMatrix
+            x = ProfileMatrix(x, rownames=names)
+        return hclust(x)
+    lab = np.asarray(split, dtype=object)
+    if lab.shape[0] != x.shape[0]:
+        raise ValueError("split has %d labels, the profiles %d rows" % (lab.shape[0], x.shape[0]))
+    out = []
+    for level in sorted(set(lab.tolist())):
+        rows = np.flatnonzero(lab == level)
+        hc = None
+        if rows.shape[0] >= 2:
+            sub = np.asfortranarray(x[rows])
+            if names is not None:
+                from .profile import ProfileMatrix
+                sub = ProfileMatrix(sub, rownames=[names[r] for r in rows])
+            hc = hclust(sub)
+        out.append((level, (rows + 1).astype(np.int32), hc))
     return out

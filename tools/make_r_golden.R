@@ -85,6 +85,12 @@ for (alg in c("Hartigan-Wong","Lloyd","MacQueen")) {
         writeLines(as.character(km$iter),paste0(f,"iter.txt"))
     }
 }
+# ---- hclust(dist(km_x)) of the same profiles (the heat-map rows of orderBy = "hca") ----
+hc <- hclust(dist(km_x))
+write.table(hc$merge,file.path(out,"hclust_merge.csv"),sep=",",quote=FALSE,col.names=FALSE,
+    row.names=FALSE)
+writeLines(sprintf("%.17g",hc$height),file.path(out,"hclust_height.txt"))
+writeLines(as.character(hc$order),file.path(out,"hclust_order.txt"))
 # ---- base-R known answers ----
 kat <- list()
 set.seed(42); kat$sample_42_10 <- sample(1:10)
