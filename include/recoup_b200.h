@@ -132,7 +132,9 @@ int rcp_coverage_path_info(int cov, int* path, int64_t* candidates);
  * chromosome id, start < 1, ...) is reported by the FIRST call that uses the reads handle
  * (rcp_coverage, rcp_coverage_list) instead of by the load itself.  Host arrays passed to a
  * deferred load must stay unchanged until that call returns.  The reference validates inside
- * GRanges construction; which call raises is the only difference. */
+ * GRanges construction; which call raises is the only difference.  A handle that failed its
+ * validation keeps the error: every later call that uses it (rcp_coverage*, rcp_coverage_list,
+ * rcp_coverage_profile) returns the same code and message; rcp_reads_info and rcp_reads_free work. */
 int rcp_set_deferred_validation(int on);
 
 /* ---------------------------------------------------------------- base-R RNG -------------- */

@@ -59,7 +59,8 @@ constexpr int ST = RCP_SPLIT_ST;                      // threads of the split ke
 constexpr int ROUND_VEC = 2048;                       // 16-byte vectors (of 4 reads) per CTA round
 constexpr int VPT = ROUND_VEC / ST;                   // vectors per thread and round
 constexpr int SLAB = 64;                              // chunks a warp takes from the pool at a time
-constexpr int MIN_P = 16, MAX_P = 22;                 // position bits of a candidate word
+// position bits of a candidate word: split_position_bits (rcp_internal.cuh), 16..22, for NG groups
+static_assert(NG == 1024, "split_position_bits assumes at most 1024 groups");
 constexpr int GT = 1024;                              // threads of the group kernel
 constexpr int CS = 1024;                              // threads of the chunk-sort kernels
 constexpr int WT = 7 * ROW;                           // outputs of a warp tile (896); regions <= 1024 bp are ONE tile
@@ -987,8 +988,9 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // anywhere.  Persistent warps; descriptors are fetched two tiles ahead, and the first CBUF candidate
 // words of the next tile are copied into shared memory (cp.async) during the current tile.  The
 // staged range starts at the 16-byte boundary below the tile's first candidate and ends at the one
-// above its last: the extra words belong to neighbouring sub-bins (or are the zero words of a
-// hole), start before the reach of the widest read or after the tile, and clip to nothing.
+// above its last.  The extra words belong to neighbouring sub-bins -- possibly of another group, or
+// more than 2^(P-1) positions away, where the P-bit distance to the tile wraps and a read far away
+// would land inside the tile -- so they are applied as zero words (width 0, never a hit).
 // Longer candidate lists continue from global memory, 128 at a time.
 #ifndef RCP_WTILE_OCC
 #define RCP_WTILE_OCC 4
@@ -1057,7 +1059,8 @@ sp_wtile_kernel(int64_t T, const SpDesc* __restrict__ desc, const uint32_t* __re
         __syncwarp();
         bool hit = false;
         const uint32_t a0 = d.c0 & ~3u;
-        const uint32_t words = (d.c0 - a0) + d.n;                       // from a0 on
+        const uint32_t lead = d.c0 - a0;
+        const uint32_t words = lead + d.n;                              // from a0 on
         const uint32_t staged = min((words + 3u) & ~3u, (uint32_t)CBUF);
         const uint32_t mine_a = cs_a + (uint32_t)buf * (CBUF * 4) + lane * 4u;
         const uint32_t diff_a = (uint32_t)__cvta_generic_to_shared(diff);
@@ -1065,8 +1068,11 @@ sp_wtile_kernel(int64_t T, const SpDesc* __restrict__ desc, const uint32_t* __re
         auto apply_all = [&](auto rev_tag) {
             constexpr bool REV = decltype(rev_tag)::value;
 #pragma unroll 4
-            for (uint32_t i = lane; i < staged; i += 32)
-                hit |= sp_apply_fast<STRANDED, REV>(lds32(mine_a + (i - lane) * 4u), d.cts, d.tlen, cls, P, diff_a);
+            for (uint32_t i = lane; i < staged; i += 32) {
+                uint32_t e = lds32(mine_a + (i - lane) * 4u);
+                if (i < lead || i >= words) e = 0u;                     // outside [c0, c0 + n)
+                hit |= sp_apply_fast<STRANDED, REV>(e, d.cts, d.tlen, cls, P, diff_a);
+            }
 #if defined(RCP_EXP_MODE) && RCP_EXP_MODE == 2     // timing experiment: staged candidates only (wrong results)
             if (d.tlen >= 0) return;
 #endif
@@ -1564,8 +1570,7 @@ static SplitGeom split_geometry(const ReadsIdx& rd) {
     SplitGeom g;
     const int64_t span = (int64_t)rd.chrom_off[(size_t)rd.n_chrom];
     g.words = (int)((span >> (BLK_SHIFT + 4)) + 2);
-    g.P = MIN_P;
-    while (g.P < MAX_P && ((span + (1ll << g.P) - 1) >> g.P) > NG) g.P++;
+    g.P = split_position_bits(span);
     g.n_groups = (int)std::max<int64_t>(1, (span + (1ll << g.P) - 1) >> g.P);
     g.nb = 1 << (g.P - SUB_SHIFT);
     g.pmask = (1u << g.P) - 1u;
@@ -1664,10 +1669,10 @@ static int split_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32
                       int strand_filter, int mem, Coverage* cv, const FusedReq* fz) {
     const bool stranded = !((strand_filter == RCP_STRAND_ANY) && (ignore_strand || strand == nullptr));
     const bool st_arr = stranded && rd.d_strand != nullptr;      // strandless reads are all '*'
+    if (rd.failed != RCP_OK) return reads_finish(rd);              // a deferred load that failed
     const int64_t span = (int64_t)rd.chrom_off[(size_t)rd.n_chrom];
     const int words = (int)((span >> (BLK_SHIFT + 4)) + 2);
-    int P = MIN_P;
-    while (P < MAX_P && ((span + (1ll << P) - 1) >> P) > NG) P++;
+    const int P = split_position_bits(span);
     const int n_groups = (int)std::max<int64_t>(1, (span + (1ll << P) - 1) >> P);
     const int wbits = 32 - P - (stranded ? 2 : 0);
     if (n_groups > NG || rd.n >= 0x7ffffff0ll || sp_split_smem(words) > SP_SMEM_MAX)

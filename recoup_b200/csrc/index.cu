@@ -737,18 +737,19 @@ int reads_pending_items(ReadsIdx& r, FetchItem* items, int* n) {
 }
 
 int reads_resolve(ReadsIdx& r) {
-    if (!r.pending) return RCP_OK;
-    FetchItem items[4];
-    int n = 0;
-    reads_pending_items(r, items, &n);
-    RCP_TRY(fetch_and_sync(items, n));
+    if (r.pending) {
+        FetchItem items[4];
+        int n = 0;
+        reads_pending_items(r, items, &n);
+        RCP_TRY(fetch_and_sync(items, n));
+    }
     return reads_finish(r);
 }
 
+namespace {
+
 // what follows the fetch of the status words (the caller has synchronised)
-int reads_finish(ReadsIdx& r) {
-    if (!r.pending) return RCP_OK;
-    r.pending = false;
+int finish_pending(ReadsIdx& r) {
     const int64_t n = r.n;
     const unsigned int h_err = r.h_err;
     dfree(r.pd_err);
@@ -762,8 +763,10 @@ int reads_finish(ReadsIdx& r) {
                     (long long)n);
     // (nearly) every read has the same width w -- fixed-length or fragment-extended libraries;
     // the few that do not (trimmed at a chromosome end) live in a correction source.  Then the
-    // sorted ends are the sorted starts shifted by w: one array, one sort.
-    if (h_err == 0 && n > 0 && r.h_w[1] > 0 && r.h_w[0] <= r.pd_exc_cap) {
+    // sorted ends are the sorted starts shifted by w: one array, one sort.  (start + w must not
+    // wrap around 2^32: a genome that ends within w of it keeps the second array.)
+    const bool w_fits = (uint64_t)r.chrom_off[(size_t)r.n_chrom] + r.h_w[1] <= 0xffffffffull;
+    if (h_err == 0 && n > 0 && r.h_w[1] > 0 && r.h_w[0] <= r.pd_exc_cap && w_fits) {
         r.uniform_w = r.h_w[1];
         r.n_exc = (int64_t)r.h_w[0];
     } else {
@@ -784,6 +787,24 @@ int reads_finish(ReadsIdx& r) {
     r.max_width = (uint32_t)r.h_cnt[3];
     r.n_long = (int64_t)r.h_w[2];
     if (r.pd_eager_index) RCP_TRY(reads_build_class(r, CLS_ALL));
+    return RCP_OK;
+}
+
+}  // namespace
+
+// A failed validation leaves the handle without its widths and class counts, so its error is kept
+// and returned again by every later call: a retry must not compute a coverage from such a handle.
+int reads_finish(ReadsIdx& r) {
+    if (r.pending) {
+        r.pending = false;
+        const int rc = finish_pending(r);
+        if (rc != RCP_OK) {
+            r.failed = rc;
+            r.failed_msg = rcp_last_error();
+        }
+        return rc;
+    }
+    if (r.failed != RCP_OK) return fail(r.failed, "%s", r.failed_msg.c_str());
     return RCP_OK;
 }
 

@@ -258,6 +258,10 @@ struct ReadsIdx {
     uint32_t* pd_run_first = nullptr;
     uint32_t pd_exc_cap = 0;
     bool pd_eager_index = false;
+    // a deferred load whose validation failed: the handle keeps its error (code and message) and
+    // every later call that uses it reports that error again (its fields were never filled in)
+    int failed = RCP_OK;
+    std::string failed_msg;
     unsigned int h_err = 0, h_w[4] = {0, 0, 0, 0}, h_total = 0;   // h_w: exceptions, width, reads wider than long_thr
     // reads wider than the packed candidate word of the split path (counted by the map kernel, so
     // that the handle's long-read list needs no counting pass and no host synchronisation)
@@ -274,7 +278,8 @@ inline int split_position_bits(int64_t span) {
     return P;
 }
 
-// deferred validation: the fetch items of a pending handle (appended), and what follows the fetch
+// deferred validation: the fetch items of a pending handle (appended), and what follows the fetch.
+// reads_finish and reads_resolve return the error of a failed validation on every call after it too.
 int reads_pending_items(ReadsIdx& r, FetchItem* items, int* n);
 int reads_finish(ReadsIdx& r);
 int reads_resolve(ReadsIdx& r);     // fetch + finish when pending
