@@ -436,6 +436,21 @@ int rcp_sort_keys_u32(uint32_t* keys, int64_t n, int key_bits, int mem);
 int rcp_matrix_col_profile(const double* m, int64_t n_rows, int64_t n_cols, int64_t ld, int stat,
                            int log2_scale, int mem, double* center /* n_cols */,
                            double* spread /* n_cols */);
+/* rcp_matrix_group_col_profile: the same curve and band per group of rows, the curves of
+ *   calcDesignPlotProfiles (one per design level).  Row i belongs to group codes[i], 1-based as R
+ *   stores a factor (as.integer(f), or rcp_kmeans's cluster); a code <= 0 (NA_integer_ included)
+ *   excludes the row; codes == NULL puts every row in group 1.  center[g + c * n_groups] and
+ *   spread[g + c * n_groups] (column-major n_groups x n_cols) are exactly what
+ *   rcp_matrix_col_profile returns for the rows of group g + 1; a group without rows gets NaN in
+ *   both.  m, codes and both outputs live in `mem`.  Errors: RCP_ERR_ARG as rcp_matrix_col_profile,
+ *   and n_groups < 1; RCP_ERR_DATA: a code greater than n_groups (found on the device);
+ *   RCP_ERR_UNSUPPORTED: more than 2^31-1 cells, or n_groups * n_cols above 2^31-1.  The launches
+ *   and passes over the matrix do not depend on n_groups; the matrix is copied once into group
+ *   order unless there is one group and no excluded row. */
+int rcp_matrix_group_col_profile(const double* m, int64_t n_rows, int64_t n_cols, int64_t ld,
+                                 const int32_t* codes /* n_rows, or NULL */, int n_groups, int stat,
+                                 int log2_scale, int mem, double* center /* n_groups x n_cols */,
+                                 double* spread /* n_groups x n_cols */);
 int rcp_matrix_row_stat(const double* m, int64_t n_rows, int64_t n_cols, int64_t ld, int what, int mem,
                         double* out /* n_rows */);
 int rcp_order(const double* v, int64_t n, int decreasing, int mem, int32_t* ix /* n */, int64_t* n_out);

@@ -7,8 +7,9 @@ compute call requires a B200 -- there is no CPU fallback.
 """
 from . import _lib
 from ._lib import RecoupError, init, set_coverage_path, shutdown
-from .consumers import (NamedVector, calcPlotProfiles, colProfile, hclust, heatmapClusters, heatmapScale, kmeans,
-                        kmeansDesign, matrixQuantile, orderProfiles, rowStat, sortIndex)
+from .consumers import (NamedVector, calcDesignPlotProfiles, calcPlotProfiles, colProfile, groupColProfile, hclust,
+                        heatmapClusters, heatmapScale, kmeans, kmeansDesign, matrixQuantile, orderProfiles, rowStat,
+                        sortIndex)
 from .coverage import (CoverageList, DeviceReads, calcCoverage, coverageRef, coverageRnaRef,
                        device_reads, set_verbose)
 from .preprocess import SelectedGRanges, preprocessRanges, readRanges, sampleSorted, widthQuantile
@@ -26,5 +27,6 @@ __all__ = [
     "heatmapScale", "colProfile", "rowStat", "sortIndex", "matrixQuantile", "preprocessRanges",
     "readRanges", "SelectedGRanges", "sampleSorted", "widthQuantile", "readBam", "readBed", "readRangesFile",
     "decodeBam", "DecodedGRanges", "ScanBamParam", "scanBamFlag", "readBigWig", "BigWigTrack",
-    "kmeans", "kmeansDesign", "NamedVector", "hclust", "heatmapClusters",
+    "kmeans", "kmeansDesign", "NamedVector", "hclust", "heatmapClusters", "calcDesignPlotProfiles",
+    "groupColProfile",
 ]

@@ -50,6 +50,8 @@ SIGNATURES = {
     "rcp_reads_load": (C.c_int, [C.c_int64, _vp, _vp, _vp, _vp, C.c_int, _i64p, C.c_int, C.c_int, _ip]),
     "rcp_matrix_col_profile": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int,
                                          _vp, _vp]),
+    "rcp_matrix_group_col_profile": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, _vp, C.c_int, C.c_int, C.c_int,
+                                               C.c_int, _vp, _vp]),
     "rcp_matrix_row_stat": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, _vp]),
     "rcp_order": (C.c_int, [_vp, C.c_int64, C.c_int, C.c_int, _vp, _i64p]),
     "rcp_matrix_quantile": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, _vp, C.c_int, C.c_int, _vp]),

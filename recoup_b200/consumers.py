@@ -2,6 +2,7 @@
 over librecoup_b200.so (SURVEY 8f, N4):
 
     calcPlotProfiles(input, opts, ...)   average curve + band per sample        plot.R:949-990
+    calcDesignPlotProfiles(input, design, opts)  the same per design level and sample
     orderProfiles(input, opts)           heat-map row order (sum / max / avg)   plot.R:1035-1150
     heatmapScale(input, ...)             upper colour limit from quantiles      plot.R:513-545
     kmeans(x, centers, ...)              stats::kmeans as kmeansDesign calls it
@@ -64,6 +65,113 @@ def calcPlotProfiles(input, opts, sdim=2, rc=None):
         center, spread = colProfile(x["profile"], pp.get("sumStat", "mean"), pp.get("signalScale", "natural"))
         out.append({"profile": center, "upper": center + spread, "lower": center - spread})
     return out
+
+
+def groupColProfile(mat, codes, n_groups, avgfun="mean", scale="natural"):
+    """colProfile of every group of rows (rcp_matrix_group_col_profile): row i belongs to group
+    codes[i], 1-based as R stores a factor; a code <= 0 excludes the row; codes None puts every
+    row in group 1.  Returns (center, spread), each n_groups x n_cols; a group without rows is NaN."""
+    if avgfun not in ("mean", "median"):
+        raise ValueError("sumStat must be mean or median")
+    m = _f(mat)
+    c = None
+    if codes is not None:
+        c = np.ascontiguousarray(codes, dtype=np.int32)
+        if c.shape != (m.shape[0],):
+            raise ValueError("%d codes for %d rows" % (c.size, m.shape[0]))
+    g = int(n_groups)
+    _lib.ensure_init()
+    center = np.empty((max(g, 0), m.shape[1]), dtype=np.float64, order="F")
+    spread = np.empty((max(g, 0), m.shape[1]), dtype=np.float64, order="F")
+    _lib.check(_lib.lib.rcp_matrix_group_col_profile(_vp(m), m.shape[0], m.shape[1], max(m.shape[0], 1),
+                                                     None if c is None else _vp(c), g, _lib.STAT[avgfun],
+                                                     1 if scale == "log2" else 0, _lib.MEM_HOST, _vp(center),
+                                                     _vp(spread)))
+    return center, spread
+
+
+def _design_levels(design, n_rows):
+    """The levels of a design (dict of equal-length label columns): the label, or the tuple of
+    labels across columns, of every combination that occurs, ordered as factor() orders each
+    column (sorted labels), first column slowest; a row with a None label is in no level.
+    Returns (levels, codes): codes[i] is the 1-based level of row i, 0 when excluded."""
+    if not design:
+        raise ValueError("calcDesignPlotProfiles needs a design with at least one column")
+    cols = [np.asarray(v, dtype=object) for v in design.values()]
+    for name, v in zip(design, cols):
+        if v.ndim != 1 or v.shape[0] != n_rows:
+            raise ValueError("design column %s has %d rows, the profiles %d" % (name, v.size, n_rows))
+    keep = np.ones(n_rows, dtype=bool)
+    for v in cols:
+        keep &= np.array([lab is not None for lab in v.tolist()], dtype=bool)
+    ranks = []
+    for v in cols:
+        labels = sorted(set(v[keep].tolist()))
+        pos = {lab: i for i, lab in enumerate(labels)}
+        ranks.append(np.array([pos[lab] if k else -1 for lab, k in zip(v.tolist(), keep)], dtype=np.int64))
+    combo = {}
+    for i in np.flatnonzero(keep):
+        key = tuple(int(r[i]) for r in ranks)
+        if key not in combo:
+            combo[key] = tuple(v[i] for v in cols)
+    order = sorted(combo)
+    code_of = {key: j + 1 for j, key in enumerate(order)}
+    codes = np.zeros(n_rows, dtype=np.int32)
+    for i in np.flatnonzero(keep):
+        codes[i] = code_of[tuple(int(r[i]) for r in ranks)]
+    levels = [combo[key][0] if len(cols) == 1 else combo[key] for key in order]
+    return levels, codes
+
+
+def _group_profiles(mats, codes, n_groups, avgfun, log2):
+    """(center, spread) of rcp_matrix_group_col_profile for every matrix, each n_groups x n_cols;
+    the codes are uploaded once, every matrix is staged and reduced on the device."""
+    import torch
+    _lib.ensure_init()
+    dev = torch.device("cuda", _lib._initialised_device)
+    d_codes = torch.from_numpy(np.ascontiguousarray(codes, dtype=np.int32)).to(dev)
+    out = []
+    for m in mats:
+        dm = torch.from_numpy(np.ascontiguousarray(m.T)).to(dev)        # m^T row-major = m column-major
+        center = torch.empty((m.shape[1], n_groups), dtype=torch.float64, device=dev)
+        spread = torch.empty_like(center)
+        torch.cuda.synchronize(dev)
+        _lib.check(_lib.lib.rcp_matrix_group_col_profile(
+            C.c_void_p(dm.data_ptr()), m.shape[0], m.shape[1], max(m.shape[0], 1), C.c_void_p(d_codes.data_ptr()),
+            n_groups, _lib.STAT[avgfun], log2, _lib.MEM_DEVICE, C.c_void_p(center.data_ptr()),
+            C.c_void_p(spread.data_ptr())))
+        _lib.check(_lib.lib.rcp_sync())
+        out.append((center.cpu().numpy().T, spread.cpu().numpy().T))
+    return out
+
+
+def calcDesignPlotProfiles(input, design, opts):
+    """The curves of a design-split profile plot (calcDesignPlotProfiles, parity unpinned): for
+    every level of `design` (see _design_levels; kmeansDesign's result can be passed as is) and
+    every sample, calcPlotProfiles over that level's rows.  Returns one (level, rows (1-based
+    int32), [dict(profile, upper, lower) per sample]) per level.  The level codes go to the
+    device once and serve every sample."""
+    pp = opts["plotParams"]
+    if pp.get("smooth"):
+        raise NotImplementedError("plotParams$smooth: smooth.spline is outside the accelerated path")
+    avgfun = pp.get("sumStat", "mean")
+    if avgfun not in ("mean", "median"):
+        raise ValueError("sumStat must be mean or median")
+    log2 = 1 if pp.get("signalScale", "natural") == "log2" else 0
+    n_rows = np.asarray(input[0]["profile"]).shape[0] if input else 0
+    levels, codes = _design_levels(design, n_rows)
+    G = len(levels)
+    rows = [(np.flatnonzero(codes == j + 1) + 1).astype(np.int32) for j in range(G)]
+    curves = [[] for _ in range(G)]
+    if G and input:
+        mats = [_f(x["profile"]) for x in input]
+        for m in mats:
+            if m.shape[0] != n_rows:
+                raise ValueError("every sample's profile must have %d rows" % n_rows)
+        for cen, spr in _group_profiles(mats, codes, G, avgfun, log2):
+            for j in range(G):
+                curves[j].append({"profile": cen[j].copy(), "upper": cen[j] + spr[j], "lower": cen[j] - spr[j]})
+    return [(levels[j], rows[j], curves[j]) for j in range(G)]
 
 
 def rowStat(mat, what):
