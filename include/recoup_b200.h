@@ -409,7 +409,7 @@ int rcp_coverage_profile(int reads, int64_t n_regions, const int32_t* chrom,
 
 /* ---------------------------------------------------------------- diagnostics ------------- */
 /* Sort n 32-bit keys whose values are < 2^key_bits with the library's index sort (in place).
- * Exposed so the hand-written sort can be tested directly against a host sort. */
+ * Exposed so that the index sort can be tested against a host sort. */
 int rcp_sort_keys_u32(uint32_t* keys, int64_t n, int key_bits, int mem);
 
 /* ---------------------------------------------------------------- matrix consumers -------- */

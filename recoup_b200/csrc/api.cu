@@ -1295,14 +1295,17 @@ int rcp_sort_keys_u32(uint32_t* keys, int64_t n, int key_bits, int mem) {
     if (n < 0 || key_bits < 1 || key_bits > 32 || (n > 0 && keys == nullptr))
         return fail(RCP_ERR_ARG, "rcp_sort_keys_u32: bad argument");
     if (n == 0) return RCP_OK;
-    if (mem == RCP_MEM_DEVICE) return sort_keys_u32(keys, n, key_bits);
+    // the sort may hand back another buffer than the one it was given: it sorts a copy owned here
+    const bool dev = mem == RCP_MEM_DEVICE;
     uint32_t* d = nullptr;
     RCP_TRY(dalloc(&d, (size_t)n));
-    RCP_CUDA(cudaMemcpyAsync(d, keys, (size_t)n * 4, cudaMemcpyHostToDevice, g_ctx.stream));
-    int rc = sort_keys_u32(d, n, key_bits);
+    RCP_CUDA(cudaMemcpyAsync(d, keys, (size_t)n * 4, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
+                             g_ctx.stream));
+    int rc = sort_keys(d, n, 0, key_bits);
     if (rc == RCP_OK) {
-        cudaError_t e = cudaMemcpyAsync(keys, d, (size_t)n * 4, cudaMemcpyDeviceToHost, g_ctx.stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(g_ctx.stream);
+        cudaError_t e = cudaMemcpyAsync(keys, d, (size_t)n * 4, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost,
+                                        g_ctx.stream);
+        if (e == cudaSuccess && !dev) e = cudaStreamSynchronize(g_ctx.stream);
         if (e != cudaSuccess) rc = fail(RCP_ERR_CUDA, "sort copy failed: %s", cudaGetErrorString(e));
     }
     dfree(d);

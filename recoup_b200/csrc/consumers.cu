@@ -9,9 +9,8 @@
 // leaves it on the device.  The curve and band of calcPlotProfiles are computed per group of rows
 // (calcDesignPlotProfiles: one curve per design level; a single group is calcPlotProfiles): means
 // are chunked exact-sum reductions, medians a segmented radix sort.  Row sums are plain streaming
-// reductions (one thread per row); orderings and quantiles go through CUB's radix sort on
-// order-preserving 64-bit keys.
-#include <cub/device/device_radix_sort.cuh>
+// reductions (one thread per row); orderings and quantiles go through the library's radix sort
+// (sort.cu) on order-preserving 64-bit keys.
 #include <cub/device/device_segmented_radix_sort.cuh>
 #include <thrust/iterator/counting_iterator.h>
 #include <thrust/iterator/transform_iterator.h>
@@ -149,48 +148,6 @@ __global__ void quantile_kernel(const unsigned long long* __restrict__ sorted, i
     const double xl = key_value(sorted[(int64_t)lo]), xh = key_value(sorted[(int64_t)hi]);
     const double h = index - lo;
     out[j] = (index > lo && xh != xl) ? (1.0 - h) * xl + h * xh : xl;
-}
-
-int sort_keys_u64(unsigned long long*& keys, int64_t n) {
-    if (n > 0x7fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^31-1 values in one sort");
-    unsigned long long* alt = nullptr;
-    RCP_TRY(dalloc(&alt, (size_t)n));
-    cub::DoubleBuffer<unsigned long long> buf(keys, alt);
-    size_t tmp_bytes = 0;
-    RCP_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, buf, (int)n, 0, 64, g_ctx.stream));
-    uint8_t* tmp = nullptr;
-    RCP_TRY(dalloc(&tmp, tmp_bytes));
-    RCP_CUDA(cub::DeviceRadixSort::SortKeys(tmp, tmp_bytes, buf, (int)n, 0, 64, g_ctx.stream));
-    g_ctx.launches += 9;
-    dfree(tmp);
-    if (buf.Current() != keys) std::swap(keys, alt);
-    dfree(alt);
-    return RCP_OK;
-}
-
-template <class K, class V>
-int sort_pairs(K*& keys, V*& vals, int64_t n, int begin_bit, int end_bit) {
-    if (n > 0x7fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^31-1 values in one sort");
-    K* kalt = nullptr;
-    V* valt = nullptr;
-    RCP_TRY(dalloc(&kalt, (size_t)n));
-    RCP_TRY(dalloc(&valt, (size_t)n));
-    cub::DoubleBuffer<K> kb(keys, kalt);
-    cub::DoubleBuffer<V> vb(vals, valt);
-    size_t tmp_bytes = 0;
-    RCP_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, kb, vb, (int)n, begin_bit, end_bit,
-                                             g_ctx.stream));
-    uint8_t* tmp = nullptr;
-    RCP_TRY(dalloc(&tmp, tmp_bytes));
-    RCP_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, kb, vb, (int)n, begin_bit, end_bit,
-                                             g_ctx.stream));
-    g_ctx.launches += 1 + (end_bit - begin_bit + 7) / 8;
-    dfree(tmp);
-    if (kb.Current() != keys) std::swap(keys, kalt);
-    if (vb.Current() != vals) std::swap(vals, valt);
-    dfree(kalt);
-    dfree(valt);
-    return RCP_OK;
 }
 
 struct MatIn {
@@ -612,10 +569,6 @@ int col_profile_args(const double* m, int64_t n_rows, int64_t n_cols, int64_t ld
 }
 }  // namespace
 
-int sort_pairs_u64_i32(unsigned long long*& keys, int32_t*& vals, int64_t n) {
-    return sort_pairs(keys, vals, n, 0, 64);
-}
-
 }  // namespace rcp
 
 using namespace rcp;
@@ -724,7 +677,7 @@ int rcp_reads_width_quantile(int64_t n, const int32_t* start, const int32_t* end
     const unsigned blocks = (unsigned)((n + TPB - 1) / TPB);
     width_keys_kernel<<<blocks, TPB, 0, g_ctx.stream>>>(n, d_start.ptr, d_end.ptr, keys);
     RCP_LAUNCHED();
-    int rc = sort_keys_u64(keys, n);
+    int rc = sort_keys(keys, n, 0, 64);
     unsigned long long h_count = 0;
     if (rc == RCP_OK) {
         quantile_kernel<<<1, 64, 0, g_ctx.stream>>>(keys, n, d_prob, 1, d_out);
@@ -768,7 +721,7 @@ int rcp_matrix_quantile(const double* m, int64_t n_rows, int64_t n_cols, int64_t
     cell_keys_kernel<<<(unsigned)((n + TPB - 1) / TPB), TPB, 0, g_ctx.stream>>>(in.in.ptr, n_rows, n_cols, ld,
                                                                                 keys, n_nan);
     RCP_LAUNCHED();
-    int rc = sort_keys_u64(keys, n);
+    int rc = sort_keys(keys, n, 0, 64);
     unsigned long long h_nan = 0;
     if (rc == RCP_OK) {
         quantile_kernel<<<(k + 63) / 64, 64, 0, g_ctx.stream>>>(keys, n, d_probs, k, d_out);

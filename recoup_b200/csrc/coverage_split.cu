@@ -1623,7 +1623,7 @@ static int reads_build_binned(ReadsIdx& rd) {
         RCP_LAUNCHED();
         dfree(d_cur);
         dbg.lap("  long: collect");
-        RCP_TRY(sort_pairs_u32(rd.ln_xs, idx, (int64_t)n, rd.key_bits));
+        RCP_TRY(sort_pairs(rd.ln_xs, idx, (int64_t)n, 0, rd.key_bits));
         dbg.lap("  long: sort");
         if (n > 0) {
             sp_long_gather_kernel<<<blocks_for((int64_t)n, CTA), CTA, 0, g_ctx.stream>>>((uint32_t)n, idx, rd.g_end1,

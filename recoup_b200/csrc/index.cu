@@ -461,12 +461,12 @@ int reads_build_class(ReadsIdx& r, int cls) {
     }
     {
         StageTimer t(ST_INDEX_SORT);
-        if (!xs_done) RCP_TRY(sort_keys_u32(sc.xs, sc.n, r.key_bits));
+        if (!xs_done) RCP_TRY(sort_keys(sc.xs, sc.n, 0, r.key_bits));
         sc.xs_sorted = true;
-        if (!uni) RCP_TRY(sort_keys_u32(sc.ye, sc.n, r.key_bits));
+        if (!uni) RCP_TRY(sort_keys(sc.ye, sc.n, 0, r.key_bits));
         if (sc.cn > 0) {
-            RCP_TRY(sort_keys_u32(sc.cxs, sc.cn, 32));
-            RCP_TRY(sort_keys_u32(sc.cye, sc.cn, 32));
+            RCP_TRY(sort_keys(sc.cxs, sc.cn, 0, 32));
+            RCP_TRY(sort_keys(sc.cye, sc.cn, 0, 32));
         }
     }
     r.device_bytes += (size_t)sc.n * (uni ? 4 : 8);
@@ -489,7 +489,7 @@ int reads_build_pairs(ReadsIdx& r) {
     RCP_LAUNCHED();
     {
         StageTimer t(ST_INDEX_SORT);
-        RCP_TRY(sort_pairs_u32(keys, perm, r.n, r.key_bits));
+        RCP_TRY(sort_pairs(keys, perm, r.n, 0, r.key_bits));
     }
     if (!all.xs_sorted) {           // hand the sorted keys to the ALL class
         dfree(all.xs);

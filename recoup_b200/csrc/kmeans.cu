@@ -770,7 +770,7 @@ int unique_rows(const double* x, int64_t m, int64_t p, int64_t ld, int32_t** uid
     RCP_TRY(dalloc(&rows, (size_t)m));
     km_row_hash_kernel<<<blocks_for(m), TPB, 0, g_ctx.stream>>>(x, m, p, ld, keys, rows);
     RCP_LAUNCHED();
-    int rc = sort_pairs_u64_i32(keys, rows, m);
+    int rc = sort_pairs(keys, rows, m, 0, 64);
     if (rc == RCP_OK) rc = dalloc(&first, (size_t)m);
     if (rc == RCP_OK) rc = dalloc(&at, (size_t)m);
     if (rc == RCP_OK) rc = dalloc(&total, 1);

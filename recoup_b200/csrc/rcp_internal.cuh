@@ -337,9 +337,16 @@ Coverage* get_coverage(int h);
 int new_coverage(Coverage** out, int* handle);
 
 // ------------------------------------------------------------------ primitives -------------
-// radix sort (sort.cu)
-int sort_keys_u32(uint32_t* keys_in_out, int64_t n, int end_bit);
-int sort_pairs_u32(uint32_t* keys_in_out, uint32_t* vals_in_out, int64_t n, int end_bit);
+// Radix sort (sort.cu) of n keys on their bits [begin_bit, end_bit); the pair sort is stable.
+// keys (and vals) must each be a whole dalloc allocation: they come back pointing at the sorted
+// data, and the other buffer CUB used is freed.  n <= 1 returns at once.  Instantiated for keys
+// uint32_t and unsigned long long, and for pairs uint32_t -> uint32_t, uint32_t -> int32_t and
+// unsigned long long -> int32_t.
+template <class K>
+int sort_keys(K*& keys, int64_t n, int begin_bit, int end_bit);
+template <class K, class V>
+int sort_pairs(K*& keys, V*& vals, int64_t n, int begin_bit, int end_bit);
+// running maximum (index.cu)
 int running_max_u32_device(const uint32_t* in, uint32_t* out, int64_t n);
 // exclusive prefix sum of int64 (scan.cu); out may alias in; total (optional) receives the sum
 // on the DEVICE (d_total) -- nothing is synchronised.
@@ -349,8 +356,6 @@ int exclusive_scan_u32(const uint32_t* in, uint32_t* out, int64_t n, uint32_t* d
 // launch is sized for n_upper and the blocks beyond the real length return at once
 int exclusive_scan_u32_bounded(const uint32_t* in, uint32_t* out, int64_t n_upper, const uint32_t* n_dev,
                                uint32_t* d_total);
-// stable radix sort of (64-bit key, int32 value) pairs over all 64 key bits (consumers.cu)
-int sort_pairs_u64_i32(unsigned long long*& keys, int32_t*& vals, int64_t n);
 // sample.int(n, k) from a running base-R stream, dispatched as base R does (api.cu); out 1-based
 struct RRng;
 void r_sample_int(RRng& rng, int64_t n, int64_t k, int32_t* out);

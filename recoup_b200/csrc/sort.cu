@@ -1,27 +1,16 @@
-// Device sort of 32-bit global genome coordinates (index build of rcp_reads_load).
+// Device radix sorts of the library: CUB's DeviceRadixSort (toolkit header templates), one pass
+// per 8-bit digit.  Every radix sort goes through the two functions here: the index (sorted
+// starts and ends, start-sorted (start, read id) pairs), the long-read list of the binned index,
+// the matrix consumers (orderings, quantiles, row groups) and k-means (distinct rows).  Only the
+// segmented sort of the group medians (consumers.cu) calls CUB itself.
 //
-// Keys-only sort, hand-written for B200 as a TWO-PASS bucket sort instead of a 4-pass LSD radix
-// sort (16 B of HBM traffic per key instead of 36 B):
-//
-//   msd_hist_kernel      shared-memory histogram of the top `top_bits` of every key
-//   msd_scatter_kernel   one pass: each CTA ranks its 16 K keys per bucket with shared-memory
-//                        atomics, reserves room per bucket with one global atomic and scatters.
-//                        Up to 16 K open buckets is fine on B200: the partially written lines sit
-//                        in the 126 MB L2 until they are full.  (Unstable -- irrelevant for keys.)
-//   bucket_sort_kernel   one CTA (1024 threads) per bucket: the whole bucket (<= 32 K keys) is
-//                        pulled into registers and sorted on its low bits by a shared-memory LSD
-//                        radix sort (7-bit digits, warp match ranking), then written once.
-//
-// Buckets larger than 32 K keys (pile-ups) are split again by the same kernels on their next
-// bits, driven by the host (rare path; costs a synchronisation per level).
-//
-// Pair sorts (start-sorted (start, read id) for the GRangesList path only) still use CUB's
-// DeviceRadixSort::SortPairs (toolkit header templates); set RCP_SORT=cub to route key sorts
-// there too (A/B testing).
+// The sorts hand back whichever buffer CUB finished in (declared in rcp_internal.cuh), so no
+// sorted array is copied back.  They are instantiated at the end of this file for the types in
+// use, which keeps the CUB header out of the other translation units.
 #include <cub/device/device_radix_sort.cuh>
 
-#include <cstdlib>
-#include <vector>
+#include <type_traits>
+#include <utility>
 
 #include "rcp_internal.cuh"
 
@@ -29,461 +18,64 @@ namespace rcp {
 
 namespace {
 
-constexpr int BS_THREADS = 1024;
-constexpr int BS_WARPS = BS_THREADS / 32;
-constexpr int BS_ITEMS = 32;                       // keys per thread
-constexpr int BS_CAP = BS_THREADS * BS_ITEMS;      // 32768 keys per bucket
-constexpr int BS_DBITS = 7;                        // digit of the shared-memory LSD passes
-constexpr int BS_BINS = 1 << BS_DBITS;
-constexpr int BS_MAX_R_BITS = 32;                  // a bucket CTA can sort any number of low bits
-constexpr int MSD_THREADS = 1024;
-constexpr int MSD_ITEMS = 16;
-constexpr int MSD_TILE = MSD_THREADS * MSD_ITEMS;  // 16384 keys per CTA
-constexpr int MSD_MAX_BITS = 14;                   // <= 16384 buckets (2 x 64 KB of smem counters)
-constexpr int MSD_SORTED_MAX_NB = 8192;            // tile-sorted scatter up to this many buckets
-
-__global__ void __launch_bounds__(MSD_THREADS)
-msd_hist_kernel(const uint32_t* __restrict__ src, int64_t n, int shift, int nb,
-                uint32_t* __restrict__ hist) {
-    extern __shared__ uint32_t sh_cnt[];
-    const uint32_t bm = (uint32_t)nb - 1u;     // keys of a segment agree above the bucket bits
-    for (int b = threadIdx.x; b < nb; b += MSD_THREADS) sh_cnt[b] = 0;
-    __syncthreads();
-    const int64_t stride = (int64_t)gridDim.x * MSD_THREADS;
-    const int64_t n4 = (reinterpret_cast<uintptr_t>(src) & 15u) == 0 ? (n >> 2) : 0;
-    const uint4* src4 = reinterpret_cast<const uint4*>(src);
-    for (int64_t v = (int64_t)blockIdx.x * MSD_THREADS + threadIdx.x; v < n4; v += stride) {
-        const uint4 k = __ldg(src4 + v);
-        atomicAdd(&sh_cnt[(k.x >> shift) & bm], 1u);
-        atomicAdd(&sh_cnt[(k.y >> shift) & bm], 1u);
-        atomicAdd(&sh_cnt[(k.z >> shift) & bm], 1u);
-        atomicAdd(&sh_cnt[(k.w >> shift) & bm], 1u);
-    }
-    for (int64_t i = n4 * 4 + (int64_t)blockIdx.x * MSD_THREADS + threadIdx.x; i < n; i += stride)
-        atomicAdd(&sh_cnt[(__ldg(src + i) >> shift) & bm], 1u);
-    __syncthreads();
-    for (int b = threadIdx.x; b < nb; b += MSD_THREADS) {
-        const uint32_t c = sh_cnt[b];
-        if (c) atomicAdd(&hist[b], c);
-    }
-}
-
-// exclusive scan of hist[0..nb) into off[0..nb], one block; flags buckets over the capacity
-__global__ void __launch_bounds__(1024)
-msd_offsets_kernel(const uint32_t* __restrict__ hist, int nb, uint32_t* __restrict__ off,
-                   uint32_t* __restrict__ n_oversized) {
-    __shared__ uint32_t wsum[32];
-    __shared__ uint32_t carry_sh;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) carry_sh = 0;
-    __syncthreads();
-    uint32_t over = 0;
-    for (int b0 = 0; b0 < nb; b0 += 1024) {
-        const int b = b0 + threadIdx.x;
-        const uint32_t v = b < nb ? hist[b] : 0u;
-        over += v > (uint32_t)BS_CAP;
-        uint32_t inc = v;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const uint32_t o = __shfl_up_sync(0xffffffffu, inc, d);
-            if (lane >= d) inc += o;
-        }
-        if (lane == 31) wsum[warp] = inc;
-        __syncthreads();
-        uint32_t pre = carry_sh;
-        for (int w = 0; w < warp; w++) pre += wsum[w];
-        if (b < nb) off[b] = pre + inc - v;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry_sh = pre + inc;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) off[nb] = carry_sh;
-    if (over) atomicAdd(n_oversized, over);
-}
-
-// Pass 1.  SORTED = true (nb <= 8192): the tile is first grouped by bucket in shared memory, so
-// consecutive threads write consecutive addresses of a bucket's run (fewer L2 sectors per
-// store); SORTED = false: every key goes straight to its slot.
-template <bool SORTED>
-__global__ void __launch_bounds__(MSD_THREADS)
-msd_scatter_kernel(const uint32_t* __restrict__ src, uint32_t* __restrict__ dst, int64_t n,
-                   int shift, int nb, const uint32_t* __restrict__ bucket_off,
-                   uint32_t* __restrict__ cursor) {
-    extern __shared__ uint32_t sh[];
-    uint32_t* cnt = sh;            // nb: keys of this tile per bucket, later a running cursor
-    uint32_t* base = sh + nb;      // nb: where the tile's run of that bucket starts in dst
-    uint32_t* loc = sh + 2 * nb;   // nb: where it starts inside the tile      (SORTED only)
-    uint32_t* tile = sh + 3 * nb;  // MSD_TILE keys grouped by bucket           (SORTED only)
-    __shared__ uint32_t wsum[32];
-    __shared__ uint32_t carry_sh;
-    const uint32_t bm = (uint32_t)nb - 1u;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int b = threadIdx.x; b < nb; b += MSD_THREADS) cnt[b] = 0;
-    if (threadIdx.x == 0) carry_sh = 0;
-    __syncthreads();
-    const int64_t tile0 = (int64_t)blockIdx.x * MSD_TILE;
-    const int tile_n = (int)min((int64_t)MSD_TILE, n - tile0);
-    uint32_t key[MSD_ITEMS], rnk[MSD_ITEMS];
-    // blocked-by-4 arrangement: 16-byte loads while the tile is full
-    const bool full = tile_n == MSD_TILE && (reinterpret_cast<uintptr_t>(src) & 15u) == 0;
-#pragma unroll
-    for (int q = 0; q < MSD_ITEMS / 4; q++) {
-        const int64_t i = tile0 + ((int64_t)q * MSD_THREADS + threadIdx.x) * 4;
-        if (full) {
-            const uint4 k = __ldg(reinterpret_cast<const uint4*>(src + i));
-            key[4 * q + 0] = k.x;
-            key[4 * q + 1] = k.y;
-            key[4 * q + 2] = k.z;
-            key[4 * q + 3] = k.w;
-        } else {
-#pragma unroll
-            for (int j = 0; j < 4; j++) key[4 * q + j] = (i + j < n) ? __ldg(src + i + j) : 0u;
-        }
-    }
-#pragma unroll
-    for (int q = 0; q < MSD_ITEMS; q++) {
-        const int64_t i = tile0 + ((int64_t)(q >> 2) * MSD_THREADS + threadIdx.x) * 4 + (q & 3);
-        rnk[q] = (i < n) ? atomicAdd(&cnt[(key[q] >> shift) & bm], 1u) : 0u;
-    }
-    __syncthreads();
-    if (SORTED) {
-        // exclusive scan of cnt -> loc (chunks of 1024 buckets), reserve the global runs
-        for (int b0 = 0; b0 < nb; b0 += MSD_THREADS) {
-            const int b = b0 + threadIdx.x;
-            const uint32_t c = b < nb ? cnt[b] : 0u;
-            uint32_t inc = c;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const uint32_t o = __shfl_up_sync(0xffffffffu, inc, d);
-                if (lane >= d) inc += o;
-            }
-            if (lane == 31) wsum[warp] = inc;
-            __syncthreads();
-            uint32_t pre = carry_sh;
-            for (int w = 0; w < warp; w++) pre += wsum[w];
-            if (b < nb) {
-                loc[b] = pre + inc - c;
-                if (c) base[b] = bucket_off[b] + atomicAdd(&cursor[b], c);
-            }
-            __syncthreads();
-            if (threadIdx.x == MSD_THREADS - 1) carry_sh = pre + inc;
-            __syncthreads();
-        }
-#pragma unroll
-        for (int q = 0; q < MSD_ITEMS; q++) {
-            const int64_t i = tile0 + ((int64_t)(q >> 2) * MSD_THREADS + threadIdx.x) * 4 + (q & 3);
-            if (i < n) tile[loc[(key[q] >> shift) & bm] + rnk[q]] = key[q];
-        }
-        __syncthreads();
-        for (int i = threadIdx.x; i < tile_n; i += MSD_THREADS) {
-            const uint32_t k = tile[i];
-            const uint32_t b = (k >> shift) & bm;
-            dst[base[b] + ((uint32_t)i - loc[b])] = k;
-        }
-    } else {
-        for (int b = threadIdx.x; b < nb; b += MSD_THREADS) {
-            const uint32_t c = cnt[b];
-            if (c) base[b] = bucket_off[b] + atomicAdd(&cursor[b], c);
-        }
-        __syncthreads();
-#pragma unroll
-        for (int q = 0; q < MSD_ITEMS; q++) {
-            const int64_t i = tile0 + ((int64_t)(q >> 2) * MSD_THREADS + threadIdx.x) * 4 + (q & 3);
-            if (i < n) dst[base[(key[q] >> shift) & bm] + rnk[q]] = key[q];
-        }
-    }
-}
-
-// One CTA per bucket: sort the low `r_bits` bits of src[off[b] .. off[b+1]) into dst (same
-// offsets; src == dst is allowed: the bucket is fully loaded before anything is written).
-__global__ void __launch_bounds__(BS_THREADS, 1)
-bucket_sort_kernel(const uint32_t* src, uint32_t* dst,   // may alias: no __restrict__
-                   const uint32_t* __restrict__ bucket_off, int r_bits) {
-    extern __shared__ __align__(16) uint32_t smem_raw[];
-    uint32_t* buf = smem_raw;                                           // BS_CAP keys
-    unsigned short* rnk = reinterpret_cast<unsigned short*>(buf + BS_CAP);   // BS_CAP ranks
-    uint32_t* whist = reinterpret_cast<uint32_t*>(rnk + BS_CAP);        // [BS_WARPS][BS_BINS]
-    uint32_t* dig = whist + BS_WARPS * BS_BINS;                         // BS_BINS exclusive starts
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t start = bucket_off[blockIdx.x];
-    const int n = (int)(bucket_off[blockIdx.x + 1] - start);
-    if (n <= 0 || n > BS_CAP) return;
-    const int items = (n + BS_THREADS - 1) / BS_THREADS;
-    // warp-striped: warp w owns [w*32*items, (w+1)*32*items); item i of lane l sits at +i*32+l
-    const int wbase = warp * 32 * items + lane;
-    uint32_t key[BS_ITEMS];
-#pragma unroll
-    for (int i = 0; i < BS_ITEMS; i++) {
-        key[i] = 0xffffffffu;
-        if (i < items) {
-            const int idx = wbase + i * 32;
-            if (idx < n) key[i] = src[start + idx];
-        }
-    }
-    const unsigned lt = (1u << lane) - 1u;
-    for (int shift = 0; shift < r_bits; shift += BS_DBITS) {
-        const int bits = min(BS_DBITS, r_bits - shift);
-        const uint32_t dmask = (1u << bits) - 1u;
-        for (int i = tid; i < BS_WARPS * BS_BINS; i += BS_THREADS) whist[i] = 0;
-        __syncthreads();
-        uint32_t* wh = whist + warp * BS_BINS;
-        // groups of four items: the 28 ballots of a group are independent and issue back to
-        // back; only the four counter updates are serial
-#pragma unroll
-        for (int i0 = 0; i0 < BS_ITEMS; i0 += 4) {
-            if (i0 < items) {
-                unsigned peers[4];
-#pragma unroll
-                for (int j = 0; j < 4; j++) {
-                    const uint32_t d = (key[i0 + j] >> shift) & dmask;
-                    unsigned pm = 0xffffffffu;
-#pragma unroll
-                    for (int bb = 0; bb < BS_DBITS; bb++) {
-                        const unsigned vote = __ballot_sync(0xffffffffu, (d >> bb) & 1u);
-                        pm &= ((d >> bb) & 1u) ? vote : ~vote;
-                    }
-                    peers[j] = pm;
-                }
-#pragma unroll
-                for (int j = 0; j < 4; j++) {
-                    if (i0 + j < items) {
-                        const uint32_t d = (key[i0 + j] >> shift) & dmask;
-                        const int leader = __ffs(peers[j]) - 1;
-                        uint32_t old = 0;
-                        if (lane == leader) {
-                            old = wh[d];
-                            wh[d] = old + __popc(peers[j]);
-                        }
-                        old = __shfl_sync(0xffffffffu, old, leader);
-                        rnk[wbase + (i0 + j) * 32] = (unsigned short)(old + __popc(peers[j] & lt));
-                        __syncwarp();
-                    }
-                }
-            }
-        }
-        __syncthreads();
-        // per digit: exclusive offsets of the warps, then of the digits
-        if (tid < BS_BINS) {
-            uint32_t run = 0;
-            for (int w = 0; w < BS_WARPS; w++) {
-                const uint32_t t = whist[w * BS_BINS + tid];
-                whist[w * BS_BINS + tid] = run;
-                run += t;
-            }
-            dig[tid] = run;
-        }
-        __syncthreads();
-        if (warp == 0) {
-            uint32_t carry = 0;
-            for (int d0 = 0; d0 < BS_BINS; d0 += 32) {
-                const uint32_t v = dig[d0 + lane];
-                uint32_t inc = v;
-#pragma unroll
-                for (int dd = 1; dd < 32; dd <<= 1) {
-                    const uint32_t o = __shfl_up_sync(0xffffffffu, inc, dd);
-                    if (lane >= dd) inc += o;
-                }
-                dig[d0 + lane] = carry + inc - v;
-                carry += __shfl_sync(0xffffffffu, inc, 31);
-            }
-        }
-        __syncthreads();
-#pragma unroll
-        for (int i = 0; i < BS_ITEMS; i++) {
-            if (i < items) {
-                const uint32_t d = (key[i] >> shift) & dmask;
-                buf[dig[d] + wh[d] + rnk[wbase + i * 32]] = key[i];
-            }
-        }
-        __syncthreads();
-#pragma unroll
-        for (int i = 0; i < BS_ITEMS; i++)
-            if (i < items) key[i] = buf[wbase + i * 32];
-        __syncthreads();
-    }
-#pragma unroll
-    for (int i = 0; i < BS_ITEMS; i++) {
-        if (i < items) {
-            const int idx = wbase + i * 32;
-            if (idx < n) dst[start + idx] = key[i];
-        }
-    }
-}
-
-constexpr size_t BS_SMEM = (size_t)BS_CAP * 4 + (size_t)BS_CAP * 2 + (size_t)BS_WARPS * BS_BINS * 4 +
-                           (size_t)BS_BINS * 4;
-
-bool g_attr_set = false;
-
-int set_attrs() {
-    if (g_attr_set) return RCP_OK;
-    RCP_CUDA(cudaFuncSetAttribute(bucket_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)BS_SMEM));
-    RCP_CUDA(cudaFuncSetAttribute(msd_scatter_kernel<false>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)(2 * (1 << MSD_MAX_BITS) * 4)));
-    RCP_CUDA(cudaFuncSetAttribute(msd_scatter_kernel<true>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)((3 * MSD_SORTED_MAX_NB + MSD_TILE) * 4)));
-    RCP_CUDA(cudaFuncSetAttribute(msd_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)((1 << MSD_MAX_BITS) * 4)));
-    g_attr_set = true;
-    return RCP_OK;
-}
-
-// Sorts the low `bits` bits of the n keys found in `data` (all higher bits are equal or already
-// ordered); the result lands in `result` (== data, or the other buffer `scratch_of_result`).
-// `data` and `other` are the two ping-pong segments of identical extent.
-int sort_segment(uint32_t* data, uint32_t* other, uint32_t* result, int64_t n, int bits,
-                 int depth) {
-    if (n <= 0) return RCP_OK;
-    if (bits <= 0 || n == 1) {
-        if (result != data)
-            RCP_CUDA(cudaMemcpyAsync(result, data, (size_t)n * 4, cudaMemcpyDeviceToDevice,
-                                     g_ctx.stream));
-        return RCP_OK;
-    }
-    if (depth > 8) return fail(RCP_ERR_CUDA, "sort: recursion too deep");
-    if (n <= BS_CAP && bits <= BS_MAX_R_BITS) {
-        uint32_t h_off[2] = {0u, (uint32_t)n};
-        uint32_t* d_off = nullptr;
-        RCP_TRY(dalloc(&d_off, 2));
-        RCP_CUDA(cudaMemcpyAsync(d_off, h_off, sizeof(h_off), cudaMemcpyHostToDevice, g_ctx.stream));
-        bucket_sort_kernel<<<1, BS_THREADS, BS_SMEM, g_ctx.stream>>>(data, result, d_off, bits);
-        RCP_LAUNCHED();
-        dfree(d_off);
-        return RCP_OK;
-    }
-    // top bits so that the average bucket is ~12 K keys (capacity 32 K)
-    int top = 1;
-    while (top < MSD_MAX_BITS && (n >> top) > 12288) top++;
-    if (depth > 0) top = MSD_MAX_BITS;     // a pile-up: few distinct values, split as finely as possible
-    if (top < bits - BS_MAX_R_BITS) top = bits - BS_MAX_R_BITS;   // a bucket CTA sorts <= 22 bits
-    if (top > bits) top = bits;
-    const int shift = bits - top;
-    const int nb = 1 << top;
-    // keys entering here agree on every bit above `bits`: bucket = (key >> shift) & (nb - 1)
-    uint32_t *hist = nullptr, *off = nullptr, *cursor = nullptr, *n_over = nullptr;
-    RCP_TRY(dalloc(&hist, (size_t)nb));
-    RCP_TRY(dalloc(&off, (size_t)nb + 1));
-    RCP_TRY(dalloc(&cursor, (size_t)nb));
-    RCP_TRY(dalloc(&n_over, 1));
-    RCP_CUDA(cudaMemsetAsync(hist, 0, (size_t)nb * 4, g_ctx.stream));
-    RCP_CUDA(cudaMemsetAsync(cursor, 0, (size_t)nb * 4, g_ctx.stream));
-    RCP_CUDA(cudaMemsetAsync(n_over, 0, 4, g_ctx.stream));
-    int hist_grid = (int)((n + MSD_TILE - 1) / MSD_TILE);
-    if (hist_grid > g_ctx.sm_count * 2) hist_grid = g_ctx.sm_count * 2;
-    msd_hist_kernel<<<hist_grid, MSD_THREADS, (size_t)nb * 4, g_ctx.stream>>>(data, n, shift, nb,
-                                                                              hist);
-    RCP_LAUNCHED();
-    msd_offsets_kernel<<<1, 1024, 0, g_ctx.stream>>>(hist, nb, off, n_over);
-    RCP_LAUNCHED();
-    const int tiles = (int)((n + MSD_TILE - 1) / MSD_TILE);
-    if (nb <= MSD_SORTED_MAX_NB)
-        msd_scatter_kernel<true><<<tiles, MSD_THREADS, ((size_t)3 * nb + MSD_TILE) * 4, g_ctx.stream>>>(
-            data, other, n, shift, nb, off, cursor);
-    else
-        msd_scatter_kernel<false><<<tiles, MSD_THREADS, (size_t)nb * 8, g_ctx.stream>>>(
-            data, other, n, shift, nb, off, cursor);
-    RCP_LAUNCHED();
-    // buckets now sit in `other`; sorted buckets go to `result`
-    bucket_sort_kernel<<<nb, BS_THREADS, BS_SMEM, g_ctx.stream>>>(other, result, off, shift);
-    RCP_LAUNCHED();
-    uint32_t h_over = 0;
-    if (n > BS_CAP) {      // with n <= BS_CAP no bucket can overflow: no need to look (or to wait)
-        RCP_CUDA(cudaMemcpyAsync(&h_over, n_over, 4, cudaMemcpyDeviceToHost, g_ctx.stream));
-        RCP_CUDA(cudaStreamSynchronize(g_ctx.stream));
-    }
-    int rc = RCP_OK;
-    if (h_over > 0) {
-        // pile-ups: split the oversized buckets again on their next bits
-        std::vector<uint32_t> h_off((size_t)nb + 1);
-        RCP_CUDA(cudaMemcpyAsync(h_off.data(), off, ((size_t)nb + 1) * 4, cudaMemcpyDeviceToHost,
-                                 g_ctx.stream));
-        RCP_CUDA(cudaStreamSynchronize(g_ctx.stream));
-        for (int b = 0; b < nb && rc == RCP_OK; b++) {
-            const int64_t cnt = (int64_t)h_off[(size_t)b + 1] - h_off[(size_t)b];
-            if (cnt > BS_CAP) {
-                // the bucket's keys are in `other`; the same extent of `data` is free (pass 1
-                // consumed it, pass 2 skipped this bucket) and serves as scratch; the sorted
-                // keys must land in `result`, which is one of the two
-                const size_t o = h_off[(size_t)b];
-                rc = sort_segment(other + o, data + o, result + o, cnt, shift, depth + 1);
-            }
-        }
-    }
-    dfree(hist);
-    dfree(off);
-    dfree(cursor);
-    dfree(n_over);
-    return rc;
-}
+// a device buffer of one sort, freed on every return path
+template <class T>
+struct Scratch {
+    T* p = nullptr;
+    ~Scratch() { dfree(p); }
+};
 
 }  // namespace
 
-int sort_keys_cub(uint32_t* keys, int64_t n, int end_bit) {
-    uint32_t* alt = nullptr;
-    RCP_TRY(dalloc(&alt, (size_t)n));
-    cub::DoubleBuffer<uint32_t> buf(keys, alt);
+template <class K>
+int sort_keys(K*& keys, int64_t n, int begin_bit, int end_bit) {
+    if (n <= 1) return RCP_OK;
+    // 32-bit keys are the index's read coordinates
+    if (sizeof(K) == 4 && n > 0x3fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^30-1 reads in one sort");
+    if (n > 0x7fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^31-1 values in one sort");
+    Scratch<K> alt;
+    Scratch<uint8_t> tmp;
+    RCP_TRY(dalloc(&alt.p, (size_t)n));
+    cub::DoubleBuffer<K> kb(keys, alt.p);
     size_t tmp_bytes = 0;
-    RCP_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, buf, (int)n, 0, end_bit,
-                                            g_ctx.stream));
-    uint8_t* tmp = nullptr;
-    RCP_TRY(dalloc(&tmp, tmp_bytes));
-    RCP_CUDA(cub::DeviceRadixSort::SortKeys(tmp, tmp_bytes, buf, (int)n, 0, end_bit,
-                                            g_ctx.stream));
-    g_ctx.launches += 1 + (end_bit + 7) / 8;
-    if (buf.Current() != keys) {
-        RCP_CUDA(cudaMemcpyAsync(keys, buf.Current(), (size_t)n * sizeof(uint32_t),
-                                 cudaMemcpyDeviceToDevice, g_ctx.stream));
-    }
-    dfree(tmp);
-    dfree(alt);
+    RCP_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, kb, (int)n, begin_bit, end_bit, g_ctx.stream));
+    RCP_TRY(dalloc(&tmp.p, tmp_bytes));
+    RCP_CUDA(cub::DeviceRadixSort::SortKeys(tmp.p, tmp_bytes, kb, (int)n, begin_bit, end_bit, g_ctx.stream));
+    g_ctx.launches += 1 + (end_bit - begin_bit + 7) / 8;
+    if (kb.Current() != keys) std::swap(keys, alt.p);
     return RCP_OK;
 }
 
-int sort_keys_u32(uint32_t* keys, int64_t n, int end_bit) {
+template <class K, class V>
+int sort_pairs(K*& keys, V*& vals, int64_t n, int begin_bit, int end_bit) {
     if (n <= 1) return RCP_OK;
-    if (n > 0x3fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^30-1 reads in one sort");
-    // Default: CUB's DeviceRadixSort (toolkit header library).  The hand-written two-pass bucket
-    // sort below (RCP_SORT=hand) is within 10 % of it on uniform reads but degrades on heavily
-    // clustered ones (RNA-seq: most MSD buckets overflow and are split again from the host).
-    const char* which = getenv("RCP_SORT");
-    if (!(which != nullptr && which[0] == 'h')) return sort_keys_cub(keys, n, end_bit);
-    RCP_TRY(set_attrs());
-    uint32_t* alt = nullptr;
-    if (n > BS_CAP || end_bit > BS_MAX_R_BITS) RCP_TRY(dalloc(&alt, (size_t)n));
-    // data in `keys`, scratch `alt`, result back in `keys`
-    int rc = sort_segment(keys, alt, keys, n, end_bit, 0);
-    dfree(alt);
-    return rc;
-}
-
-int sort_pairs_u32(uint32_t* keys, uint32_t* vals, int64_t n, int end_bit) {
-    if (n <= 1) return RCP_OK;
-    if (n > 0x7fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^31-1 reads in one sort");
-    uint32_t *kalt = nullptr, *valt = nullptr;
-    RCP_TRY(dalloc(&kalt, (size_t)n));
-    RCP_TRY(dalloc(&valt, (size_t)n));
-    cub::DoubleBuffer<uint32_t> kb(keys, kalt), vb(vals, valt);
+    // uint32_t values are read ids (the index), int32_t ones rows or cells (the matrix consumers)
+    if (n > 0x7fffffff)
+        return fail(RCP_ERR_UNSUPPORTED, "more than 2^31-1 %s in one sort",
+                    std::is_same<V, uint32_t>::value ? "reads" : "values");
+    Scratch<K> kalt;
+    Scratch<V> valt;
+    Scratch<uint8_t> tmp;
+    RCP_TRY(dalloc(&kalt.p, (size_t)n));
+    RCP_TRY(dalloc(&valt.p, (size_t)n));
+    cub::DoubleBuffer<K> kb(keys, kalt.p);
+    cub::DoubleBuffer<V> vb(vals, valt.p);
     size_t tmp_bytes = 0;
-    RCP_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, kb, vb, (int)n, 0, end_bit,
+    RCP_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, kb, vb, (int)n, begin_bit, end_bit,
                                              g_ctx.stream));
-    uint8_t* tmp = nullptr;
-    RCP_TRY(dalloc(&tmp, tmp_bytes));
-    RCP_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, kb, vb, (int)n, 0, end_bit,
+    RCP_TRY(dalloc(&tmp.p, tmp_bytes));
+    RCP_CUDA(cub::DeviceRadixSort::SortPairs(tmp.p, tmp_bytes, kb, vb, (int)n, begin_bit, end_bit,
                                              g_ctx.stream));
-    g_ctx.launches += 1 + (end_bit + 7) / 8;
-    if (kb.Current() != keys)
-        RCP_CUDA(cudaMemcpyAsync(keys, kb.Current(), (size_t)n * sizeof(uint32_t),
-                                 cudaMemcpyDeviceToDevice, g_ctx.stream));
-    if (vb.Current() != vals)
-        RCP_CUDA(cudaMemcpyAsync(vals, vb.Current(), (size_t)n * sizeof(uint32_t),
-                                 cudaMemcpyDeviceToDevice, g_ctx.stream));
-    dfree(tmp);
-    dfree(kalt);
-    dfree(valt);
+    g_ctx.launches += 1 + (end_bit - begin_bit + 7) / 8;
+    if (kb.Current() != keys) std::swap(keys, kalt.p);
+    if (vb.Current() != vals) std::swap(vals, valt.p);
     return RCP_OK;
 }
+
+template int sort_keys<uint32_t>(uint32_t*&, int64_t, int, int);
+template int sort_keys<unsigned long long>(unsigned long long*&, int64_t, int, int);
+template int sort_pairs<uint32_t, uint32_t>(uint32_t*&, uint32_t*&, int64_t, int, int);
+template int sort_pairs<uint32_t, int32_t>(uint32_t*&, int32_t*&, int64_t, int, int);
+template int sort_pairs<unsigned long long, int32_t>(unsigned long long*&, int32_t*&, int64_t, int, int);
 
 }  // namespace rcp

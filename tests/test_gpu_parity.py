@@ -857,7 +857,7 @@ def test_consumers_on_the_fixture_profile(gpu_auto, fixture_data):
 
 
 # ------------------------------------------------------------------------------------------------
-# the hand-written index sort, directly
+# the index sort, directly
 # ------------------------------------------------------------------------------------------------
 def _gpu_sort(keys, bits):
     from recoup_b200 import _lib
@@ -868,19 +868,15 @@ def _gpu_sort(keys, bits):
 
 @pytest.mark.parametrize("n,bits", [(1, 32), (2, 32), (1000, 32), (32768, 32), (32769, 32),
                                     (100_000, 27), (1_000_003, 32), (3_000_000, 17), (5_000_000, 32)])
-@pytest.mark.parametrize("which", ["cub", "hand"])
-def test_index_sort_uniform_keys(gpu, monkeypatch, n, bits, which):
-    monkeypatch.setenv("RCP_SORT", which)      # RCP_SORT=hand: the hand-written bucket sort
+def test_index_sort_uniform_keys(gpu, n, bits):
     rng = np.random.default_rng(n)
     keys = rng.integers(0, 1 << bits, size=n, dtype=np.uint64).astype(np.uint32)
     assert np.array_equal(_gpu_sort(keys, bits), np.sort(keys))
 
 
-@pytest.mark.parametrize("which", ["cub", "hand"])
-def test_index_sort_pileups_and_recursion(gpu, monkeypatch, which):
-    """Buckets far over the 32 K-key capacity: one value repeated 400 K times, 150 K keys inside a
-    512-wide window, 90 K inside a 40 K-wide window, sorted / reversed inputs, all-equal input."""
-    monkeypatch.setenv("RCP_SORT", which)
+def test_index_sort_pileups_and_recursion(gpu):
+    """Pile-ups: one value repeated 400 K times, 150 K keys inside a 512-wide window, 90 K inside a
+    40 K-wide window, sorted / reversed inputs, all-equal input, keys of 2 significant bits."""
     rng = np.random.default_rng(5)
     parts = [np.full(400_000, 2_000_000_123, dtype=np.uint32),
              (3_000_000_000 + rng.integers(0, 512, size=150_000)).astype(np.uint32),

@@ -18,6 +18,7 @@ The branch meta-test restates the dispatch of bin_desc_kernel and the host sizin
 bin_matrix_impl (recoup_b200/csrc/profile.cu) and checks that the case matrix reaches every
 branch under every storage.  Run the GPU tests with `-m gpu` on a B200."""
 import ctypes as C
+import gc
 import math
 import struct
 from collections import namedtuple
@@ -746,6 +747,7 @@ def test_bin_count_limits_fail_cleanly(store):
     cov = store.coverage(lens, starts, targets, clen, check=False)
     for stat in ("mean", "median"):
         for n in (MAX_BINS + 1, INTERP_MAX_BINS + 1, 6000):
+            gc.collect()        # else a collection during the call may free device memory of earlier tests
             _lib.check(_lib.lib.rcp_sync())
             before = pool_used()
             with pytest.raises(_lib.RecoupError) as e:
