@@ -105,15 +105,13 @@ const char* rcp_timing_stage_name(int stage);
  *                     dense masks / stranded calls); otherwise the call uses the paths below;
  *   RCP_PATH_BUCKETS  two passes over the unsorted reads drop each read into the buckets of the
  *                     output tiles it overlaps (cell table + hit list, no sort);
- *   RCP_PATH_BLOCKS   the reads that pass a block bitmap are partitioned by 16-kb genome block
- *                     (two multisplit passes, no per-read random access) and every output tile
- *                     scans the candidates of the blocks under it;
  *   RCP_PATH_INDEX    the reads are radix-sorted once per handle and every region is served by
  *                     rank searches (cheaper when one handle serves many masks);
  *   RCP_PATH_AUTO     (default) the index when the handle already has one; else split when the
- *                     reads fit its packed word; else the index when the mask is dense and the
- *                     reads many, blocks for masks made of tiled regions (> 1024 bp: TSS windows,
- *                     gene bodies), buckets for masks dominated by short regions.
+ *                     reads fit its packed word; else buckets, which hand the call to the index
+ *                     when the mask is dense and the reads many;
+ *   RCP_PATH_BLOCKS   retired value: still accepted, selects RCP_PATH_BUCKETS (no coverage
+ *                     reports it).
  * The reference has one path (findOverlaps per region, coverage.R:189-193); this is a tuning
  * knob with no counterpart there. */
 #define RCP_PATH_AUTO 0
@@ -122,8 +120,8 @@ const char* rcp_timing_stage_name(int stage);
 #define RCP_PATH_BLOCKS 3
 #define RCP_PATH_SPLIT 4
 int rcp_set_coverage_path(int path);
-/* Which path produced a coverage (RCP_PATH_INDEX / BUCKETS / BLOCKS; 0 for GRangesList and
- * concatenated coverages) and, for the block path, how many reads passed its bitmap filter
+/* Which path produced a coverage (RCP_PATH_SPLIT / BUCKETS / INDEX; 0 for GRangesList and
+ * concatenated coverages) and, for the split path, how many reads passed its bitmap filter
  * (bench.py derives that path's algorithmic bytes from it). */
 int rcp_coverage_path_info(int cov, int* path, int64_t* candidates);
 

@@ -171,8 +171,9 @@ def shutdown():
 
 
 def set_coverage_path(path):
-    """"auto" | "index" | "buckets": how rcp_coverage finds each region's reads (same results;
-    see include/recoup_b200.h).  Takes effect for reads uploaded afterwards."""
+    """"auto" | "split" | "buckets" | "index" ("blocks" is a retired name for "buckets"): how
+    rcp_coverage finds each region's reads (same results; see include/recoup_b200.h).  Applies to
+    every later coverage call; "index" also sorts reads at load time from then on."""
     ensure_init()
     check(lib.rcp_set_coverage_path(COVERAGE_PATH[path]))
 

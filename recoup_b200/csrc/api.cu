@@ -103,11 +103,11 @@ static std::vector<TimerRec> g_pending;
 static std::vector<cudaEvent_t> g_free_events;
 static double g_stage_ms[ST_N];
 static int64_t g_stage_count[ST_N];
-static const char* const g_stage_names[ST_N] = {
+static const char* const g_stage_names[] = {
     "index_map", "index_sort", "cov_plan", "cov_tile", "cov_small", "cov_list", "cov_concat",
     "prof_bin", "prof_interp", "prof_base", "fused", "bkt_plan", "bkt_count", "bkt_scatter",
-    "bkt_tile", "bkt_small", "blk_filter", "blk_hist", "blk_scatter", "blk_tile", "blk_small",
-    "sp_plan", "sp_split", "sp_sort", "sp_tile", "sp_small"};
+    "bkt_tile", "bkt_small", "sp_plan", "sp_split", "sp_sort", "sp_tile"};
+static_assert(sizeof(g_stage_names) / sizeof(g_stage_names[0]) == ST_N, "one name per Stage");
 
 static cudaEvent_t take_event() {
     if (!g_free_events.empty()) {
@@ -261,9 +261,6 @@ int coverage_list(ReadsIdx& rd, int64_t G, const int64_t* ptr, const int64_t n_r
                   const int32_t* chrom, const int32_t* start, const int32_t* end,
                   const int8_t* strand, int ignore_strand, int strand_filter, int mem,
                   Coverage* cv);
-int coverage_ranges_blocks(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32_t* start,
-                           const int32_t* end, const int8_t* strand, int ignore_strand,
-                           int strand_filter, int mem, Coverage* cv);
 int coverage_ranges_split(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32_t* start,
                           const int32_t* end, const int8_t* strand, int ignore_strand,
                           int strand_filter, int mem, Coverage* cv);
@@ -659,7 +656,8 @@ int rcp_set_coverage_path(int path) {
     if (path != RCP_PATH_AUTO && path != RCP_PATH_INDEX && path != RCP_PATH_BUCKETS &&
         path != RCP_PATH_BLOCKS && path != RCP_PATH_SPLIT)
         return fail(RCP_ERR_ARG, "unknown coverage path %d", path);
-    g_ctx.coverage_path = path;
+    // RCP_PATH_BLOCKS is retired: callers built against it get the bucket path
+    g_ctx.coverage_path = path == RCP_PATH_BLOCKS ? RCP_PATH_BUCKETS : path;
     return RCP_OK;
 }
 
@@ -872,8 +870,7 @@ int rcp_coverage(int reads, int64_t n_regions, const int32_t* chrom, const int32
     // (reads narrower than the packed candidate word allows); it also validates a deferred load.
     int rc = RCP_SPLIT_NOT_APPLICABLE;
     const bool try_split = g_ctx.coverage_path == RCP_PATH_SPLIT ||
-                           (g_ctx.coverage_path == RCP_PATH_AUTO && !use_index &&
-                            getenv("RCP_AUTO_NO_SPLIT") == nullptr);
+                           (g_ctx.coverage_path == RCP_PATH_AUTO && !use_index);
     if (try_split) {
         rc = coverage_ranges_split(*r, n_regions, chrom, start, end, strand, ignore_strand != 0,
                                    strand_filter, mem, cv);
@@ -881,10 +878,7 @@ int rcp_coverage(int reads, int64_t n_regions, const int32_t* chrom, const int32
     if (rc == RCP_SPLIT_NOT_APPLICABLE) {
         rc = reads_resolve(*r);
         if (rc == RCP_OK) rc = RCP_SWITCH_TO_INDEX;
-        if (rc == RCP_SWITCH_TO_INDEX && g_ctx.coverage_path == RCP_PATH_BLOCKS) {
-            rc = coverage_ranges_blocks(*r, n_regions, chrom, start, end, strand, ignore_strand != 0,
-                                        strand_filter, mem, cv);
-        } else if (rc == RCP_SWITCH_TO_INDEX && !use_index) {
+        if (rc == RCP_SWITCH_TO_INDEX && !use_index) {
             rc = coverage_ranges_bucketed(*r, n_regions, chrom, start, end, strand, ignore_strand != 0,
                                           strand_filter, mem,
                                           g_ctx.coverage_path == RCP_PATH_AUTO ||
@@ -933,8 +927,7 @@ int rcp_coverage_list(int reads, int64_t n_elements, const int64_t* ptr, const i
     // the handle's binned index (built on first use) serves the call when the reads fit its packed
     // word; the start-sorted pairs (one radix sort of every read) otherwise or on request
     int rc = RCP_SPLIT_NOT_APPLICABLE;
-    if ((g_ctx.coverage_path == RCP_PATH_AUTO || g_ctx.coverage_path == RCP_PATH_SPLIT) && !r->pairs_built &&
-        getenv("RCP_AUTO_NO_SPLIT") == nullptr) {
+    if ((g_ctx.coverage_path == RCP_PATH_AUTO || g_ctx.coverage_path == RCP_PATH_SPLIT) && !r->pairs_built) {
         rc = coverage_list_split(*r, n_elements, ptr, n_ranges, chrom, start, end, strand, ignore_strand != 0,
                                  strand_filter, mem, cv);
         if (rc == RCP_SPLIT_NOT_APPLICABLE) coverage_release(*cv);
@@ -1222,8 +1215,7 @@ int rcp_coverage_profile(int reads, int64_t n_regions, const int32_t* chrom, con
     if (!valid_strand_filter(strand_filter)) return fail(RCP_ERR_ARG, "bad strand filter %d", strand_filter);
     if (mem != RCP_MEM_HOST && mem != RCP_MEM_DEVICE) return fail(RCP_ERR_ARG, "bad mem kind");
     if (n_regions > 0x7fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^31-1 regions");
-    const bool may_split = g_ctx.coverage_path == RCP_PATH_SPLIT ||
-                           (g_ctx.coverage_path == RCP_PATH_AUTO && getenv("RCP_AUTO_NO_SPLIT") == nullptr);
+    const bool may_split = g_ctx.coverage_path == RCP_PATH_SPLIT || g_ctx.coverage_path == RCP_PATH_AUTO;
     if (n_bins >= 1 && may_split && !r->any_na) {      // (NA seqlengths: the rule needs the coverage itself)
         MatrixOut m;
         RCP_TRY(m.init(out, ld, n_regions, n_bins, mem));

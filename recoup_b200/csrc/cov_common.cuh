@@ -1,5 +1,6 @@
 // Device helpers shared by the coverage kernels (coverage.cu: sorted-index path and
-// GRangesList path; coverage_buckets.cu: reads bucketed per output tile, no sort).
+// GRangesList path; coverage_buckets.cu: reads bucketed per output tile, no sort;
+// coverage_split.cu: the one-pass split path).
 #pragma once
 #include "rcp_internal.cuh"
 

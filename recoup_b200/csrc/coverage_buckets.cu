@@ -1,8 +1,7 @@
 // Coverage without a sort (sm_100a): calcCoverage / coverageFromRanges of the reference
-// (/root/reference/R/coverage.R:126-226) straight from the UNSORTED reads.  Two ways of doing it
-// live here and share the region plan, the tiles and the scan / store code (cov_common.cuh):
-// the BUCKET path (bkt_*, described next; default for masks of short regions) and the BLOCK path
-// (blk_*, described at "BLOCKS mode" below; default for masks made of tiled regions).
+// (/root/reference/R/coverage.R:126-226) straight from the UNSORTED reads: the BUCKET path
+// (bkt_*).  RCP_PATH_AUTO takes it for GRanges masks whose reads are too wide for the split path
+// (coverage_split.cu); the scan / store code of its tiles is shared (cov_common.cuh).
 //
 // Only reads that overlap a region contribute to that region's coverage, and a region's coverage
 // does not depend on the order of its reads.  So instead of sorting every read by coordinate
@@ -606,529 +605,6 @@ inline unsigned reads_grid(int64_t n, size_t smem) {
     return (unsigned)b;
 }
 
-// ================================================================================================
-// BLOCKS mode: the same coverage without the cell table, the hit list and the place pass.
-//   filter     reads that pass the block bitmap, compacted into one dense candidate array (one
-//              atomic reservation per 256+ survivors of a warp)
-//   partition  the survivors are grouped by 16-kb genome block (start >> 14) with two 9-bit
-//              multisplit passes: per-chunk histograms in shared memory, one prefix sum over
-//              (digit, chunk), then a scatter whose ranks come from shared-memory counters --
-//              no global atomic per element, every pass is a streaming pass
-//   tiles      a tile scans the candidates of the 1-2 blocks under it (those that can reach it:
-//              start >= tile start - widest read) and clips them itself
-// The NULL rule ("no read in any tile") is a warp-per-tile any-hit scan of the same candidates.
-// ================================================================================================
-constexpr int DIG_BITS = 9;                      // bits per multisplit pass
-constexpr int ND = 1 << DIG_BITS;                // digits per pass
-constexpr int BLK_SHIFT = 32 - 2 * DIG_BITS;     // 16-kb blocks (the granule of the bitmap)
-constexpr int N_BLOCKS = 1 << (2 * DIG_BITS);
-constexpr int SHIFT1 = 32 - DIG_BITS, SHIFT2 = BLK_SHIFT;
-constexpr int PCH = 4096;            // elements per partition chunk (one CTA)
-constexpr int PT = 256;              // threads of the partition kernels
-static_assert(BLK_SHIFT == BM_SHIFT, "the filter bitmap and the partition use the same blocks");
-
-struct Cands {
-    uint32_t* s;
-    uint32_t* e;         // end + 1
-    int8_t* st;          // strand (stranded calls only)
-};
-
-// The survivors leave through a per-warp shared-memory buffer that is flushed 256+ at a time with
-// ONE atomic reservation in the dense candidate array and coalesced stores (their order is not
-// deterministic; the coverage, a sum of integers, is).
-constexpr int FB_FLUSH = 256;
-constexpr int FB_CAP = FB_FLUSH + 128;
-template <bool STRANDED>
-__host__ __device__ constexpr size_t filter_smem_fixed() {
-    return (size_t)RWARPS * FB_CAP * (sizeof(uint2) + (STRANDED ? 1 : 0));
-}
-
-template <bool STRANDED>
-__global__ void __launch_bounds__(RTPB)
-blk_filter_kernel(int64_t n, const uint32_t* __restrict__ g_start,
-                  const uint32_t* __restrict__ g_end1, const int8_t* __restrict__ strand,
-                  const uint32_t* __restrict__ bitmap, int bm_words, Cands out,
-                  uint32_t* __restrict__ total) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    uint2* fb = reinterpret_cast<uint2*>(smem_raw) + (threadIdx.x >> 5) * FB_CAP;
-    int8_t* fst = reinterpret_cast<int8_t*>(smem_raw + (size_t)RWARPS * FB_CAP * sizeof(uint2)) +
-                  (threadIdx.x >> 5) * FB_CAP;
-    uint32_t* bm = reinterpret_cast<uint32_t*>(smem_raw + filter_smem_fixed<STRANDED>());
-    for (int i = threadIdx.x; i < bm_words; i += RTPB) bm[i] = bitmap[i];
-    __syncthreads();
-    const unsigned lane = threadIdx.x & 31;
-    const unsigned lt = (1u << lane) - 1u;
-    int fill = 0;                   // warp-uniform
-    auto flush = [&]() {
-        __syncwarp();
-        uint32_t base = 0;
-        if (lane == 0) base = atomicAdd(total, (uint32_t)fill);
-        base = __shfl_sync(0xffffffffu, base, 0);
-        for (int i = lane; i < fill; i += 32) {
-            const uint2 x = fb[i];
-            out.s[base + i] = x.x;
-            out.e[base + i] = x.y;
-            if (STRANDED) out.st[base + i] = fst[i];
-        }
-        fill = 0;
-        __syncwarp();
-    };
-    auto keep = [&](uint32_t s, uint32_t e1, int st) {
-        bool ok = e1 > s;
-        if (ok) {
-            const uint32_t b0 = s >> BM_SHIFT, b1 = (e1 - 1u) >> BM_SHIFT;
-            uint32_t w = bm[b0 >> 5] >> (b0 & 31u);
-            if (b1 != b0) w |= bm[b1 >> 5] >> (b1 & 31u);
-            ok = (b1 > b0 + 1u) || (w & 1u);
-        }
-        const unsigned m = __ballot_sync(0xffffffffu, ok);
-        if (ok) {
-            const int p = fill + __popc(m & lt);
-            fb[p] = make_uint2(s, e1);
-            if (STRANDED) fst[p] = (int8_t)st;
-        }
-        fill += __popc(m);
-    };
-    const int64_t n_vec = n >> 2;
-    const int64_t warps_total = (int64_t)gridDim.x * RWARPS;
-    const int64_t gw = (int64_t)blockIdx.x * RWARPS + (threadIdx.x >> 5);
-    for (int64_t base = gw * 32; base < n_vec; base += warps_total * 32) {
-        const int64_t v = base + lane;
-        uint4 s4 = make_uint4(0, 0, 0, 0), e4 = make_uint4(0, 0, 0, 0);
-        char4 t4 = make_char4(0, 0, 0, 0);
-        if (v < n_vec) {
-            s4 = __ldcs(reinterpret_cast<const uint4*>(g_start) + v);
-            e4 = __ldcs(reinterpret_cast<const uint4*>(g_end1) + v);
-            if (STRANDED && strand) t4 = __ldcs(reinterpret_cast<const char4*>(strand) + v);
-        }
-        keep(s4.x, e4.x, t4.x);
-        keep(s4.y, e4.y, t4.y);
-        keep(s4.z, e4.z, t4.z);
-        keep(s4.w, e4.w, t4.w);
-        if (fill >= FB_FLUSH) flush();
-    }
-    if (gw == 0) {                  // the n % 4 tail
-        const int64_t i = n_vec * 4 + lane;
-        const bool ok = i < n;
-        keep(ok ? g_start[i] : 0u, ok ? g_end1[i] : 0u, (ok && STRANDED && strand) ? (int)strand[i] : 0);
-    }
-    if (fill > 0) flush();
-}
-
-// Histogram of one chunk (<= PCH keys at keys[lo, hi)) over the digit (key >> shift) & (ND - 1);
-// written digit-major: hist[digit * stride + column]
-__device__ __forceinline__ void blk_hist_chunk(const uint32_t* __restrict__ keys, uint32_t lo,
-                                               uint32_t hi, int shift, uint32_t* __restrict__ hist,
-                                               size_t stride, size_t column) {
-    __shared__ uint32_t h[ND];
-    for (int d = threadIdx.x; d < ND; d += PT) h[d] = 0;
-    __syncthreads();
-    for (uint32_t i = lo + threadIdx.x; i < hi; i += PT)
-        atomicAdd(&h[(__ldg(keys + i) >> shift) & (ND - 1)], 1u);
-    __syncthreads();
-    for (int d = threadIdx.x; d < ND; d += PT) hist[(size_t)d * stride + column] = h[d];
-}
-
-// Scatter of one chunk by the same digit: ranks from shared-memory counters, elements regrouped
-// by digit in shared memory, then written out so that consecutive threads write consecutive
-// addresses of a digit's run (whole sectors instead of one partial sector per element).
-// gbase[digit * stride + column] = global position of this chunk's first element with that digit.
-template <bool STRANDED>
-__device__ __forceinline__ void blk_scatter_chunk(const Cands& in, uint32_t lo, uint32_t hi, int shift,
-                                                  const uint32_t* __restrict__ gbase, size_t stride,
-                                                  size_t column, const Cands& out) {
-    __shared__ uint32_t cnt[ND];            // count, then local offset of each digit
-    __shared__ uint32_t gb[ND];
-    __shared__ uint32_t wsum[PT / 32];
-    __shared__ uint2 stage[PCH];
-    __shared__ int8_t stage_st[STRANDED ? PCH : 1];
-    const int tid = threadIdx.x;
-    for (int d = tid; d < ND; d += PT) cnt[d] = 0;
-    constexpr int DPT = ND / PT;
-    // the global bases of this thread's digits: issued first, needed only after the local scan
-    uint32_t gbv[DPT];
-#pragma unroll
-    for (int q = 0; q < DPT; q++) gbv[q] = __ldg(gbase + (size_t)(tid * DPT + q) * stride + column);
-    __syncthreads();
-    constexpr int PER = PCH / PT;           // 16 elements per thread
-    uint16_t rk[PER];                       // rank of the element inside its digit in this chunk
-    const uint32_t n = hi - lo;
-#pragma unroll
-    for (int k = 0; k < PER; k++) {
-        const uint32_t i = (uint32_t)k * PT + tid;
-        if (i < n) {
-            rk[k] = (uint16_t)atomicAdd(&cnt[(__ldg(in.s + lo + i) >> shift) & (ND - 1)], 1u);
-            // the ends are read in the staging phase: start them towards L2 now (one per sector)
-            if ((tid & 7) == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(in.e + lo + i));
-        }
-    }
-    __syncthreads();
-    // exclusive scan of the ND digit counts (ND / PT consecutive digits per thread)
-    uint32_t c[DPT], mine = 0;
-#pragma unroll
-    for (int q = 0; q < DPT; q++) {
-        c[q] = cnt[tid * DPT + q];
-        mine += c[q];
-    }
-    uint32_t inc = mine;
-    const unsigned lane = tid & 31;
-#pragma unroll
-    for (int dd = 1; dd < 32; dd <<= 1) {
-        const uint32_t o = __shfl_up_sync(0xffffffffu, inc, dd);
-        if (lane >= (unsigned)dd) inc += o;
-    }
-    if (lane == 31) wsum[tid >> 5] = inc;
-    __syncthreads();
-    uint32_t run = inc - mine;
-    for (int k = 0; k < (tid >> 5); k++) run += wsum[k];
-#pragma unroll
-    for (int q = 0; q < DPT; q++) {
-        const int d = tid * DPT + q;
-        cnt[d] = run;                                       // local offset of digit d
-        gb[d] = gbv[q] - run;                               // global position = gb[d] + local position
-        run += c[q];
-    }
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < PER; k++) {
-        const uint32_t i = (uint32_t)k * PT + tid;
-        if (i < n) {
-            const uint32_t sv = __ldg(in.s + lo + i);       // second read: L1 / L2 hit
-            const uint32_t p = cnt[(sv >> shift) & (ND - 1)] + rk[k];
-            stage[p] = make_uint2(sv, __ldcs(in.e + lo + i));
-            if (STRANDED) stage_st[p] = __ldcs(in.st + lo + i);
-        }
-    }
-    __syncthreads();
-    for (uint32_t i = tid; i < n; i += PT) {
-        const uint2 x = stage[i];
-        const uint32_t g = gb[(x.x >> shift) & (ND - 1)] + i;
-        out.s[g] = x.x;
-        out.e[g] = x.y;
-        if (STRANDED) out.st[g] = stage_st[i];
-    }
-}
-
-// pass 1: one CTA per chunk of the dense candidate array.  The number of chunks is only known on
-// the device (nc1 = ceil(candidates / PCH)); the launches are sized for the upper bound and the
-// histogram is laid out compactly, hist1[digit * nc1 + chunk], so that its prefix sum runs over
-// ND * nc1 entries (sizes[0], written here) instead of the upper bound.
-__device__ __forceinline__ uint32_t blk_nc1(uint32_t total) { return (total + PCH - 1) / PCH; }
-
-__global__ void __launch_bounds__(PT)
-blk_hist1_kernel(const uint32_t* __restrict__ keys, const uint32_t* __restrict__ total,
-                 uint32_t* __restrict__ hist, uint32_t* __restrict__ sizes) {
-    const uint32_t c = blockIdx.x;
-    const uint32_t tot = *total, nc1 = blk_nc1(tot);
-    if (c == 0 && threadIdx.x == 0) sizes[0] = (uint32_t)ND * nc1;
-    if (c >= nc1) return;
-    const uint32_t lo = c * PCH;
-    blk_hist_chunk(keys, lo, min(lo + (uint32_t)PCH, tot), SHIFT1, hist, (size_t)nc1, (size_t)c);
-}
-
-template <bool STRANDED>
-__global__ void __launch_bounds__(PT, 5)
-blk_scatter1_kernel(Cands in, const uint32_t* __restrict__ total, const uint32_t* __restrict__ pos,
-                    Cands out) {
-    const uint32_t c = blockIdx.x;
-    const uint32_t tot = *total, nc1 = blk_nc1(tot);
-    if (c >= nc1) return;
-    const uint32_t lo = c * PCH;
-    blk_scatter_chunk<STRANDED>(in, lo, min(lo + (uint32_t)PCH, tot), SHIFT1, pos, (size_t)nc1, (size_t)c, out);
-}
-
-// After pass 1: start of each top-digit run (S1[ND + 1]) and the prefix of the chunk counts of
-// pass 2 (CP[ND + 1]): run d is cut into ceil(size / PCH) chunks; sizes[1] = entries of the
-// pass-2 histogram.  One CTA of ND threads.
-__global__ void __launch_bounds__(ND)
-blk_runs_kernel(const uint32_t* __restrict__ cand_total, const uint32_t* __restrict__ pos /* scan of hist1 */,
-                uint32_t* __restrict__ S1, uint32_t* __restrict__ CP, uint32_t* __restrict__ sizes) {
-    __shared__ uint32_t w[ND / 32];
-    const int d = threadIdx.x;
-    const uint32_t total = *cand_total, nc1 = blk_nc1(total);
-    const uint32_t s = total ? pos[(size_t)d * nc1] : 0u;
-    const uint32_t e = (d == ND - 1 || total == 0u) ? total : pos[(size_t)(d + 1) * nc1];
-    S1[d] = s;
-    if (d == ND - 1) S1[ND] = total;
-    const uint32_t nch = (e - s + PCH - 1) / PCH;
-    uint32_t inc = nch;
-    const unsigned lane = d & 31;
-#pragma unroll
-    for (int dd = 1; dd < 32; dd <<= 1) {
-        const uint32_t o = __shfl_up_sync(0xffffffffu, inc, dd);
-        if (lane >= (unsigned)dd) inc += o;
-    }
-    if (lane == 31) w[d >> 5] = inc;
-    __syncthreads();
-    uint32_t pre = 0;
-    for (int k = 0; k < (d >> 5); k++) pre += w[k];
-    CP[d] = pre + inc - nch;
-    if (d == ND - 1) {
-        CP[ND] = pre + inc;
-        sizes[1] = (uint32_t)ND * (pre + inc);
-    }
-}
-
-// which (run, chunk) a pass-2 CTA owns; false past the last chunk
-__device__ __forceinline__ bool blk_chunk_of(uint32_t g, const uint32_t* __restrict__ CP,
-                                             const uint32_t* __restrict__ S1, int* d_out,
-                                             uint32_t* lo, uint32_t* hi, uint32_t* nch, uint32_t* j) {
-    if (g >= CP[ND]) return false;
-    int a = 0, b = ND;                  // largest d with CP[d] <= g
-    while (b - a > 1) {
-        const int mid = (a + b) >> 1;
-        if (CP[mid] <= g) a = mid;
-        else b = mid;
-    }
-    *d_out = a;
-    *nch = CP[a + 1] - CP[a];
-    *j = g - CP[a];
-    *lo = S1[a] + *j * PCH;
-    *hi = min(*lo + (uint32_t)PCH, S1[a + 1]);
-    return true;
-}
-
-// pass 2 inside the runs of pass 1; hist2[CP[d] * ND + digit * nch_d + j]
-__global__ void __launch_bounds__(PT)
-blk_hist2_kernel(const uint32_t* __restrict__ keys, const uint32_t* __restrict__ CP,
-                 const uint32_t* __restrict__ S1, uint32_t* __restrict__ hist) {
-    int d;
-    uint32_t lo, hi, nch, j;
-    if (!blk_chunk_of(blockIdx.x, CP, S1, &d, &lo, &hi, &nch, &j)) return;
-    blk_hist_chunk(keys, lo, hi, SHIFT2, hist + (size_t)CP[d] * ND, (size_t)nch, (size_t)j);
-}
-
-template <bool STRANDED>
-__global__ void __launch_bounds__(PT, 5)
-blk_scatter2_kernel(Cands in, const uint32_t* __restrict__ CP, const uint32_t* __restrict__ S1,
-                    const uint32_t* __restrict__ pos, Cands out) {
-    int d;
-    uint32_t lo, hi, nch, j;
-    if (!blk_chunk_of(blockIdx.x, CP, S1, &d, &lo, &hi, &nch, &j)) return;
-    blk_scatter_chunk<STRANDED>(in, lo, hi, SHIFT2, pos + (size_t)CP[d] * ND, (size_t)nch, (size_t)j, out);
-}
-
-// first candidate of every block (N_BLOCKS + 1 entries) from the scanned pass-2 histogram
-__global__ void __launch_bounds__(PT)
-blk_offsets_kernel(const uint32_t* __restrict__ CP, const uint32_t* __restrict__ S1,
-                   const uint32_t* __restrict__ pos2, uint32_t* __restrict__ boff) {
-    const uint32_t b = blockIdx.x * PT + threadIdx.x;
-    if (b > (uint32_t)N_BLOCKS) return;
-    if (b == (uint32_t)N_BLOCKS) {
-        boff[b] = S1[ND];
-        return;
-    }
-    const uint32_t d = b >> DIG_BITS, low = b & (ND - 1);
-    const uint32_t nch = CP[d + 1] - CP[d];
-    boff[b] = nch ? pos2[(size_t)CP[d] * ND + (size_t)low * nch] : S1[d];
-}
-
-// candidates that can reach the tile [ts, ts + tl): those of the blocks from (ts - widest + 1)
-// to the tile's last base
-__device__ __forceinline__ void blk_range(uint32_t ts, uint32_t tl, uint32_t max_w,
-                                          const uint32_t* __restrict__ boff, uint32_t* c0,
-                                          uint32_t* c1) {
-    const uint32_t first = ts >= max_w ? ts - max_w + 1u : 0u;
-    *c0 = __ldg(boff + (first >> BLK_SHIFT));
-    *c1 = __ldg(boff + ((ts + tl - 1u) >> BLK_SHIFT) + 1u);
-}
-
-__device__ __forceinline__ bool blk_hit(uint32_t s, uint32_t e1, int st, uint32_t ts, uint32_t tl,
-                                        uint32_t flags, bool stranded, uint32_t* packed) {
-    if (!(s < ts + tl && e1 > ts)) return false;
-    if (stranded) {
-        const unsigned bit = st > 0 ? 0u : (st < 0 ? 1u : 2u);
-        if (!((flags >> (1 + bit)) & 1u)) return false;       // flags: bit0 reverse, bits1..3 classes
-    }
-    uint32_t lo = max(s, ts) - ts, hi = min(e1, ts + tl) - ts;
-    if (flags & 1u) {
-        const uint32_t l2 = tl - hi;
-        hi = tl - lo;
-        lo = l2;
-    }
-    *packed = lo | (hi << 16);
-    return true;
-}
-
-// NULL rule: does any candidate overlap the tile?  One warp per tile, early exit.
-__global__ void __launch_bounds__(CTA)
-blk_any_kernel(int64_t T, Tiles tiles, Cands c, const uint32_t* __restrict__ boff, uint32_t max_w,
-               int stranded, uint32_t* __restrict__ tile_any) {
-    const int64_t t = (int64_t)blockIdx.x * WARPS + (threadIdx.x >> 5);
-    if (t >= T) return;
-    const unsigned lane = threadIdx.x & 31;
-    const uint2 a = tiles.a[t];
-    const uint32_t ts = a.x, tl = a.y & 0xffffu, flags = a.y >> 16;
-    uint32_t c0, c1, packed;
-    blk_range(ts, tl, max_w, boff, &c0, &c1);
-    bool any = false;
-    for (uint32_t i0 = c0; i0 < c1 && !any; i0 += 32) {
-        const uint32_t i = i0 + lane;
-        bool hit = false;
-        if (i < c1) hit = blk_hit(__ldg(c.s + i), __ldg(c.e + i), (stranded && c.st) ? (int)__ldg(c.st + i) : 0, ts, tl,
-                                  flags, stranded != 0, &packed);
-        any = __any_sync(0xffffffffu, hit);
-    }
-    if (lane == 0) tile_any[t] = any ? 1u : 0u;
-}
-
-// descriptors of blocks mode: b0 / n = the candidate range, pad[0] = tile start, pad[1] = flags
-__global__ void __launch_bounds__(CTA)
-blk_desc_kernel(int64_t T, Tiles tiles, const uint32_t* __restrict__ boff, uint32_t max_w,
-                const uint8_t* __restrict__ is_null, const int64_t* __restrict__ off,
-                TileDesc* __restrict__ desc) {
-    const int64_t t = (int64_t)blockIdx.x * CTA + threadIdx.x;
-    if (t >= T) return;
-    const uint2 a = tiles.a[t], b = tiles.b[t];
-    const uint32_t tl = a.y & 0xffffu;
-    uint32_t c0, c1;
-    blk_range(a.x, tl, max_w, boff, &c0, &c1);
-    TileDesc d;
-    d.out = off[b.x] + b.y;
-    d.b0 = c0;
-    d.n = c1 - c0;
-    d.tlen = is_null[b.x] ? 0 : (int32_t)tl;
-    d.pad[0] = (int32_t)a.x;
-    d.pad[1] = (int32_t)(a.y >> 16);
-    d.pad[2] = 0;
-    desc[t] = d;
-}
-
-__device__ __forceinline__ TileDesc load_desc_full(const TileDesc* __restrict__ p) {
-    const int4 a = __ldg(reinterpret_cast<const int4*>(p));
-    const int4 b = __ldg(reinterpret_cast<const int4*>(p) + 1);
-    TileDesc d;
-    d.out = (int64_t)(((uint64_t)(uint32_t)a.y << 32) | (uint32_t)a.x);
-    d.b0 = (uint32_t)a.z;
-    d.n = (uint32_t)a.w;
-    d.tlen = b.x;
-    d.pad[0] = b.y;
-    d.pad[1] = b.z;
-    d.pad[2] = b.w;
-    return d;
-}
-
-// The candidate loads are issued four per thread at a time (the first batch before the tile is
-// cleared): a tile has ~10^3 candidates, so one batch usually covers it and the loop pays the
-// L2 / HBM latency once instead of once per candidate.
-template <int RPW, bool STRANDED>
-__device__ __forceinline__ void blk_tile_body(int* diff, int* wtot, const TileDesc& d, Cands c,
-                                              int32_t* __restrict__ dst) {
-    constexpr int B = 4;
-    const uint32_t tid = threadIdx.x;
-    const int tlen = d.tlen;
-    const uint32_t n = d.n;
-    const uint32_t* cs = c.s + d.b0;
-    const uint32_t* ce = c.e + d.b0;
-    const int8_t* ct = (STRANDED && c.st) ? c.st + d.b0 : nullptr;    // no strand array: every read is '*'
-    uint32_t s[B], e[B];
-    int st[B];
-    auto load = [&](uint32_t i0) {
-#pragma unroll
-        for (int k = 0; k < B; k++) {
-            const uint32_t i = i0 + (uint32_t)k * CTA + tid;
-            const bool ok = i < n;
-            s[k] = ok ? __ldg(cs + i) : 0u;
-            e[k] = ok ? __ldg(ce + i) : 0u;            // end 0: never a hit
-            st[k] = (STRANDED && ok && ct) ? (int)__ldg(ct + i) : 0;
-        }
-    };
-    load(0);
-#pragma unroll
-    for (int k = 0; k < RPW; k++)
-        reinterpret_cast<int4*>(diff)[k * CTA + tid] = make_int4(0, 0, 0, 0);
-    __syncthreads();
-    const uint32_t ts = (uint32_t)d.pad[0], flags = (uint32_t)d.pad[1];
-    for (uint32_t i0 = 0; i0 < n; i0 += B * CTA) {
-        if (i0) load(i0);
-#pragma unroll
-        for (int k = 0; k < B; k++) {
-            uint32_t packed;
-            if (blk_hit(s[k], e[k], st[k], ts, (uint32_t)tlen, flags, STRANDED, &packed)) {
-                const int lo = (int)(packed & 0xffffu), hi = (int)(packed >> 16);
-                atomicAdd(diff + lo, 1);
-                if (hi < tlen) atomicSub(diff + hi, 1);
-            }
-        }
-    }
-    __syncthreads();
-    block_scan_store_fwd<RPW, true>(diff, tlen, wtot, dst);
-}
-
-template <bool STRANDED>
-__device__ __forceinline__ void blk_tile_dispatch(int* diff, int* wtot, const TileDesc& d, Cands c,
-                                                  int32_t* __restrict__ dst) {
-    const int rpw = ((d.tlen + ROW - 1) / ROW + WARPS - 1) / WARPS;
-    switch (rpw) {
-        case 1: blk_tile_body<1, STRANDED>(diff, wtot, d, c, dst); break;
-        case 2: blk_tile_body<2, STRANDED>(diff, wtot, d, c, dst); break;
-        case 3: blk_tile_body<3, STRANDED>(diff, wtot, d, c, dst); break;
-        case 4: blk_tile_body<4, STRANDED>(diff, wtot, d, c, dst); break;
-        case 5: blk_tile_body<5, STRANDED>(diff, wtot, d, c, dst); break;
-        case 6: blk_tile_body<6, STRANDED>(diff, wtot, d, c, dst); break;
-        default: blk_tile_body<7, STRANDED>(diff, wtot, d, c, dst); break;
-    }
-}
-
-__global__ void __launch_bounds__(CTA, 5)
-blk_tile_kernel(int64_t Tb, const TileDesc* __restrict__ desc, Cands c, int stranded,
-                int32_t* __restrict__ cov) {
-    __shared__ __align__(16) int diff[TILE];
-    __shared__ int wtot[WARPS];
-    const uint32_t tid = threadIdx.x;
-    const int64_t step = gridDim.x;
-    int64_t t = blockIdx.x;
-    if (t >= Tb) return;
-    TileDesc d = load_desc_full(desc + t);
-    for (;;) {
-        TileDesc dn;
-        dn.tlen = 0;
-        if (t + step < Tb) dn = load_desc_full(desc + t + step);
-        if (d.tlen > 0) {
-            if (stranded) blk_tile_dispatch<true>(diff, wtot, d, c, cov + d.out);
-            else blk_tile_dispatch<false>(diff, wtot, d, c, cov + d.out);
-        }
-        t += step;
-        if ((tid & 31u) == 0) tma_store_wait_read();
-        if (t >= Tb) break;
-        __syncthreads();
-        d = dn;
-    }
-}
-
-__global__ void __launch_bounds__(CTA)
-blk_small_kernel(int64_t Ts, const TileDesc* __restrict__ desc, Cands c, int stranded,
-                 int32_t* __restrict__ cov) {
-    __shared__ __align__(16) int sm[WARPS][SMALL_MAX];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t ts_i = (int64_t)blockIdx.x * WARPS + warp;
-    if (ts_i >= Ts) return;
-    const TileDesc d = load_desc_full(desc + ts_i);
-    const int L = d.tlen;
-    if (L == 0) return;
-    int* diff = sm[warp];
-    const int nrows = (L + ROW - 1) / ROW;
-    for (int i = lane; i < nrows * (ROW / 4); i += 32)
-        reinterpret_cast<int4*>(diff)[i] = make_int4(0, 0, 0, 0);
-    __syncwarp();
-    const uint32_t ts = (uint32_t)d.pad[0], flags = (uint32_t)d.pad[1];
-    for (uint32_t i = lane; i < d.n; i += 32) {
-        const uint32_t s = __ldg(c.s + d.b0 + i), e1 = __ldg(c.e + d.b0 + i);
-        uint32_t packed;
-        if (blk_hit(s, e1, (stranded && c.st) ? (int)__ldg(c.st + d.b0 + i) : 0, ts, (uint32_t)L, flags, stranded != 0,
-                    &packed)) {
-            const int lo = (int)(packed & 0xffffu), hi = (int)(packed >> 16);
-            atomicAdd(diff + lo, 1);
-            if (hi < L) atomicSub(diff + hi, 1);
-        }
-    }
-    __syncwarp();
-    int32_t* dst = cov + d.out;
-    int pre = 0;
-    for (int row = 0; row < nrows; row++)
-        pre += warp_row_scan_store(diff + row * ROW, pre, 0, false, L - row * ROW, dst + row * ROW);
-}
-
 // Device scratch of one call.  Three arenas (one allocation each: the host is on the critical
 // path right after the two synchronisation points, and ~30 stream-ordered allocations plus as
 // many frees cost more than the small kernels between them): A sized by the regions, B by the
@@ -1192,11 +668,6 @@ int launch_rescatter(const ReadsIdx& rd, const Work& w) {
 // the mask is dense AND the read set is very large: there the random accesses of the two read
 // passes leave L2 (C5 at full size: 200 M reads, 10^6 windows: 12.3 ms against 10.6 ms through
 // the sorted index), while for sparse masks or fewer reads the buckets win (C2, C3, C5 / 4).
-static int blocks_ranges_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32_t* start,
-                             const int32_t* end, const int8_t* strand, int ignore_strand,
-                             int strand_filter, int mem, Coverage* cv, Work* plan, int64_t plan_Tb,
-                             int64_t plan_Ts);
-
 int coverage_ranges_bucketed(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32_t* start,
                              const int32_t* end, const int8_t* strand, int ignore_strand,
                              int strand_filter, int mem, bool may_switch, Coverage* cv) {
@@ -1265,16 +736,6 @@ int coverage_ranges_bucketed(ReadsIdx& rd, int64_t R, const int32_t* chrom, cons
     if (may_switch && rd.n >= switch_reads &&
         (double)Tb * TILE + (double)Ts * SMALL_MAX >= 0.25 * (double)rd.chrom_off[(size_t)rd.n_chrom])
         return RCP_SWITCH_TO_INDEX;
-    // Masks made of tiled regions (TSS windows, gene bodies) go through the block partition, which
-    // has no per-read random access (C2 1.40 vs 1.54 ms, C3 7.7 vs 8.0 ms); masks dominated by
-    // short regions keep the buckets: a short region would scan every candidate of its 16-kb block
-    // (C5 at 1/4 scale: 2.84 vs 2.35 ms).
-    // (a tile looks back by the widest read for its candidates: a sample with very long reads
-    // would make every tile scan many blocks, so those stay with the buckets too)
-    if (may_switch && Ts * 4 <= Tb && rd.n < 0xfffff000ll && rd.max_width <= (2u << BM_SHIFT) &&
-        getenv("RCP_AUTO_NO_BLOCKS") == nullptr)
-        return blocks_ranges_impl(rd, R, chrom, start, end, strand, ignore_strand, strand_filter, mem, cv,
-                                  &w, Tb, Ts);
 
     // ---- 2. tiles, cell table, block bitmap -------------------------------------------------
     const int64_t span = (int64_t)rd.chrom_off[(size_t)rd.n_chrom];
@@ -1394,228 +855,6 @@ int coverage_ranges_bucketed(ReadsIdx& rd, int64_t R, const int32_t* chrom, cons
         RCP_LAUNCHED();
     }
     return RCP_OK;
-}
-
-// BLOCKS mode (see the kernels above): same contract as coverage_ranges_bucketed.
-// `plan` (with its tile counts) is the finished region plan of coverage_ranges_bucketed when that
-// function hands the call over; nullptr: plan here.
-static int blocks_ranges_impl(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32_t* start,
-                             const int32_t* end, const int8_t* strand, int ignore_strand,
-                             int strand_filter, int mem, Coverage* cv, Work* plan, int64_t plan_Tb,
-                             int64_t plan_Ts) {
-    const bool stranded = !((strand_filter == RCP_STRAND_ANY) && (ignore_strand || strand == nullptr));
-    const bool st_arr = stranded && rd.d_strand != nullptr;      // strandless reads are all '*'
-    if (rd.n >= 0xfffff000ll) return fail(RCP_ERR_UNSUPPORTED, "blocks mode: more than 2^32 reads");
-    Work own;
-    Work& w = plan ? *plan : own;
-    struct Host {
-        int64_t Tb, Ts, total_padded;
-        unsigned long long stats[3];
-        unsigned int err;
-    } h = {plan_Tb, plan_Ts, 0, {0, 0, 0}, 0};
-    if (!plan) {
-    DevIn<int32_t> d_chrom, d_start, d_end;
-    DevIn<int8_t> d_strand;
-    RCP_TRY(d_chrom.init(chrom, (size_t)R, mem));
-    RCP_TRY(d_start.init(start, (size_t)R, mem));
-    RCP_TRY(d_end.init(end, (size_t)R, mem));
-    RCP_TRY(d_strand.init(strand, (size_t)R, mem));
-    cv->n_regions = R;
-    RCP_TRY(dalloc(&cv->off, (size_t)R + 1));
-    RCP_TRY(dalloc(&cv->len, (size_t)R));
-    RCP_TRY(dalloc(&cv->is_null, (size_t)R));
-    {
-        const size_t r = (size_t)R;
-        RCP_TRY(w.A.reserve(Arena::pad(r * 4) * 2 + Arena::pad(r) + Arena::pad(r * 8) * 3 +
-                            Arena::pad((r + 1) * 8) * 2 + Arena::pad(4) + Arena::pad(24)));
-        w.err = w.A.take<unsigned int>(1);
-        w.stats = w.A.take<unsigned long long>(3);
-        w.gs = w.A.take<uint32_t>(r);
-        w.plen = w.A.take<int32_t>(r);
-        w.flags = w.A.take<uint8_t>(r);
-        w.nbig = w.A.take<int64_t>(r);
-        w.nsmall = w.A.take<int64_t>(r);
-        w.padded = w.A.take<int64_t>(r);
-        w.off_big = w.A.take<int64_t>(r + 1);
-        w.off_small = w.A.take<int64_t>(r + 1);
-        if (w.A.used > w.A.cap) return fail(RCP_ERR_CUDA, "internal: region arena overrun");
-    }
-    RCP_CUDA(cudaMemsetAsync(w.err, 0, 512, g_ctx.stream));
-    {
-        StageTimer t(ST_BKT_PLAN);
-        if (R > 0) {
-            bkt_plan_kernel<<<blocks_for(R, CTA), CTA, 0, g_ctx.stream>>>(
-                R, d_chrom.ptr, d_start.ptr, d_end.ptr, d_strand.ptr, rd.d_chrom_off,
-                rd.d_chrom_len, rd.n_chrom, ignore_strand, strand_filter, w.gs, w.plen, w.flags,
-                w.nbig, w.nsmall, w.err);
-            RCP_LAUNCHED();
-        }
-        RCP_TRY(exclusive_scan2_i64(w.nbig, w.off_big, w.off_big + R, w.nsmall, w.off_small,
-                                    w.off_small + R, R));
-    }
-    {
-        const FetchItem items[3] = {{w.off_big + R, &h.Tb, 8}, {w.off_small + R, &h.Ts, 8}, {w.err, &h.err, 4}};
-        RCP_TRY(fetch_and_sync(items, 3));
-    }
-    if (h.err & 1u) return fail(RCP_ERR_DATA, "a region has a chromosome id outside [0, n_chrom)");
-    if (h.err & 2u) return fail(RCP_ERR_DATA, "a region has end < start - 1");
-    }   // !plan
-    const int64_t Tb = h.Tb, Ts = h.Ts, T = Tb + Ts;
-    if (T > 0x7fffffff) return fail(RCP_ERR_UNSUPPORTED, "more than 2^31-1 coverage tiles");
-
-    // ---- tiles + block bitmap; filter; two multisplit passes ---------------------------------
-    const int64_t span = (int64_t)rd.chrom_off[(size_t)rd.n_chrom];
-    const int64_t n_cell = (span >> CELL_SHIFT) + 2;
-    w.bm_words = (int)(((span >> BM_SHIFT) + 32) / 32);
-    const int64_t n_chunks = (rd.n + PCH - 1) / PCH + 1;                       // pass-1 chunks (upper bound)
-    const int64_t tc_upper = (rd.n + PCH - 1) / PCH + ND;                      // pass-2 chunks
-    Cands ca, cb;
-    uint32_t *cand_total, *scan_sizes, *hist1, *hist2, *S1, *CP, *blk_off;
-    size_t zero_bytes = 0;
-    {
-        const size_t t = (size_t)T, c = (size_t)n_cell, nc = (size_t)n_chunks, cap = nc * PCH;
-        const size_t st_bytes = st_arr ? Arena::pad(cap) : 0;
-        RCP_TRY(w.B.reserve(Arena::pad((c + 1) * 4) + Arena::pad((size_t)w.bm_words * 4) +
-                            Arena::pad((t + 1) * 4) + Arena::pad((size_t)ND * (size_t)tc_upper * 4 + 4) +
-                            Arena::pad(t * 8) * 2 + Arena::pad(cap * 4) * 4 + st_bytes * 2 +
-                            Arena::pad(8) * 2 + Arena::pad(((size_t)ND * nc + 1) * 4) + Arena::pad((ND + 1) * 4) * 2 +
-                            Arena::pad(((size_t)N_BLOCKS + 1) * 4)));
-        // zero-initialised block first: cell counts (unused here, but bkt_tiles_kernel bumps them),
-        // bitmap, tile flags, candidate counter (the histograms are written in full by their kernels)
-        w.cells.cnt = w.B.take<uint32_t>(c + 1);
-        w.cells.bitmap = w.B.take<uint32_t>((size_t)w.bm_words);
-        w.tile_cnt = w.B.take<uint32_t>(t + 1);
-        cand_total = w.B.take<uint32_t>(1);           // number of candidates
-        zero_bytes = w.B.used;
-        scan_sizes = w.B.take<uint32_t>(2);           // entries of the pass-1 / pass-2 histograms
-        hist1 = w.B.take<uint32_t>((size_t)ND * nc + 1);
-        hist2 = w.B.take<uint32_t>((size_t)ND * (size_t)tc_upper + 1);
-        w.tiles.a = w.B.take<uint2>(t);
-        w.tiles.b = w.B.take<uint2>(t);
-        ca.s = w.B.take<uint32_t>(cap);
-        ca.e = w.B.take<uint32_t>(cap);
-        cb.s = w.B.take<uint32_t>(cap);
-        cb.e = w.B.take<uint32_t>(cap);
-        ca.st = st_arr ? w.B.take<int8_t>(cap) : nullptr;
-        cb.st = st_arr ? w.B.take<int8_t>(cap) : nullptr;
-        S1 = w.B.take<uint32_t>(ND + 1);
-        CP = w.B.take<uint32_t>(ND + 1);
-        blk_off = w.B.take<uint32_t>((size_t)N_BLOCKS + 1);
-        if (w.B.used > w.B.cap) return fail(RCP_ERR_CUDA, "internal: blocks arena overrun");
-    }
-    {
-        StageTimer t(ST_BKT_PLAN);
-        RCP_CUDA(cudaMemsetAsync(w.B.base, 0, zero_bytes, g_ctx.stream));
-        if (T > 0) {
-            bkt_tiles_kernel<<<blocks_for(T, CTA), CTA, 0, g_ctx.stream>>>(
-                R, Tb, Ts, w.off_big, w.off_small, w.gs, w.plen, w.flags, w.tiles, w.cells.cnt,
-                w.cells.bitmap);
-            RCP_LAUNCHED();
-        }
-    }
-    {
-        StageTimer t(ST_BLK_FILTER);
-        if (st_arr) {
-            const size_t smem = filter_smem_fixed<true>() + (size_t)w.bm_words * 4;
-            RCP_CUDA(cudaFuncSetAttribute(blk_filter_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            blk_filter_kernel<true><<<reads_grid(rd.n, smem), RTPB, smem, g_ctx.stream>>>(
-                rd.n, rd.g_start, rd.g_end1, rd.d_strand, w.cells.bitmap, w.bm_words, ca, cand_total);
-        } else {
-            const size_t smem = filter_smem_fixed<false>() + (size_t)w.bm_words * 4;
-            RCP_CUDA(cudaFuncSetAttribute(blk_filter_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            blk_filter_kernel<false><<<reads_grid(rd.n, smem), RTPB, smem, g_ctx.stream>>>(
-                rd.n, rd.g_start, rd.g_end1, rd.d_strand, w.cells.bitmap, w.bm_words, ca, cand_total);
-        }
-        RCP_LAUNCHED();
-    }
-    {
-        StageTimer t(ST_BLK_HIST);          // pass 1
-        blk_hist1_kernel<<<(unsigned)n_chunks, PT, 0, g_ctx.stream>>>(ca.s, cand_total, hist1, scan_sizes);
-        RCP_LAUNCHED();
-        RCP_TRY(exclusive_scan_u32_bounded(hist1, hist1, (int64_t)ND * n_chunks, scan_sizes, nullptr));
-    }
-    {
-        StageTimer t(ST_BLK_SCATTER);
-        if (st_arr) blk_scatter1_kernel<true><<<(unsigned)n_chunks, PT, 0, g_ctx.stream>>>(ca, cand_total, hist1, cb);
-        else blk_scatter1_kernel<false><<<(unsigned)n_chunks, PT, 0, g_ctx.stream>>>(ca, cand_total, hist1, cb);
-        RCP_LAUNCHED();
-    }
-    {
-        StageTimer t(ST_BLK_HIST);          // pass 2
-        blk_runs_kernel<<<1, ND, 0, g_ctx.stream>>>(cand_total, hist1, S1, CP, scan_sizes);
-        RCP_LAUNCHED();
-        blk_hist2_kernel<<<(unsigned)tc_upper, PT, 0, g_ctx.stream>>>(cb.s, CP, S1, hist2);
-        RCP_LAUNCHED();
-        RCP_TRY(exclusive_scan_u32_bounded(hist2, hist2, (int64_t)ND * tc_upper, scan_sizes + 1, nullptr));
-    }
-    {
-        StageTimer t(ST_BLK_SCATTER);
-        if (st_arr) blk_scatter2_kernel<true><<<(unsigned)tc_upper, PT, 0, g_ctx.stream>>>(cb, CP, S1, hist2, ca);
-        else blk_scatter2_kernel<false><<<(unsigned)tc_upper, PT, 0, g_ctx.stream>>>(cb, CP, S1, hist2, ca);
-        RCP_LAUNCHED();
-    }
-    // ---- NULL rule, offsets ---------------------------------------------------------------------
-    const uint32_t max_w = rd.max_width > 0 ? rd.max_width : 1u;
-    {
-        StageTimer t(ST_BKT_PLAN);
-        blk_offsets_kernel<<<(N_BLOCKS + 1 + PT - 1) / PT, PT, 0, g_ctx.stream>>>(CP, S1, hist2, blk_off);
-        RCP_LAUNCHED();
-        if (T > 0) {
-            blk_any_kernel<<<blocks_for(T, WARPS), CTA, 0, g_ctx.stream>>>(T, w.tiles, ca, blk_off, max_w,
-                                                                           stranded ? 1 : 0, w.tile_cnt);
-            RCP_LAUNCHED();
-        }
-        if (R > 0) {
-            bkt_null_kernel<<<blocks_for(R, CTA), CTA, 0, g_ctx.stream>>>(
-                R, Tb, w.off_big, w.off_small, w.plen, w.tile_cnt, cv->len, cv->is_null, w.padded,
-                w.stats);
-            RCP_LAUNCHED();
-        }
-        RCP_TRY(exclusive_scan_i64(w.padded, cv->off, R, cv->off + R));
-    }
-    uint32_t h_cand = 0;
-    {
-        const FetchItem items[3] = {{cv->off + R, &h.total_padded, 8}, {w.stats, h.stats, 24},
-                                    {cand_total, &h_cand, 4}};
-        RCP_TRY(fetch_and_sync(items, 3));
-    }
-    cv->path = RCP_PATH_BLOCKS;
-    cv->candidates = (int64_t)h_cand;
-    cv->total_padded = h.total_padded;
-    cv->n_null = (int64_t)h.stats[0];
-    cv->total_len = (int64_t)h.stats[1];
-    cv->max_len = (int32_t)h.stats[2];
-    RCP_TRY(dalloc(&cv->cov, (size_t)h.total_padded));
-    if (T == 0 || cv->n_null == R) return RCP_OK;
-    RCP_TRY(w.C.reserve(Arena::pad((size_t)T * sizeof(TileDesc))));
-    w.desc = w.C.take<TileDesc>((size_t)T);
-    blk_desc_kernel<<<blocks_for(T, CTA), CTA, 0, g_ctx.stream>>>(T, w.tiles, blk_off, max_w, cv->is_null,
-                                                                 cv->off, w.desc);
-    RCP_LAUNCHED();
-    if (Tb > 0) {
-        StageTimer t(ST_BLK_TILE);
-        int per_sm = 0;
-        RCP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, blk_tile_kernel, CTA, 0));
-        if (per_sm < 1) per_sm = 1;
-        blk_tile_kernel<<<(unsigned)std::min<int64_t>(Tb, (int64_t)g_ctx.sm_count * per_sm), CTA, 0,
-                          g_ctx.stream>>>(Tb, w.desc, ca, stranded ? 1 : 0, cv->cov);
-        RCP_LAUNCHED();
-    }
-    if (Ts > 0) {
-        StageTimer t(ST_BLK_SMALL);
-        blk_small_kernel<<<blocks_for(Ts, WARPS), CTA, 0, g_ctx.stream>>>(Ts, w.desc + Tb, ca,
-                                                                         stranded ? 1 : 0, cv->cov);
-        RCP_LAUNCHED();
-    }
-    return RCP_OK;
-}
-
-// RCP_PATH_BLOCKS: the block partition for every GRanges mask
-int coverage_ranges_blocks(ReadsIdx& rd, int64_t R, const int32_t* chrom, const int32_t* start,
-                           const int32_t* end, const int8_t* strand, int ignore_strand,
-                           int strand_filter, int mem, Coverage* cv) {
-    return blocks_ranges_impl(rd, R, chrom, start, end, strand, ignore_strand, strand_filter, mem, cv,
-                              nullptr, 0, 0);
 }
 
 }  // namespace rcp

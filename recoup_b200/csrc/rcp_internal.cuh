@@ -69,16 +69,10 @@ enum Stage {
     ST_BKT_SCATTER,     // bucket path: scatter pass over the reads
     ST_BKT_TILE,        // bucket path: bkt_tile_kernel
     ST_BKT_SMALL,       // bucket path: bkt_small_kernel
-    ST_BLK_FILTER,      // block path: blk_filter_kernel (one launch)
-    ST_BLK_HIST,        // block path: per-chunk digit histograms + their prefix sums (two passes)
-    ST_BLK_SCATTER,     // block path: blk_scatter1/2_kernel (one launch per pass)
-    ST_BLK_TILE,        // block path: blk_tile_kernel
-    ST_BLK_SMALL,       // block path: blk_small_kernel
     ST_SP_PLAN,         // split path: windows, bitmap + ranks, tiles, descriptors, NULL rule
     ST_SP_SPLIT,        // split path: sp_split_kernel (filter + one-pass split into groups)
     ST_SP_SORT,         // split path: chunk lists per group + sp_group_kernel (sub-bin sort)
     ST_SP_TILE,         // split path: sp_tile_kernel
-    ST_SP_SMALL,        // split path: sp_small_kernel
     ST_N
 };
 struct StageTimer {
@@ -296,7 +290,7 @@ struct Coverage {
     int64_t n_null = 0;
     int32_t max_len = 0;         // longest region (sizes the staging buffers of the bin kernel)
     int path = 0;                // RCP_PATH_* that produced it (0: list / concat)
-    int64_t candidates = 0;      // block / split path: reads that passed the bitmap filter
+    int64_t candidates = 0;      // split path: reads that passed the bitmap filter
     // split path: n_null / total_len / candidates are produced on the device after the call has
     // returned; they are fetched on first use (coverage_resolve_stats)
     unsigned long long* d_stats = nullptr;   // [0] n_null [1] total_len [2] max_len [3] candidates [4] bound

@@ -1131,24 +1131,37 @@ def test_fused_coverage_profile_device_memory_and_errors(gpu):
 
 def test_auto_serves_ordinary_samples_through_the_split_path(gpu_auto):
     """RCP_PATH_AUTO: short reads over a GRanges mask go through the one-pass split path; reads
-    wider than its packed word allows fall back (same results either way)."""
+    wider than its packed word allows take the buckets (same results either way).  The retired
+    RCP_PATH_BLOCKS selects the buckets too."""
     from recoup_b200 import _lib
     rb = gpu_auto
     rng = np.random.default_rng(8)
     clen = [90000, 30000]
-    for width, want_path in (((30, 250), 4), ((9000, 12000), None)):
+
+    def path_of(cov):
+        pth, cand = C.c_int(0), C.c_int64(0)
+        _lib.check(_lib.lib.rcp_coverage_path_info(cov.handle, C.byref(pth), C.byref(cand)))
+        return pth.value, cand.value
+
+    for width, want_path in (((30, 250), 4), ((9000, 12000), 2)):
         chrom, s, e, st = synth_reads(rng, 5000, clen, width=width)
         o_reads, g_reads = both_reads(chrom, s, e, st, clen)
         rc, rs, re_, rst = _equal_windows(rng, 100, clen, 2500)
         o_mask, g_mask = both_regions(rc, rs, re_, rst, len(clen))
+        want = O.calc_coverage(o_reads, o_mask, None, True)
         cov = rb.calcCoverage(g_reads, g_mask)
-        pth, cand = C.c_int(0), C.c_int64(0)
-        _lib.check(_lib.lib.rcp_coverage_path_info(cov.handle, C.byref(pth), C.byref(cand)))
-        if want_path is not None:
-            assert pth.value == want_path and cand.value > 0
-        else:
-            assert pth.value != 4
-        assert_coverage_equal(cov.to_list(), O.calc_coverage(o_reads, o_mask, None, True))
+        pth, cand = path_of(cov)
+        assert pth == want_path
+        if want_path == 4:
+            assert cand > 0
+        assert_coverage_equal(cov.to_list(), want)
+    rb.set_coverage_path("blocks")
+    try:
+        cov = rb.calcCoverage(g_reads, g_mask)
+    finally:
+        rb.set_coverage_path("auto")
+    assert path_of(cov)[0] == 2
+    assert_coverage_equal(cov.to_list(), want)
 
 
 def test_region_sharded_run_equals_the_single_gpu_matrix(gpu_auto):
