@@ -422,12 +422,21 @@ int rcp_sort_keys_u32(uint32_t* keys, int64_t n, int key_bits, int mem);
  *   forms upper/lower = center +- spread.  sd of a single row is NaN (R: NA).
  * rcp_matrix_row_stat: apply(x, 1, sum | max | mean), the ordering values of orderProfiles
  *   (plot.R:1076-1081, 1110-1131, 1135-1146; the max variant's sample() among tied maxima
- *   returns the same value whichever it picks).
+ *   returns the same value whichever it picks).  Sums and means are the correctly rounded exact
+ *   value in all but pathological rows (double-double accumulation).  Non-finite cells: a sum or
+ *   mean is NaN if a cell is NaN or the row holds both +Inf and -Inf, otherwise +-Inf if a cell
+ *   is infinite; a finite row whose running double sum (column order) overflows gives that
+ *   infinity -- R's long-double accumulator can return a finite value there.  The same rule holds
+ *   for the column means of rcp_matrix_col_profile / rcp_matrix_group_col_profile.  max is NaN
+ *   if a cell is NaN.
  * rcp_order: sort(v, decreasing, index.return=TRUE)$ix (plot.R:1038-1041,1100-1103): 1-based,
  *   ties keep their input order in both directions (R's default radix method), NaN/NA dropped:
  *   *n_out entries of ix are valid (R drops them: na.last = NA).
  * rcp_matrix_quantile: quantile(x, probs), type 7, over every cell (plot.R:519,536); a NaN
- *   anywhere is RCP_ERR_DATA like R's error without na.rm. */
+ *   anywhere is RCP_ERR_DATA like R's error without na.rm.  The arithmetic is quantile.default's,
+ *   each operation rounded on its own: index = 1 + (n - 1) * p, lo = floor(index),
+ *   h = index - lo, (1 - h) * x[lo] + h * x[hi] (1-based), R's operations in R's order; the same
+ *   holds for rcp_reads_width_quantile. */
 #define RCP_ROW_SUM 0
 #define RCP_ROW_MAX 1
 #define RCP_ROW_MEAN 2

@@ -605,19 +605,22 @@ def r_sort_index(v, decreasing=False):
 
 
 def r_quantile7(x, probs):
-    """stats::quantile(x, probs, type = 7) (plot.R:519,536)."""
+    """stats::quantile(x, probs, type = 7) (plot.R:519,536), in quantile.default's own
+    arithmetic: index <- 1 + max(n - 1, 0) * probs, lo <- floor(index), 1-based reads,
+    h <- index - lo.  Adding the 1 before taking h rounds h differently from (n - 1) * p - lo:
+    quantile(c(0, 1), 0.1) is 0.10000000000000009, not 0.1."""
     x = np.sort(np.asarray(x, dtype=np.float64).ravel())
     if x.shape[0] and np.isnan(x[-1]):
         raise ValueError("missing values and NaN's not allowed if 'na.rm' is FALSE")
     n = x.shape[0]
     out = []
     for p in np.atleast_1d(probs):
-        index = (n - 1) * float(p)
+        index = 1.0 + max(n - 1, 0) * float(p)
         lo, hi = int(math.floor(index)), int(math.ceil(index))
-        q = x[lo]
+        q = x[lo - 1]
         h = index - lo
-        if index > lo and x[hi] != q:
-            q = (1.0 - h) * q + h * x[hi]
+        if index > lo and x[hi - 1] != q:
+            q = (1.0 - h) * q + h * x[hi - 1]
         out.append(float(q))
     return np.array(out)
 

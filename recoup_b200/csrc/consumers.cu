@@ -49,6 +49,8 @@ __device__ __forceinline__ double key_value(unsigned long long k) {
 // sums here are carried as unevaluated pairs hi + lo (error-free TwoSum), so that the value
 // handed back is the correctly rounded exact sum in all but pathological cases -- the same
 // double R's 64-bit-mantissa accumulator rounds to.
+// Once the plain sum hi is not finite (an infinite or NaN cell, or an overflow) the pair is
+// {hi, 0}: TwoSum's error term would be inf - inf = NaN and turn a +-Inf sum into NaN.
 struct DD {
     double hi, lo;
 };
@@ -56,7 +58,7 @@ __device__ __forceinline__ DD dd_add(DD a, double x) {
     const double s = a.hi + x;
     const double bb = s - a.hi;
     const double err = (a.hi - (s - bb)) + (x - bb);
-    return {s, a.lo + err};
+    return {s, isfinite(s) ? a.lo + err : 0.0};
 }
 __device__ __forceinline__ DD dd_merge(DD a, DD b) {
     DD r = dd_add(a, b.hi);
@@ -67,8 +69,9 @@ __device__ __forceinline__ double dd_value(DD a) { return a.hi + a.lo; }
 // (hi + lo) / n, correctly rounded in practice
 __device__ __forceinline__ double dd_div(DD a, double n) {
     const double s = a.hi + a.lo;
-    const double rest = (a.hi - s) + a.lo;
     const double q = s / n;
+    if (!isfinite(s)) return q;
+    const double rest = (a.hi - s) + a.lo;
     const double r = fma(-q, n, s) + rest;
     return q + r / n;
 }
@@ -138,16 +141,19 @@ count_le_kernel(int64_t n, const unsigned long long* __restrict__ keys, const do
     if ((threadIdx.x & 31) == 0 && m) atomicAdd(count, (unsigned long long)__popc(m));
 }
 
-// quantile type 7 on sorted keys: index = 1 + (n - 1) p; (1 - h) x[lo] + h x[hi]
+// quantile type 7 on sorted keys, R's quantile.default operation for operation:
+//   index <- 1 + (n - 1) * p; lo <- floor(index); hi <- ceiling(index) (1-based);
+//   h <- index - lo; (1 - h) * x[lo] + h * x[hi] where index > lo and x[hi] != x[lo].
+// Every product and sum is rounded on its own (no FMA contraction), as R rounds them.
 __global__ void quantile_kernel(const unsigned long long* __restrict__ sorted, int64_t n,
                                 const double* __restrict__ probs, int k, double* __restrict__ out) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= k) return;
-    const double index = (double)(n - 1) * probs[j];
+    const double index = __dadd_rn(1.0, __dmul_rn((double)(n - 1), probs[j]));
     const double lo = floor(index), hi = ceil(index);
-    const double xl = key_value(sorted[(int64_t)lo]), xh = key_value(sorted[(int64_t)hi]);
+    const double xl = key_value(sorted[(int64_t)lo - 1]), xh = key_value(sorted[(int64_t)hi - 1]);
     const double h = index - lo;
-    out[j] = (index > lo && xh != xl) ? (1.0 - h) * xl + h * xh : xl;
+    out[j] = (index > lo && xh != xl) ? __dadd_rn(__dmul_rn(1.0 - h, xl), __dmul_rn(h, xh)) : xl;
 }
 
 struct MatIn {

@@ -99,6 +99,8 @@ for (n in c(50,100,150,200)) { set.seed(42); kat[[paste0("perm_42_",n)]] <- samp
 set.seed(1); kat$runif_1 <- runif(3)
 kat$spline_fmm <- spline(c(3,0,7,7,2,9,1,4,4),n=17)$y
 kat$quantile7 <- unname(quantile(1:10,c(0.95,0.25,0.5)))
+# tells index <- 1 + (n - 1) * p (quantile.default) from (n - 1) * p: 0.10000000000000009 vs 0.1
+kat$quantile7_index <- unname(quantile(c(0,1),0.1))
 kat$r_version <- paste(R.version$major,R.version$minor,sep=".")
 kat$sample_kind <- RNGkind()[3]
 con <- file(file.path(out,"kat.txt"),"w")
